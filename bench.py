@@ -3,6 +3,7 @@
 then GCN-input build + AdjMatSeer + bond argmax), one process per GPU.
 
   python bench.py [--gpus N] [--steps K] [--warmup W] [--precision fp16|bf16|tf32] [--workload C3|C2|C1|C4|C5]
+                  [--dump-outputs DIR]
   python -m torch.distributed.run --nproc-per-node N ... bench.py --gpus N ...      (N > 1)
   python bench.py --impl reference ...        (the reference's own torch CPU path on the host cores)
 
@@ -11,7 +12,8 @@ architecture; the HuggingFace checkpoints are not available offline).  Default w
 (8192 molecules of 15-39 atoms + AdjMatSeer) per GPU, weak scaling -- at 8 GPUs that is configs[4]'s 65 536 samples,
 sharded by the product path (parallel.generate_sharded_engine: size-balanced shards keyed by global sample ids, one
 packed NCCL all-gather).  `value` is timed with inputs resident in HBM; `e2e` goes through the host-buffer API (pinned
-host -> device -> pinned host inside the timed region)."""
+host -> device -> pinned host inside the timed region).  Inputs, weights and noise seeds depend only on the arguments, so
+`--dump-outputs DIR` lets two builds of the project be compared output for output."""
 import argparse
 import json
 import os
@@ -72,6 +74,24 @@ def workload(name, world=1, rank=0):
         return dict(B=20, N=19, global_n_nodes=rng.randint(15, 20, 20).astype(np.int32), ctx=CEYYAG_CONTEXT,
                     desc="C1 (configs[0]): B=20 samples, 15-19 atoms (ceyyag), T=100 + AdjMatSeer GCN")
     raise SystemExit("unknown workload " + name)
+
+
+DUMP_BYTES = 64 * 10 ** 6
+
+
+def dump_outputs(path, x, cls, bonds):
+    """Writes what a caller of the timed path receives -- coordinates x (B,N,3), atom classes (B,N) (-1 = padding) and bond
+    orders (B,42,42) -- as float32 .npy files, with the global sample id of each row (float64).  When all molecules
+    exceed DUMP_BYTES, a fixed seeded sample of them is written, so that two builds can be compared file for file."""
+    n = x.shape[0]
+    per_mol = 4 * (x[0].numel() + cls[0].numel() + bonds[0].numel()) + 8
+    keep = min(n, DUMP_BYTES // per_mol)
+    ids = np.arange(n) if keep == n else np.sort(np.random.RandomState(0).choice(n, keep, replace=False))
+    rows = torch.from_numpy(ids).to(x.device)
+    os.makedirs(path, exist_ok=True)
+    for name, t in (("x", x), ("atom_class", cls), ("bond_orders", bonds)):
+        np.save(os.path.join(path, name + ".npy"), t.index_select(0, rows).float().cpu().numpy())
+    np.save(os.path.join(path, "sample_id.npy"), ids.astype(np.float64))
 
 
 def alg_flops_forward(n_nodes):
@@ -384,7 +404,13 @@ def main():
     ap.add_argument("--ref-device", default="cpu", choices=["cpu", "cuda"])
     ap.add_argument("--ref-mols", type=int, default=0)
     ap.add_argument("--ref-full", action="store_true", help="reference arm: time the whole 100-step loop, no extrapolation")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the results of the last timed step to DIR/<name>.npy (float32, at most 64 MB)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes the results of the b200 arm")
     if args.impl == "reference":
         run_reference(args)
         return
@@ -430,7 +456,7 @@ def main():
         fm_dev = torch.from_numpy(wl["fixed_mask"]).to(dev) if mode != "forward" else None
 
         def device_step(seed):
-            out = None
+            outs = []
             for ids, cdev in zip(subs, ctx_dev):
                 if len(subs) > 1 or eng.B != len(ids):
                     eng.set_batch(gn[ids], N)   # the batch plan (edge-tile table) is part of the job when it changes
@@ -438,8 +464,8 @@ def main():
                                     sample_ids=ids)
                 el, dmat, adj = eng.seer_inputs(x, cls)
                 _, bonds = eng.seer_forward(el, dmat, adj, want_logits=False)
-                out = (x, cls, bonds)
-            return out
+                outs.append((x, cls, bonds))
+            return outs
         eng.set_batch(gn[subs[0]], N)
     else:
         if mode != "forward":
@@ -448,7 +474,7 @@ def main():
         def device_step(seed):
             # the multi-GPU product path: size-balanced shards by global id, one launch sequence per rank (CUDA graph
             # replay), results stay on the device, ONE packed NCCL all-gather
-            return P.generate_sharded_engine(eng, gn, N, ctx_all, T_STEPS, 0, seed=seed, max_batch=max_batch)
+            return [P.generate_sharded_engine(eng, gn, N, ctx_all, T_STEPS, 0, seed=seed, max_batch=max_batch)]
 
     def sync():
         if world > 1:
@@ -463,12 +489,16 @@ def main():
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     e0.record()
     for i in range(args.steps):
-        device_step(200 + i)
+        outs = device_step(200 + i)
     e1.record()
     sync()
     ms = e0.elapsed_time(e1) / args.steps
     launches = eng.kernel_launches() - l0
     clocks = sampler.stop() if sampler else None
+    if args.dump_outputs and rank == 0:
+        # sub-batches are consecutive ranges of the global ids; the multi-GPU path returns the gathered job in id order
+        dump_outputs(args.dump_outputs, *(torch.cat(t) for t in zip(*outs)))
+    del outs
 
     # ---- end to end: host buffers in, pinned host buffers out, copies inside the timed region -----------------------
     e2e_ms = float("nan")

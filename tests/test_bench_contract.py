@@ -56,3 +56,38 @@ def test_committed_bench_lines_follow_contract():
         if d["n_gpus"] == 1 and "cpu_baseline" in d:
             b = d["cpu_baseline"]
             assert b["kind"] in ("reference", "port") and b["cores"] >= 1 and b["unit"] == "mols/s" and b["value"] > 0
+
+
+def test_dump_outputs_writes_float_arrays_within_budget(tmp_path):
+    """--dump-outputs: every array is float32 / float64, all of them together fit DUMP_BYTES, and a job larger than that is
+    written as the same seeded sample of molecules on every run."""
+    import numpy as np
+    import torch
+    import bench
+    g = torch.Generator().manual_seed(0)
+    for B, whole in ((20, True), (9000, False)):
+        x = torch.randn(B, 39, 3, generator=g)
+        cls = torch.randint(-1, 7, (B, 39), generator=g, dtype=torch.int32)
+        bonds = torch.randint(0, 5, (B, 42, 42), generator=g).to(torch.int8)
+        runs = []
+        for k in range(2):
+            d = tmp_path / ("%d_%d" % (B, k))
+            bench.dump_outputs(str(d), x, cls, bonds)
+            out = {p.stem: np.load(p) for p in d.glob("*.npy")}
+            assert sorted(out) == ["atom_class", "bond_orders", "sample_id", "x"]
+            assert all(a.dtype in (np.float32, np.float64) for a in out.values())
+            assert sum(p.stat().st_size for p in d.glob("*.npy")) <= bench.DUMP_BYTES
+            ids = out["sample_id"].astype(np.int64)
+            assert np.array_equal(out["sample_id"], ids) and np.all(np.diff(ids) > 0)
+            assert (len(ids) == B) == whole and np.array_equal(ids, np.arange(B)) == whole
+            assert np.array_equal(out["x"], x.numpy()[ids]) and np.array_equal(out["atom_class"], cls.numpy()[ids])
+            assert np.array_equal(out["bond_orders"], bonds.numpy()[ids])
+            runs.append(ids)
+        assert np.array_equal(runs[0], runs[1])
+
+
+def test_bench_rejects_arguments_it_cannot_honour():
+    for extra in (["--steps", "0"], ["--impl", "reference", "--dump-outputs", "out"]):
+        out = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py")] + extra, capture_output=True, text=True,
+                             timeout=300, cwd=ROOT)
+        assert out.returncode == 2 and "error" in out.stderr, (extra, out.stderr[-500:])

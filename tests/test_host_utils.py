@@ -5,7 +5,7 @@ import numpy as np
 import pytest
 import torch
 
-from conftest import golden
+from conftest import GOLDEN, golden
 from ml_conformer_generator_b200 import mol_utils as M
 from ml_conformer_generator_b200.config import CONTEXT_NORMS
 
@@ -79,12 +79,13 @@ def test_prepare_fragment_and_symbols():
         M.symbols_to_one_hot(["Si"])
 
 
-@pytest.mark.skipif(not os.path.isdir("/root/reference/assets/demo_files"), reason="reference assets not present")
 def test_v2000_reader_on_reference_assets():
+    """The heavy-atom rows of the reference's demo molfiles ceyyag.mol and yibfeu.mol, stored under tests/golden/, read
+    back to the coordinates and context the reference computed from the originals."""
     g = golden("host_utils")
-    sym, xyz = M.read_mol_heavy_atoms("/root/reference/assets/demo_files/ceyyag.mol")
-    assert len(sym) == 17 and np.allclose(xyz.numpy(), g["ceyyag_xyz"])
-    ctx, n, _ = M.reference_context_from_mol_file("/root/reference/assets/demo_files/yibfeu.mol")
+    sym, xyz = M.read_mol_heavy_atoms(os.path.join(GOLDEN, "ceyyag.mol"))
+    assert len(sym) == 17 and sym == [str(s) for s in g["ceyyag_symbols"]] and np.allclose(xyz.numpy(), g["ceyyag_xyz"])
+    ctx, n, _ = M.reference_context_from_mol_file(os.path.join(GOLDEN, "yibfeu.mol"))
     assert n == 23 and np.allclose(ctx.numpy(), g["yibfeu_context"], rtol=1e-5)
 
 
