@@ -9,7 +9,7 @@
  *  - plain pointers and sizes only; no torch types.  Unless a parameter says "host", pointers are DEVICE pointers
  *    owned by the caller; the library never frees caller memory.
  *  - every call enqueues its work on `stream` (a cudaStream_t passed as void*) and returns without synchronising,
- *    except mlcg_generate / mlcg_load_* / mlcg_set_batch which are synchronous.
+ *    except mlcg_generate / mlcg_generate_fragment / mlcg_load_* / mlcg_set_batch which are synchronous.
  *  - return value: 0 = ok, < 0 = argument / state error (see mlcg_last_error), > 0 = cudaError_t.
  *  - one handle per (device, stream); a handle is thread-compatible, not thread-safe.
  *  - layouts are the reference's: z / eps / noise are (B, N, 11) float32 row-major with N = the call's max_n_nodes
@@ -154,6 +154,42 @@ int mlcg_generate(mlcg_handle* h, const int32_t* n_nodes_host, int B, int N, con
                   const mlcg_step_scalars* steps, int resample_steps, float sigma_0, float alpha_0, float sigma_x,
                   uint64_t seed, int64_t sample_offset, const int64_t* sample_ids_host, float* x_out,
                   int32_t* atom_class_out, int8_t* bonds_out, void* stream);
+
+/* The fixed fragment of mlcg_generate_fragment (the reference's `fixed_fragment=`; one fragment per call).  All HOST
+ * pointers. */
+typedef struct {
+  int mode;                          /* 1 = inpainting (EquivariantDiffusion.inpaint, equivariant_diffusion.py:423-513);
+                                        2 = inertial fragment matching (inertial_fragment_matching=True, the reference's
+                                        default; conformer_generator.py:178-236): a forward loop on the n - n_ff atoms still
+                                        to be generated (padded to N - n_ff), the mlcg_ifm_merge_inputs step, then the
+                                        merge_fragments loop on the whole molecules */
+  int n_ff;                          /* fixed atoms, 1 <= n_ff < min(n_nodes) */
+  const float* ff_x_host;            /* (n_ff,3) fragment coordinates */
+  const float* ff_h_host;            /* (n_ff,8) raw 0/1 one-hot atom classes */
+  int diffusion_level;               /* mode 2: merge_fragments' diffusion_level */
+  float merge_alpha, merge_sigma;    /* mode 2: alpha / sigma of that level (mlcg_sample's merge_alpha / merge_sigma) */
+  const float* moi_gen_origin_host;  /* mode 2: 3x3, exactly as mlcg_ifm_context takes it */
+  const float* ff_weighted_com_host; /* mode 2: 3, exactly as mlcg_ifm_context takes it */
+  const float* norm_mean_host;       /* mode 2: 3, CONTEXT_NORMS mean */
+  const float* norm_mad_host;        /* mode 2: 3, CONTEXT_NORMS mad */
+} mlcg_fragment;
+
+/* Fragment-conditioned counterpart of mlcg_generate: same inputs, outputs, synchronous behaviour and CUDA-graph replay
+ * (from the second call with the same key on), plus the fragment.  ctx_host (B,3) is the normalised reference context
+ * of every sample.  The device sequence is the eager composition of MLConformerGenerator.edm_sample_tensors followed by
+ * the GCN -- mode 1: z_known / fixed_mask from the fragment (prepare_fragment, utils/mol_utils.py:298-342),
+ * mlcg_sample(mode 1); mode 2: mlcg_ifm_context on the whole atom counts, mlcg_sample(mode 0) on the atoms still to be
+ * generated with the context it wrote, mlcg_ifm_merge_inputs, mlcg_sample(mode 2) -- then mlcg_seer_inputs +
+ * mlcg_seer_forward, with the same noise keys and draw numbers; the results equal that composition bit for bit.  The
+ * fragment, context, sample ids and {seed, sample_offset} are uploaded on every call, so a replay never sees a previous
+ * call's inputs; a different mode-2 prologue (another fragment or reference context) is a new key.  A call of
+ * mlcg_generate and one of mlcg_generate_fragment invalidate each other's graph.  Returns MLCG_E_ARG for a mode other
+ * than 1 or 2, n_ff < 1, n_ff >= min(n_nodes), N - n_ff < 1, a null pointer or weights not loaded. */
+int mlcg_generate_fragment(mlcg_handle* h, const mlcg_fragment* frag, const int32_t* n_nodes_host, int B, int N,
+                           const float* ctx_host, int T, const mlcg_step_scalars* steps, int resample_steps, float sigma_0,
+                           float alpha_0, float sigma_x, uint64_t seed, int64_t sample_offset,
+                           const int64_t* sample_ids_host, float* x_out, int32_t* atom_class_out, int8_t* bonds_out,
+                           void* stream);
 
 /* ---- Inertial fragment matching (the default fragment mode) between the two reverse loops ---------------------------
  * Replaces: ifm_prepare_gen_fragment_context (utils/mol_utils.py:373-457) after its batch-independent prologue.  The

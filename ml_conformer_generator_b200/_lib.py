@@ -20,6 +20,7 @@ EXPORTS = [
     "mlcg_num_edges", "mlcg_kernel_launches", "mlcg_time_edge_kernel", "mlcg_edge_phase_profile", "mlcg_test_gemm",
     "mlcg_shape_moments", "mlcg_shape_tanimoto", "mlcg_gemm_phase_profile", "mlcg_plan_edge_tiles",
     "mlcg_egnn_forward_breakdown", "mlcg_ifm_context", "mlcg_ifm_merge_inputs", "mlcg_nonfinite", "mlcg_edge_block_order",
+    "mlcg_generate_fragment",
 ]
 
 
@@ -35,6 +36,13 @@ class Noise(C.Structure):
 class StepScalars(C.Structure):
     _fields_ = [("t", C.c_float), ("alpha_ts", C.c_float), ("c_eps", C.c_float), ("c_sigma", C.c_float),
                 ("alpha_s", C.c_float), ("sigma_s", C.c_float), ("blend", C.c_float)]
+
+
+class Fragment(C.Structure):
+    _fields_ = [("mode", C.c_int), ("n_ff", C.c_int), ("ff_x_host", C.c_void_p), ("ff_h_host", C.c_void_p),
+                ("diffusion_level", C.c_int), ("merge_alpha", C.c_float), ("merge_sigma", C.c_float),
+                ("moi_gen_origin_host", C.c_void_p), ("ff_weighted_com_host", C.c_void_p), ("norm_mean_host", C.c_void_p),
+                ("norm_mad_host", C.c_void_p)]
 
 
 STAMP_PATH = LIB_PATH + ".stamp"
@@ -108,6 +116,8 @@ def load() -> C.CDLL:
     lib.mlcg_seer_forward.argtypes = [vp, vp, vp, vp, vp, vp, ci, vp]
     lib.mlcg_generate.argtypes = [vp, vp, ci, ci, vp, ci, C.POINTER(StepScalars), ci, cf, cf, cf, C.c_uint64,
                                   C.c_int64, vp, vp, vp, vp, vp]
+    lib.mlcg_generate_fragment.argtypes = [vp, C.POINTER(Fragment), vp, ci, ci, vp, ci, C.POINTER(StepScalars), ci, cf, cf,
+                                           cf, C.c_uint64, C.c_int64, vp, vp, vp, vp, vp]
     lib.mlcg_nonfinite.argtypes = [vp, vp]
     lib.mlcg_num_edge_tiles.argtypes = [vp]
     lib.mlcg_num_edges.argtypes = [vp]

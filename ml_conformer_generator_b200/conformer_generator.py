@@ -201,23 +201,31 @@ class MLConformerGenerator:
         return samples_to_sdf_blocks(t["x"], t["atom_class"], t["bonds"], t["n_nodes"])
 
     def generate_stream(self, reference_context: torch.Tensor, n_atoms: int, n_samples: int, batch_size: int = 8192,
-                        variance: int = 2, postprocess=None, n_workers: int = 8, seed: int = 0):
+                        variance: int = 2, postprocess=None, n_workers: int = 8, seed: int = 0,
+                        fixed_fragment: Optional[Tuple[torch.Tensor, torch.Tensor]] = None,
+                        inertial_fragment_matching: bool = True, blend_power: int = 3, ifm_diffusion_level: int = 50):
         """Generates `n_samples` molecules in batches and post-processes batch k on a pool of CPU threads WHILE the GPU
         generates batch k + 1 (SURVEY.md 8f-3; `pipeline.GenerationPipeline`).  `postprocess(x (n,3), atom_class (n,),
         bonds (42,42), n, index)` -> result or None runs once per molecule; the default writes an RDKit-free V2000 block
         (provisional bond orders, see generate_tensors) -- where RDKit is installed pass a callable that builds the Mol and
-        runs the reference's redefine_bonds + standardize_mol.  Yields one list of results per batch, in order."""
+        runs the reference's redefine_bonds + standardize_mol.  Yields one list of results per batch, in order.
+        `fixed_fragment` and the IFM arguments are those of edm_sample_tensors (Engine.generate_fragment_host)."""
         import numpy as np
 
+        from .mol_utils import _check_fragment_size
         from .pipeline import GenerationPipeline, engine_batches, sdf_postprocess
         lo, hi = max(n_atoms - variance, self.min_n_nodes), min(n_atoms + variance, self.max_n_nodes)
+        if fixed_fragment is not None:
+            _check_fragment_size(int(fixed_fragment[0].size(0)), lo, hi)
         g = torch.Generator().manual_seed(seed)
         sizes = torch.randint(lo, hi + 1, (n_samples,), generator=g).numpy().astype(np.int32)   # as prepare_edm_input
         ctx = normalise_context(reference_context, self.context_norms).numpy().reshape(1, 3)
         nn = [sizes[s:s + batch_size] for s in range(0, n_samples, batch_size)]
         cx = [np.tile(ctx, (len(b), 1)).astype(np.float32) for b in nn]
-        pipe = GenerationPipeline(engine_batches(self.engine, nn, hi, cx, self.generative_model.T, seed),
-                                  postprocess or sdf_postprocess, n_workers=n_workers)
+        gen = engine_batches(self.engine, nn, hi, cx, self.generative_model.T, seed, fixed_fragment,
+                             inertial_fragment_matching, reference_context, self.context_norms, blend_power,
+                             ifm_diffusion_level)
+        pipe = GenerationPipeline(gen, postprocess or sdf_postprocess, n_workers=n_workers)
         yield from pipe.run(len(nn))
 
     # ------------------------------------------------------------------------------------------------------------

@@ -1,6 +1,7 @@
 // C-ABI of libmlcg_b200.so (see include/mlcg.h).  Host-side orchestration only: weight repacking at load time, batch
 // plan (edge-tile table), kernel sequencing of one EGNN forward / the reverse-diffusion loop / the AdjMatSeer GCN.
 #include <algorithm>
+#include <cstddef>
 #include <cstdlib>
 #include <cstring>
 #include <map>
@@ -62,6 +63,22 @@ struct SeerLayer {
 
 struct SimtChunk { int node_begin, node_end, edge_base, edge_rows; };
 
+// Batch plan: the geometry of one batch (atom counts, edge-tile table, split targets) and its device copies.  The kernels
+// read the handle's active plan; the workspaces they write are shared by all plans and sized to the largest.
+struct BatchPlan {
+  int B = 0, N = 0, M = 0, n_mtiles = 0, n_etiles = 0;
+  long long n_edges = 0;
+  std::vector<int> h_n_nodes, h_node_off;
+  std::vector<SimtChunk> simt_chunks;
+  DevBuf d_n_nodes, d_node_off, d_node_mol, d_node_edge_off, d_tiles, d_fix_node;
+  DevBuf fix_agg, fix_dx;  // side buffers of the split targets: zero between edge-kernel launches
+  int n_fix = 0;           // target nodes whose neighbour list is split over two edge tiles
+  void release() {
+    for (DevBuf* b : {&d_n_nodes, &d_node_off, &d_node_mol, &d_node_edge_off, &d_tiles, &d_fix_node, &fix_agg, &fix_dx})
+      b->release();
+  }
+};
+
 }  // namespace
 
 struct mlcg_handle {
@@ -75,19 +92,18 @@ struct mlcg_handle {
   LayerW layers[27];
   SeerLayer seer_gcn[7];  // gcn1_dm gcn2_dm gcn3_dm gcn1 gcn2 gcn3 gcn4
   SeerLayer seer_resize;
-  // batch plan
-  int B = 0, N = 0, M = 0, n_mtiles = 0, n_etiles = 0;
-  long long n_edges = 0;
-  std::vector<int> h_n_nodes, h_node_off;
-  std::vector<SimtChunk> simt_chunks;
-  DevBuf d_n_nodes, d_node_off, d_node_mol, d_node_edge_off, d_tiles, d_fix_node, fix_agg, fix_dx;
-  int n_fix = 0;  // target nodes whose neighbour list is split over two edge tiles
+  // batch plans: plans[0] is the one mlcg_set_batch builds; mlcg_generate_fragment keeps the geometry of its first loop
+  // (inertial fragment matching: the atoms still to be generated) in plans[1] and switches `pl` between launches
+  BatchPlan plans[2];
+  BatchPlan* pl = &plans[0];
   // EGNN workspaces
   DevBuf x0, xa, xb, h_res, pq, h_op, agg_op, t_op, agg_f32, t_f32, a1, m2, t_dev, eps_dev;
   // seer workspaces
   DevBuf s_ld, s_la, s_rowd, s_rowa, s_x64, s_y_op, s_x, s_emb, s_add, s_raw, s_y_f32;
   // mlcg_generate device buffers
   DevBuf g_ctx, g_z, g_x, g_cls, g_el, g_dist, g_adj, g_bonds, g_ids;
+  // mlcg_generate_fragment device buffers: fragment, z_known / fixed_mask, and the first IFM loop's context and outputs
+  DevBuf f_ffx, f_ffh, f_zk, f_fm, f_ctx, f_shift, f_rot, f_ngen, f_xg, f_clsg;
   DevBuf nf_flag;  // set by k_decode when a generated coordinate is not finite (mlcg_nonfinite)
   std::vector<int64_t> ids_stage;
   // test gemm
@@ -345,24 +361,24 @@ static cudaError_t launch_edge_mode(int mode, bool equiv, const EdgeArgs& a, int
 }
 // second half of an edge layer: completes the targets whose neighbour list is split over two tiles
 static cudaError_t launch_edge_fixup(mlcg_handle* h, int mode, bool equiv, const EdgeArgs& a, cudaStream_t st) {
-  if (h->n_fix == 0) return cudaSuccess;
-  const int* fn = h->d_fix_node.as<int>();
+  if (h->pl->n_fix == 0) return cudaSuccess;
+  const int* fn = h->pl->d_fix_node.as<int>();
   if (equiv) {
-    const int grid = (h->n_fix * 4 + 127) / 128;
+    const int grid = (h->pl->n_fix * 4 + 127) / 128;
     if (is16(mode))  // the coordinate fix-up does not depend on the operand format
-      k_edge_fixup<PREC_BF16, true><<<grid, 128, 0, st>>>(fn, h->n_fix, a.fix_agg, a.fix_dx, a.agg_op, a.agg_chunks, a.x_cur, a.x_next);
+      k_edge_fixup<PREC_BF16, true><<<grid, 128, 0, st>>>(fn, h->pl->n_fix, a.fix_agg, a.fix_dx, a.agg_op, a.agg_chunks, a.x_cur, a.x_next);
     else
-      k_edge_fixup<PREC_TF32, true><<<grid, 128, 0, st>>>(fn, h->n_fix, a.fix_agg, a.fix_dx, a.agg_op, a.agg_chunks, a.x_cur, a.x_next);
+      k_edge_fixup<PREC_TF32, true><<<grid, 128, 0, st>>>(fn, h->pl->n_fix, a.fix_agg, a.fix_dx, a.agg_op, a.agg_chunks, a.x_cur, a.x_next);
   } else {
     if (mode == PREC_FP16) {
-      const int grid = (h->n_fix * (HP / epp(PREC_FP16)) + 127) / 128;
-      k_edge_fixup<PREC_FP16, false><<<grid, 128, 0, st>>>(fn, h->n_fix, a.fix_agg, a.fix_dx, a.agg_op, a.agg_chunks, a.x_cur, a.x_next);
+      const int grid = (h->pl->n_fix * (HP / epp(PREC_FP16)) + 127) / 128;
+      k_edge_fixup<PREC_FP16, false><<<grid, 128, 0, st>>>(fn, h->pl->n_fix, a.fix_agg, a.fix_dx, a.agg_op, a.agg_chunks, a.x_cur, a.x_next);
     } else if (mode == PREC_BF16) {
-      const int grid = (h->n_fix * (HP / epp(PREC_BF16)) + 127) / 128;
-      k_edge_fixup<PREC_BF16, false><<<grid, 128, 0, st>>>(fn, h->n_fix, a.fix_agg, a.fix_dx, a.agg_op, a.agg_chunks, a.x_cur, a.x_next);
+      const int grid = (h->pl->n_fix * (HP / epp(PREC_BF16)) + 127) / 128;
+      k_edge_fixup<PREC_BF16, false><<<grid, 128, 0, st>>>(fn, h->pl->n_fix, a.fix_agg, a.fix_dx, a.agg_op, a.agg_chunks, a.x_cur, a.x_next);
     } else {
-      const int grid = (h->n_fix * (HP / epp(PREC_TF32)) + 127) / 128;
-      k_edge_fixup<PREC_TF32, false><<<grid, 128, 0, st>>>(fn, h->n_fix, a.fix_agg, a.fix_dx, a.agg_op, a.agg_chunks, a.x_cur, a.x_next);
+      const int grid = (h->pl->n_fix * (HP / epp(PREC_TF32)) + 127) / 128;
+      k_edge_fixup<PREC_TF32, false><<<grid, 128, 0, st>>>(fn, h->pl->n_fix, a.fix_agg, a.fix_dx, a.agg_op, a.agg_chunks, a.x_cur, a.x_next);
     }
   }
   h->launches++;
@@ -427,11 +443,13 @@ extern "C" void mlcg_destroy(mlcg_handle* h) {
   if (h->gen_graph) cudaGraphExecDestroy(h->gen_graph);
   if (h->own_stream) cudaStreamDestroy(h->own_stream);
   h->noise_ctl.release();
-  for (DevBuf* b : {&h->d_n_nodes, &h->d_node_off, &h->d_node_mol, &h->d_node_edge_off, &h->d_tiles, &h->d_fix_node, &h->fix_agg, &h->fix_dx, &h->x0, &h->xa, &h->xb,
+  for (BatchPlan& p : h->plans) p.release();
+  for (DevBuf* b : {&h->x0, &h->xa, &h->xb,
                     &h->h_res, &h->pq, &h->h_op, &h->agg_op, &h->t_op, &h->agg_f32, &h->t_f32, &h->a1, &h->m2, &h->t_dev,
                     &h->eps_dev, &h->s_ld, &h->s_la, &h->s_rowd, &h->s_rowa, &h->s_x64, &h->s_y_op, &h->s_x, &h->s_emb,
                     &h->s_add, &h->s_raw, &h->s_y_f32, &h->g_ctx, &h->g_z, &h->g_x, &h->g_cls, &h->g_el, &h->g_dist,
-                    &h->g_adj, &h->g_bonds, &h->g_ids, &h->nf_flag, &h->tg_a, &h->tg_w, &h->tg_b, &h->tg_c})
+                    &h->g_adj, &h->g_bonds, &h->g_ids, &h->f_ffx, &h->f_ffh, &h->f_zk, &h->f_fm, &h->f_ctx, &h->f_shift,
+                    &h->f_rot, &h->f_ngen, &h->f_xg, &h->f_clsg, &h->nf_flag, &h->tg_a, &h->tg_w, &h->tg_b, &h->tg_c})
     b->release();
   delete h;
 }
@@ -702,28 +720,19 @@ extern "C" int mlcg_plan_edge_tiles(const int32_t* n_nodes, int B, int N, int nu
   return (int)tiles.size();
 }
 
-extern "C" int mlcg_set_batch(mlcg_handle* h, const int32_t* n_nodes, int B, int N) {
-  if (!h) return MLCG_E_ARG;
-  if (!n_nodes || B <= 0 || N <= 0 || N > EDGE_MAXN) FAIL(MLCG_E_ARG, "set_batch: need B > 0 and 1 <= N <= 39");
-  CK(cudaSetDevice(h->device));
-  // The plan buffers below are rewritten with synchronous copies on the NULL stream while earlier calls may still be
-  // running on the caller's (possibly non-blocking) streams: drain the device first.  set_batch is documented synchronous.
-  CK(cudaDeviceSynchronize());
-  // any change of the batch plan invalidates the graph captured by mlcg_generate
-  if (h->gen_graph) { cudaGraphExecDestroy(h->gen_graph); h->gen_graph = nullptr; }
-  h->gen_key.clear();
-  h->gen_key_hits = 0;
-  h->batch_set = false;
-  h->B = B;
-  h->N = N;
-  h->h_n_nodes.assign(n_nodes, n_nodes + B);
-  h->h_node_off.assign(B + 1, 0);
+// Builds plan `p` for a batch (n_nodes HOST, 1 <= n_nodes[b] <= N) and grows the shared workspaces to fit it.  Synchronous
+// copies on the NULL stream: the caller drains the device first and never calls it inside a stream capture.
+static int build_plan(mlcg_handle* h, BatchPlan& p, const int32_t* n_nodes, int B, int N) {
+  p.B = B;
+  p.N = N;
+  p.h_n_nodes.assign(n_nodes, n_nodes + B);
+  p.h_node_off.assign(B + 1, 0);
   std::vector<int> node_mol, node_edge_off;
   std::vector<EdgeTile> tiles;
   std::vector<int> fix_node;
   {
     std::string perr;
-    const int prc = plan_edge_tiles(n_nodes, B, N, h->num_sms, tiles, fix_node, h->h_node_off, perr);
+    const int prc = plan_edge_tiles(n_nodes, B, N, h->num_sms, tiles, fix_node, p.h_node_off, perr);
     if (prc) FAIL(prc, perr.c_str());
   }
   long long edges = 0;
@@ -736,30 +745,30 @@ extern "C" int mlcg_set_batch(mlcg_handle* h, const int32_t* n_nodes, int B, int
     }
     edges += (long long)n * (n - 1);
   }
-  h->n_etiles = (int)tiles.size();
-  h->n_edges = edges;
-  h->M = h->h_node_off[B];
-  h->n_mtiles = (h->M + TILE_M - 1) / TILE_M;
-  h->n_etiles = (int)tiles.size();
-  const size_t mpad = (size_t)h->n_mtiles * TILE_M;
-  CK(h->d_n_nodes.ensure(B * sizeof(int)));
-  CK(h->d_node_off.ensure((B + 1) * sizeof(int)));
-  CK(h->d_node_mol.ensure(h->M * sizeof(int)));
-  CK(h->d_node_edge_off.ensure(h->M * sizeof(int)));
-  CK(h->d_tiles.ensure(tiles.size() * sizeof(EdgeTile)));
-  h->n_fix = (int)fix_node.size();
-  CK(h->d_fix_node.ensure(std::max<size_t>(fix_node.size(), 1) * sizeof(int)));
-  CK(h->fix_agg.ensure(std::max<size_t>(fix_node.size(), 1) * HP * sizeof(float)));
-  CK(h->fix_dx.ensure(std::max<size_t>(fix_node.size(), 1) * 4 * sizeof(float)));
-  CK(cudaMemcpy(h->d_n_nodes.p, n_nodes, B * sizeof(int), cudaMemcpyHostToDevice));
-  CK(cudaMemcpy(h->d_node_off.p, h->h_node_off.data(), (B + 1) * sizeof(int), cudaMemcpyHostToDevice));
-  CK(cudaMemcpy(h->d_node_mol.p, node_mol.data(), h->M * sizeof(int), cudaMemcpyHostToDevice));
-  CK(cudaMemcpy(h->d_node_edge_off.p, node_edge_off.data(), h->M * sizeof(int), cudaMemcpyHostToDevice));
-  CK(cudaMemcpy(h->d_tiles.p, tiles.data(), tiles.size() * sizeof(EdgeTile), cudaMemcpyHostToDevice));
-  if (h->n_fix) CK(cudaMemcpy(h->d_fix_node.p, fix_node.data(), fix_node.size() * sizeof(int), cudaMemcpyHostToDevice));
+  p.n_etiles = (int)tiles.size();
+  p.n_edges = edges;
+  p.M = p.h_node_off[B];
+  p.n_mtiles = (p.M + TILE_M - 1) / TILE_M;
+  p.n_etiles = (int)tiles.size();
+  const size_t mpad = (size_t)p.n_mtiles * TILE_M;
+  CK(p.d_n_nodes.ensure(B * sizeof(int)));
+  CK(p.d_node_off.ensure((B + 1) * sizeof(int)));
+  CK(p.d_node_mol.ensure(p.M * sizeof(int)));
+  CK(p.d_node_edge_off.ensure(p.M * sizeof(int)));
+  CK(p.d_tiles.ensure(tiles.size() * sizeof(EdgeTile)));
+  p.n_fix = (int)fix_node.size();
+  CK(p.d_fix_node.ensure(std::max<size_t>(fix_node.size(), 1) * sizeof(int)));
+  CK(p.fix_agg.ensure(std::max<size_t>(fix_node.size(), 1) * HP * sizeof(float)));
+  CK(p.fix_dx.ensure(std::max<size_t>(fix_node.size(), 1) * 4 * sizeof(float)));
+  CK(cudaMemcpy(p.d_n_nodes.p, n_nodes, B * sizeof(int), cudaMemcpyHostToDevice));
+  CK(cudaMemcpy(p.d_node_off.p, p.h_node_off.data(), (B + 1) * sizeof(int), cudaMemcpyHostToDevice));
+  CK(cudaMemcpy(p.d_node_mol.p, node_mol.data(), p.M * sizeof(int), cudaMemcpyHostToDevice));
+  CK(cudaMemcpy(p.d_node_edge_off.p, node_edge_off.data(), p.M * sizeof(int), cudaMemcpyHostToDevice));
+  CK(cudaMemcpy(p.d_tiles.p, tiles.data(), tiles.size() * sizeof(EdgeTile), cudaMemcpyHostToDevice));
+  if (p.n_fix) CK(cudaMemcpy(p.d_fix_node.p, fix_node.data(), fix_node.size() * sizeof(int), cudaMemcpyHostToDevice));
   // the side buffers of split targets are zero between edge-kernel launches (k_edge_fixup re-zeroes what it consumes)
-  CK(cudaMemset(h->fix_agg.p, 0, std::max<size_t>(fix_node.size(), 1) * HP * sizeof(float)));
-  CK(cudaMemset(h->fix_dx.p, 0, std::max<size_t>(fix_node.size(), 1) * 4 * sizeof(float)));
+  CK(cudaMemset(p.fix_agg.p, 0, std::max<size_t>(fix_node.size(), 1) * HP * sizeof(float)));
+  CK(cudaMemset(p.fix_dx.p, 0, std::max<size_t>(fix_node.size(), 1) * 4 * sizeof(float)));
   // workspaces (zero-initialised on growth; padded rows / columns are never written afterwards)
   CK(h->x0.ensure(mpad * 3 * sizeof(float)));
   CK(h->xa.ensure(mpad * 3 * sizeof(float)));
@@ -774,28 +783,46 @@ extern "C" int mlcg_set_batch(mlcg_handle* h, const int32_t* n_nodes, int B, int
     CK(h->t_f32.ensure(mpad * HP * sizeof(float)));
     // chunk the edge list so the materialised edge activations stay bounded
     const int cap = 49152;
-    h->simt_chunks.clear();
+    p.simt_chunks.clear();
     int nb = 0;
-    while (nb < h->M) {
+    while (nb < p.M) {
       SimtChunk c{nb, nb, node_edge_off[nb], 0};
-      while (c.node_end < h->M) {
+      while (c.node_end < p.M) {
         const int b = node_mol[c.node_end];
         const int deg = n_nodes[b] - 1;
         if (c.edge_rows + deg > cap && c.edge_rows > 0) break;
         c.edge_rows += deg;
         c.node_end++;
       }
-      h->simt_chunks.push_back(c);
+      p.simt_chunks.push_back(c);
       nb = c.node_end;
     }
     CK(h->a1.ensure((size_t)(cap + 64) * HP * sizeof(float)));
     CK(h->m2.ensure((size_t)(cap + 64) * HP * sizeof(float)));
   } else {
-    const size_t opb = (size_t)h->n_mtiles * h->kc448() * A_CHUNK_BYTES;
+    const size_t opb = (size_t)p.n_mtiles * h->kc448() * A_CHUNK_BYTES;
     CK(h->h_op.ensure(opb));
     CK(h->agg_op.ensure(opb));
     CK(h->t_op.ensure(opb));
   }
+  return MLCG_OK;
+}
+
+extern "C" int mlcg_set_batch(mlcg_handle* h, const int32_t* n_nodes, int B, int N) {
+  if (!h) return MLCG_E_ARG;
+  if (!n_nodes || B <= 0 || N <= 0 || N > EDGE_MAXN) FAIL(MLCG_E_ARG, "set_batch: need B > 0 and 1 <= N <= 39");
+  CK(cudaSetDevice(h->device));
+  // The plan buffers below are rewritten with synchronous copies on the NULL stream while earlier calls may still be
+  // running on the caller's (possibly non-blocking) streams: drain the device first.  set_batch is documented synchronous.
+  CK(cudaDeviceSynchronize());
+  // any change of the batch plan invalidates the graph captured by mlcg_generate / mlcg_generate_fragment
+  if (h->gen_graph) { cudaGraphExecDestroy(h->gen_graph); h->gen_graph = nullptr; }
+  h->gen_key.clear();
+  h->gen_key_hits = 0;
+  h->batch_set = false;
+  h->pl = &h->plans[0];
+  const int rc = build_plan(h, h->plans[0], n_nodes, B, N);
+  if (rc) return rc;
   h->batch_set = true;
   return MLCG_OK;
 }
@@ -810,22 +837,22 @@ extern "C" int mlcg_nonfinite(mlcg_handle* h, void* stream) {
   if (v) cudaMemset(h->nf_flag.p, 0, sizeof(int));
   return v != 0;
 }
-extern "C" int mlcg_num_edge_tiles(mlcg_handle* h) { return h ? h->n_etiles : -1; }
-extern "C" int64_t mlcg_num_edges(mlcg_handle* h) { return h ? h->n_edges : -1; }
+extern "C" int mlcg_num_edge_tiles(mlcg_handle* h) { return h ? h->pl->n_etiles : -1; }
+extern "C" int64_t mlcg_num_edges(mlcg_handle* h) { return h ? h->pl->n_edges : -1; }
 extern "C" int64_t mlcg_kernel_launches(mlcg_handle* h) { return h ? h->launches : -1; }
 
 // ---------------------------------------------------------------------------------------------------------------
 // EGNN forward
 // ---------------------------------------------------------------------------------------------------------------
-static int edge_grid(mlcg_handle* h) { return edge_grid_for(h->n_etiles, h->num_sms); }
+static int edge_grid(mlcg_handle* h) { return edge_grid_for(h->pl->n_etiles, h->num_sms); }
 
 static EdgeArgs edge_args(mlcg_handle* h, const LayerW& L, const float* x_cur, float* x_next) {
   EdgeArgs a{};
-  a.tiles = h->d_tiles.as<int4>();
-  a.n_tiles = h->n_etiles;
-  a.fix_agg = h->fix_agg.as<float>();
-  a.fix_dx = h->fix_dx.as<float>();
-  a.node_off = h->d_node_off.as<int>();
+  a.tiles = h->pl->d_tiles.as<int4>();
+  a.n_tiles = h->pl->n_etiles;
+  a.fix_agg = h->pl->fix_agg.as<float>();
+  a.fix_dx = h->pl->fix_dx.as<float>();
+  a.node_off = h->pl->d_node_off.as<int>();
   a.pq = h->pq.p;
   a.x_cur = x_cur;
   a.x0 = h->x0.as<float>();
@@ -868,13 +895,13 @@ static int egnn_forward_tc(mlcg_handle* h, cudaStream_t st) {
   auto gemm_pq = [&](const LayerW& L) -> cudaError_t {
     GemmArgs a{};
     a.a0 = h->h_op.as<uint8_t>(); a.a0_chunks = kc; a.a0_per_tile = kc; a.n_kc = kc;
-    a.w = L.w1ab_op.as<uint8_t>(); a.bias = L.bias_pq.as<float>(); a.m_rows = h->M;
+    a.w = L.w1ab_op.as<uint8_t>(); a.bias = L.bias_pq.as<float>(); a.m_rows = h->pl->M;
     a.out_f32 = h->pq.as<float>(); a.ldo = 2 * HP; a.n_valid = 2 * HP; a.rowscale = nullptr; a.relu = 0;
     // bf16 mode keeps the P/Q projections in bf16 (halves their HBM and shared-memory traffic; no accuracy cost)
     a.out_scale = act_scale(mode);  // fp16: P/Q rows are stored scaled by ACT
-    if (mode == PREC_FP16) return launch_gemm<PREC_FP16, HP, EPI_BF16>(a, h->n_mtiles, 2, st);
-    if (mode == PREC_BF16) return launch_gemm<PREC_BF16, HP, EPI_BF16>(a, h->n_mtiles, 2, st);
-    return launch_gemm<PREC_TF32, HP, EPI_F32>(a, h->n_mtiles, 2, st);
+    if (mode == PREC_FP16) return launch_gemm<PREC_FP16, HP, EPI_BF16>(a, h->pl->n_mtiles, 2, st);
+    if (mode == PREC_BF16) return launch_gemm<PREC_BF16, HP, EPI_BF16>(a, h->pl->n_mtiles, 2, st);
+    return launch_gemm<PREC_TF32, HP, EPI_F32>(a, h->pl->n_mtiles, 2, st);
   };
   float* xa = h->xa.as<float>();
   float* xb = h->xb.as<float>();
@@ -896,17 +923,17 @@ static int egnn_forward_tc(mlcg_handle* h, cudaStream_t st) {
       GemmArgs a{};
       a.a0 = h->h_op.as<uint8_t>(); a.a0_chunks = kc; a.a0_per_tile = kc;
       a.a1 = h->agg_op.as<uint8_t>(); a.a1_per_tile = kc; a.n_kc = 2 * kc;
-      a.w = L.w3_op.as<uint8_t>(); a.bias = L.b3p.as<float>(); a.m_rows = h->M;
+      a.w = L.w3_op.as<uint8_t>(); a.bias = L.b3p.as<float>(); a.m_rows = h->pl->M;
       a.out_op = h->t_op.as<uint8_t>(); a.out_op_chunks = kc; a.out_scale = op_scale(mode);
-      CK((launch_gemm_mode<HP, EPI_SILU_OP>(mode, a, h->n_mtiles, 1, st)));
+      CK((launch_gemm_mode<HP, EPI_SILU_OP>(mode, a, h->pl->n_mtiles, 1, st)));
       h->launches++;
       bd_mark(h, BD_MLP1, st);
       GemmArgs b{};
       b.a0 = h->t_op.as<uint8_t>(); b.a0_chunks = kc; b.a0_per_tile = kc; b.n_kc = kc;
-      b.w = L.w4_op.as<uint8_t>(); b.bias = L.b4p.as<float>(); b.m_rows = h->M;
+      b.w = L.w4_op.as<uint8_t>(); b.bias = L.b4p.as<float>(); b.m_rows = h->pl->M;
       b.out_op = h->h_op.as<uint8_t>(); b.out_op_chunks = kc; b.resid = h->h_res.as<float>(); b.ldr = 0;  // tiled residual layout
       b.out_scale = op_scale(mode);
-      CK((launch_gemm_mode<HP, EPI_RESID_OP>(mode, b, h->n_mtiles, 1, st)));
+      CK((launch_gemm_mode<HP, EPI_RESID_OP>(mode, b, h->pl->n_mtiles, 1, st)));
       h->launches++;
       bd_mark(h, BD_MLP2, st);
     }
@@ -933,9 +960,9 @@ static int egnn_forward_simt(mlcg_handle* h, cudaStream_t st) {
   float* xb = h->xb.as<float>();
   float* hres = h->h_res.as<float>();
   float* pq = h->pq.as<float>();
-  const int* node_mol = h->d_node_mol.as<int>();
-  const int* node_off = h->d_node_off.as<int>();
-  const int* neo = h->d_node_edge_off.as<int>();
+  const int* node_mol = h->pl->d_node_mol.as<int>();
+  const int* node_off = h->pl->d_node_off.as<int>();
+  const int* neo = h->pl->d_node_edge_off.as<int>();
   int rc;
   for (int l = 0; l < 27; ++l) {
     const LayerW& L = h->layers[l];
@@ -943,10 +970,10 @@ static int egnn_forward_simt(mlcg_handle* h, cudaStream_t st) {
     const float* x_cur = (blk & 1) ? xb : xa;
     float* x_next = (blk & 1) ? xa : xb;
     // P = h.W1[:, :420]^T ; Q = h.W1[:, 420:840]^T + b1
-    if ((rc = simt_gemm(h, hres, HP, L.w1.d, 2 * HID + 2, nullptr, pq, 2 * HP, h->M, HID, HID, 0, nullptr, st))) return rc;
-    if ((rc = simt_gemm(h, hres, HP, L.w1.d + HID, 2 * HID + 2, L.b1.d, pq + HP, 2 * HP, h->M, HID, HID, SG_BIAS, nullptr, st)))
+    if ((rc = simt_gemm(h, hres, HP, L.w1.d, 2 * HID + 2, nullptr, pq, 2 * HP, h->pl->M, HID, HID, 0, nullptr, st))) return rc;
+    if ((rc = simt_gemm(h, hres, HP, L.w1.d + HID, 2 * HID + 2, L.b1.d, pq + HP, 2 * HP, h->pl->M, HID, HID, SG_BIAS, nullptr, st)))
       return rc;
-    for (const SimtChunk& c : h->simt_chunks) {
+    for (const SimtChunk& c : h->pl->simt_chunks) {
       const int nn = c.node_end - c.node_begin;
       k_simt_build_a1<<<nn, HP, 0, st>>>(pq, x_cur, h->x0.as<float>(), node_mol, node_off, neo, c.node_begin, c.edge_base,
                                          L.w1.d, h->a1.as<float>());
@@ -964,11 +991,11 @@ static int egnn_forward_simt(mlcg_handle* h, cudaStream_t st) {
     }
     if (!L.equiv) {
       float* t = h->t_f32.as<float>();
-      if ((rc = simt_gemm(h, hres, HP, L.w3.d, 2 * HID, L.b3.d, t, HP, h->M, HID, HID, SG_BIAS, nullptr, st))) return rc;
-      if ((rc = simt_gemm(h, h->agg_f32.as<float>(), HP, L.w3.d + HID, 2 * HID, nullptr, t, HP, h->M, HID, HID,
+      if ((rc = simt_gemm(h, hres, HP, L.w3.d, 2 * HID, L.b3.d, t, HP, h->pl->M, HID, HID, SG_BIAS, nullptr, st))) return rc;
+      if ((rc = simt_gemm(h, h->agg_f32.as<float>(), HP, L.w3.d + HID, 2 * HID, nullptr, t, HP, h->pl->M, HID, HID,
                           SG_ACC | SG_SILU, nullptr, st)))
         return rc;
-      if ((rc = simt_gemm(h, t, HP, L.w4.d, HID, L.b4.d, hres, HP, h->M, HID, HID, SG_BIAS | SG_ACC, nullptr, st))) return rc;
+      if ((rc = simt_gemm(h, t, HP, L.w4.d, HID, L.b4.d, hres, HP, h->pl->M, HID, HID, SG_BIAS | SG_ACC, nullptr, st))) return rc;
     }
   }
   return MLCG_OK;
@@ -982,19 +1009,19 @@ extern "C" int mlcg_egnn_forward(mlcg_handle* h, const float* t, const float* z,
   const int kc = h->kc448();
   bd_mark(h, BD_START, st);
   if (h->precision == PREC_FP16)
-    k_egnn_prepare<PREC_FP16><<<(h->M + PREP_NPB - 1) / PREP_NPB, HP, 0, st>>>(z, t, ctx, h->d_node_mol.as<int>(), h->d_node_off.as<int>(), h->N, h->M, h->w_emb.d,
+    k_egnn_prepare<PREC_FP16><<<(h->pl->M + PREP_NPB - 1) / PREP_NPB, HP, 0, st>>>(z, t, ctx, h->pl->d_node_mol.as<int>(), h->pl->d_node_off.as<int>(), h->pl->N, h->pl->M, h->w_emb.d,
                                                   h->b_emb.d, h->h_res.as<float>(), 0, h->h_op.as<uint8_t>(), kc,
                                                   h->x0.as<float>(), h->xa.as<float>());
   else if (h->precision == PREC_BF16)
-    k_egnn_prepare<PREC_BF16><<<(h->M + PREP_NPB - 1) / PREP_NPB, HP, 0, st>>>(z, t, ctx, h->d_node_mol.as<int>(), h->d_node_off.as<int>(), h->N, h->M, h->w_emb.d,
+    k_egnn_prepare<PREC_BF16><<<(h->pl->M + PREP_NPB - 1) / PREP_NPB, HP, 0, st>>>(z, t, ctx, h->pl->d_node_mol.as<int>(), h->pl->d_node_off.as<int>(), h->pl->N, h->pl->M, h->w_emb.d,
                                                   h->b_emb.d, h->h_res.as<float>(), 0, h->h_op.as<uint8_t>(), kc,
                                                   h->x0.as<float>(), h->xa.as<float>());
   else if (h->precision == PREC_TF32)
-    k_egnn_prepare<PREC_TF32><<<(h->M + PREP_NPB - 1) / PREP_NPB, HP, 0, st>>>(z, t, ctx, h->d_node_mol.as<int>(), h->d_node_off.as<int>(), h->N, h->M, h->w_emb.d,
+    k_egnn_prepare<PREC_TF32><<<(h->pl->M + PREP_NPB - 1) / PREP_NPB, HP, 0, st>>>(z, t, ctx, h->pl->d_node_mol.as<int>(), h->pl->d_node_off.as<int>(), h->pl->N, h->pl->M, h->w_emb.d,
                                                   h->b_emb.d, h->h_res.as<float>(), 0, h->h_op.as<uint8_t>(), kc,
                                                   h->x0.as<float>(), h->xa.as<float>());
   else
-    k_egnn_prepare<PREC_FP32_SIMT><<<(h->M + PREP_NPB - 1) / PREP_NPB, HP, 0, st>>>(z, t, ctx, h->d_node_mol.as<int>(), h->d_node_off.as<int>(), h->N, h->M,
+    k_egnn_prepare<PREC_FP32_SIMT><<<(h->pl->M + PREP_NPB - 1) / PREP_NPB, HP, 0, st>>>(z, t, ctx, h->pl->d_node_mol.as<int>(), h->pl->d_node_off.as<int>(), h->pl->N, h->pl->M,
                                                        h->w_emb.d, h->b_emb.d, h->h_res.as<float>(), HP, nullptr, 0,
                                                        h->x0.as<float>(), h->xa.as<float>());
   KCHECK();
@@ -1002,8 +1029,8 @@ extern "C" int mlcg_egnn_forward(mlcg_handle* h, const float* t, const float* z,
   int rc = (h->precision == PREC_FP32_SIMT) ? egnn_forward_simt(h, st) : egnn_forward_tc(h, st);
   if (rc) return rc;
   // 9 blocks: blocks 0,2,4,6,8 write xb -> final coordinates are in xb
-  k_egnn_readout<<<h->B, 256, 0, st>>>(h->h_res.as<float>(), h->precision == PREC_FP32_SIMT ? HP : 0, h->xb.as<float>(), h->x0.as<float>(), h->d_n_nodes.as<int>(),
-                                       h->d_node_off.as<int>(), h->N, h->w_out.d, h->b_out.d, eps);
+  k_egnn_readout<<<h->pl->B, 256, 0, st>>>(h->h_res.as<float>(), h->precision == PREC_FP32_SIMT ? HP : 0, h->xb.as<float>(), h->x0.as<float>(), h->pl->d_n_nodes.as<int>(),
+                                       h->pl->d_node_off.as<int>(), h->pl->N, h->w_out.d, h->b_out.d, eps);
   KCHECK();
   bd_mark(h, BD_READOUT, st);
   return MLCG_OK;
@@ -1049,7 +1076,7 @@ static inline int warp_grid(int B) { return (B * 32 + 127) / 128; }
 extern "C" int mlcg_noise_init(mlcg_handle* h, float* z, const mlcg_noise* noise, void* stream) {
   STEP_PROLOGUE("noise_init");
   if (!z || !noise) FAIL(MLCG_E_ARG, "noise_init: null pointer");
-  k_noise_init<<<warp_grid(h->B), 128, 0, st>>>(z, h->d_n_nodes.as<int>(), h->B, h->N, to_src(h, noise));
+  k_noise_init<<<warp_grid(h->pl->B), 128, 0, st>>>(z, h->pl->d_n_nodes.as<int>(), h->pl->B, h->pl->N, to_src(h, noise));
   KCHECK();
   return MLCG_OK;
 }
@@ -1057,7 +1084,7 @@ extern "C" int mlcg_step(mlcg_handle* h, float* z, const float* eps, const mlcg_
                          void* stream) {
   STEP_PROLOGUE("step");
   if (!z || !eps || !sc || !noise) FAIL(MLCG_E_ARG, "step: null pointer");
-  k_step<<<warp_grid(h->B), 128, 0, st>>>(z, eps, h->d_n_nodes.as<int>(), h->B, h->N, sc->alpha_ts, sc->c_eps, sc->c_sigma,
+  k_step<<<warp_grid(h->pl->B), 128, 0, st>>>(z, eps, h->pl->d_n_nodes.as<int>(), h->pl->B, h->pl->N, sc->alpha_ts, sc->c_eps, sc->c_sigma,
                                           to_src(h, noise));
   KCHECK();
   return MLCG_OK;
@@ -1066,7 +1093,7 @@ extern "C" int mlcg_reinject(mlcg_handle* h, float* z, const float* z_known, con
                              const mlcg_step_scalars* sc, const mlcg_noise* noise, void* stream) {
   STEP_PROLOGUE("reinject");
   if (!z || !z_known || !fixed_mask || !sc || !noise) FAIL(MLCG_E_ARG, "reinject: null pointer");
-  k_reinject<<<warp_grid(h->B), 128, 0, st>>>(z, z_known, fixed_mask, h->d_n_nodes.as<int>(), h->B, h->N, sc->alpha_s,
+  k_reinject<<<warp_grid(h->pl->B), 128, 0, st>>>(z, z_known, fixed_mask, h->pl->d_n_nodes.as<int>(), h->pl->B, h->pl->N, sc->alpha_s,
                                               sc->sigma_s, sc->blend, to_src(h, noise));
   KCHECK();
   return MLCG_OK;
@@ -1075,7 +1102,7 @@ extern "C" int mlcg_forward_diffuse(mlcg_handle* h, float* z, const float* z_kno
                                     const mlcg_noise* noise, void* stream) {
   STEP_PROLOGUE("forward_diffuse");
   if (!z || !z_known || !noise) FAIL(MLCG_E_ARG, "forward_diffuse: null pointer");
-  k_forward_diffuse<<<warp_grid(h->B), 128, 0, st>>>(z, z_known, h->d_n_nodes.as<int>(), h->B, h->N, alpha, sigma,
+  k_forward_diffuse<<<warp_grid(h->pl->B), 128, 0, st>>>(z, z_known, h->pl->d_n_nodes.as<int>(), h->pl->B, h->pl->N, alpha, sigma,
                                                      to_src(h, noise));
   KCHECK();
   return MLCG_OK;
@@ -1084,7 +1111,7 @@ extern "C" int mlcg_decode(mlcg_handle* h, const float* z0, const float* eps0, f
                            const mlcg_noise* noise, float* x, int32_t* atom_class, void* stream) {
   STEP_PROLOGUE("decode");
   if (!z0 || !eps0 || !noise || !x || !atom_class) FAIL(MLCG_E_ARG, "decode: null pointer");
-  k_decode<<<warp_grid(h->B), 128, 0, st>>>(z0, eps0, h->d_n_nodes.as<int>(), h->B, h->N, sigma_0, alpha_0, sigma_x,
+  k_decode<<<warp_grid(h->pl->B), 128, 0, st>>>(z0, eps0, h->pl->d_n_nodes.as<int>(), h->pl->B, h->pl->N, sigma_0, alpha_0, sigma_x,
                                             to_src(h, noise), x, atom_class, h->nf_flag.as<int>());
   KCHECK();
   return MLCG_OK;
@@ -1093,20 +1120,21 @@ extern "C" int mlcg_decode(mlcg_handle* h, const float* z0, const float* eps0, f
 // ---------------------------------------------------------------------------------------------------------------
 // whole reverse loop
 // ---------------------------------------------------------------------------------------------------------------
-extern "C" int mlcg_sample(mlcg_handle* h, int mode, int T, const mlcg_step_scalars* steps, int resample_steps,
-                           int diffusion_level, float merge_alpha, float merge_sigma, float sigma_0, float alpha_0,
-                           float sigma_x, const float* ctx, const float* z_known, const float* fixed_mask,
-                           const float* noise_tape, uint64_t seed, int64_t sample_offset, const int64_t* sample_ids, float* z,
-                           float* x_out, int32_t* atom_class_out, float* trace_z, float* trace_eps, void* stream) {
+// The reverse loop of mlcg_sample with its noise draws numbered from `draw0` on (mlcg_sample: 0).
+static int sample_loop(mlcg_handle* h, int mode, int T, const mlcg_step_scalars* steps, int resample_steps,
+                       int diffusion_level, float merge_alpha, float merge_sigma, float sigma_0, float alpha_0, float sigma_x,
+                       const float* ctx, const float* z_known, const float* fixed_mask, const float* noise_tape, uint64_t seed,
+                       int64_t sample_offset, const int64_t* sample_ids, float* z, float* x_out, int32_t* atom_class_out,
+                       float* trace_z, float* trace_eps, uint64_t draw0, void* stream) {
   STEP_PROLOGUE("sample");
   if (!h->egnn_loaded) FAIL(MLCG_E_STATE, "sample: load the EGNN weights first");
   if (mode < 0 || mode > 2 || T <= 0 || !steps || !ctx || !z || !x_out || !atom_class_out || resample_steps < 0)
     FAIL(MLCG_E_ARG, "sample: bad argument");
   if (mode != 0 && (!z_known || !fixed_mask)) FAIL(MLCG_E_ARG, "sample: inpaint / merge need z_known and fixed_mask");
-  const size_t zsz = (size_t)h->B * h->N * ZC;
+  const size_t zsz = (size_t)h->pl->B * h->pl->N * ZC;
   float* eps = h->eps_dev.as<float>();
   float* tdev = h->t_dev.as<float>();
-  uint64_t draw = 0;
+  uint64_t draw = draw0;
   long long fwd = 0;
   auto next_noise = [&]() {
     mlcg_noise n;
@@ -1119,7 +1147,7 @@ extern "C" int mlcg_sample(mlcg_handle* h, int mode, int T, const mlcg_step_scal
     return n;
   };
   auto network = [&](float tval) -> int {
-    k_fill_f32<<<(h->B + 127) / 128, 128, 0, st>>>(tdev, tval, h->B);
+    k_fill_f32<<<(h->pl->B + 127) / 128, 128, 0, st>>>(tdev, tval, h->pl->B);
     KCHECK();
     if (trace_z) CK(cudaMemcpyAsync(trace_z + (size_t)fwd * zsz, z, zsz * sizeof(float), cudaMemcpyDeviceToDevice, st));
     int rc = mlcg_egnn_forward(h, tdev, z, ctx, eps, stream);
@@ -1165,6 +1193,16 @@ extern "C" int mlcg_sample(mlcg_handle* h, int mode, int T, const mlcg_step_scal
   return mlcg_decode(h, z, eps, sigma_0, alpha_0, sigma_x, &n, x_out, atom_class_out, stream);
 }
 
+extern "C" int mlcg_sample(mlcg_handle* h, int mode, int T, const mlcg_step_scalars* steps, int resample_steps,
+                           int diffusion_level, float merge_alpha, float merge_sigma, float sigma_0, float alpha_0,
+                           float sigma_x, const float* ctx, const float* z_known, const float* fixed_mask,
+                           const float* noise_tape, uint64_t seed, int64_t sample_offset, const int64_t* sample_ids, float* z,
+                           float* x_out, int32_t* atom_class_out, float* trace_z, float* trace_eps, void* stream) {
+  return sample_loop(h, mode, T, steps, resample_steps, diffusion_level, merge_alpha, merge_sigma, sigma_0, alpha_0, sigma_x,
+                     ctx, z_known, fixed_mask, noise_tape, seed, sample_offset, sample_ids, z, x_out, atom_class_out, trace_z,
+                     trace_eps, 0, stream);
+}
+
 // ---------------------------------------------------------------------------------------------------------------
 // AdjMatSeer
 // ---------------------------------------------------------------------------------------------------------------
@@ -1172,7 +1210,7 @@ extern "C" int mlcg_seer_inputs(mlcg_handle* h, const float* x, const int32_t* a
                                 float* adj, void* stream) {
   STEP_PROLOGUE("seer_inputs");
   if (!x || !atom_class || !elements || !dist || !adj) FAIL(MLCG_E_ARG, "seer_inputs: null pointer");
-  k_seer_inputs<<<h->B, 128, 0, st>>>(x, atom_class, h->d_n_nodes.as<int>(), h->N, elements, dist, adj);
+  k_seer_inputs<<<h->pl->B, 128, 0, st>>>(x, atom_class, h->pl->d_n_nodes.as<int>(), h->pl->N, elements, dist, adj);
   KCHECK();
   return MLCG_OK;
 }
@@ -1283,6 +1321,15 @@ extern "C" int mlcg_seer_forward(mlcg_handle* h, const int32_t* elements, const 
 // ---------------------------------------------------------------------------------------------------------------
 // end-to-end with host buffers
 // ---------------------------------------------------------------------------------------------------------------
+// GCN inputs + GCN on the decoded batch in g_x / g_cls (active plan) -> g_bonds.
+static int seer_device(mlcg_handle* h, void* stream) {
+  int rc = mlcg_seer_inputs(h, h->g_x.as<float>(), h->g_cls.as<int32_t>(), h->g_el.as<int32_t>(), h->g_dist.as<float>(),
+                            h->g_adj.as<float>(), stream);
+  if (rc) return rc;
+  return mlcg_seer_forward(h, h->g_el.as<int32_t>(), h->g_dist.as<float>(), h->g_adj.as<float>(), nullptr,
+                           h->g_bonds.as<int8_t>(), h->pl->B, stream);
+}
+
 // The device part of mlcg_generate: reverse loop + GCN inputs + GCN.  Pure kernel / async-copy sequence on `stream`
 // (no allocation, no synchronisation once the workspaces exist), hence capturable into a CUDA graph.
 static int generate_device(mlcg_handle* h, int T, const mlcg_step_scalars* steps, int resample_steps, float sigma_0,
@@ -1291,20 +1338,26 @@ static int generate_device(mlcg_handle* h, int T, const mlcg_step_scalars* steps
                        nullptr, nullptr, seed, sample_offset, h->g_ids.as<int64_t>(), h->g_z.as<float>(), h->g_x.as<float>(),
                        h->g_cls.as<int32_t>(), nullptr, nullptr, stream);
   if (rc) return rc;
-  if ((rc = mlcg_seer_inputs(h, h->g_x.as<float>(), h->g_cls.as<int32_t>(), h->g_el.as<int32_t>(), h->g_dist.as<float>(),
-                             h->g_adj.as<float>(), stream)))
-    return rc;
-  return mlcg_seer_forward(h, h->g_el.as<int32_t>(), h->g_dist.as<float>(), h->g_adj.as<float>(), nullptr,
-                           h->g_bonds.as<int8_t>(), h->B, stream);
+  return seer_device(h, stream);
 }
 
-extern "C" int mlcg_generate(mlcg_handle* h, const int32_t* n_nodes_host, int B, int N, const float* ctx_host, int T,
-                             const mlcg_step_scalars* steps, int resample_steps, float sigma_0, float alpha_0, float sigma_x,
-                             uint64_t seed, int64_t sample_offset, const int64_t* sample_ids_host, float* x_host,
-                             int32_t* atom_class_host, int8_t* bonds_host, void* stream) {
-  if (!h) return MLCG_E_ARG;
-  if (!h->egnn_loaded || !h->seer_loaded) FAIL(MLCG_E_STATE, "generate: load both weight sets first");
-  if (!n_nodes_host || !ctx_host || !steps || !x_host || !atom_class_host || !bonds_host) FAIL(MLCG_E_ARG, "generate: null pointer");
+static inline long long fbits(float f) {
+  int32_t i;
+  memcpy(&i, &f, 4);
+  return (long long)i;
+}
+
+// Host side shared by mlcg_generate and mlcg_generate_fragment.  `key` holds everything the device sequence bakes into
+// kernel arguments.  A new key rebuilds the batch plan (mlcg_set_batch: plan 0 = n_nodes_host / N, plus plan 1 =
+// plan1_n_nodes / plan1_N when given) and drops the captured graph.  Every call uploads the per-call inputs -- context,
+// sample ids, {seed, sample_offset}, and whatever `upload(stream)` adds -- to handle-owned device buffers, then runs
+// `device(stream)`: eagerly on the first call with a key, captured into a CUDA graph on the second, replayed from then on.
+// The outputs are copied to x_out / atom_class_out / bonds_out (pinned host or device) and the stream is synchronised.
+template <class Upload, class Device>
+static int generate_graphed(mlcg_handle* h, const std::vector<long long>& key, const int32_t* n_nodes_host, int B, int N,
+                            const int32_t* plan1_n_nodes, int plan1_N, const float* ctx_host, uint64_t seed,
+                            int64_t sample_offset, const int64_t* sample_ids_host, float* x_out, int32_t* atom_class_out,
+                            int8_t* bonds_out, void* stream, Upload upload, Device device) {
   CK(cudaSetDevice(h->device));  // the call may come from any host thread (pipeline.GenerationPipeline's feeder)
   cudaStream_t st = (cudaStream_t)stream;
   if (st == nullptr) {
@@ -1315,21 +1368,12 @@ extern "C" int mlcg_generate(mlcg_handle* h, const int32_t* n_nodes_host, int B,
     st = h->own_stream;
     stream = (void*)st;
   }
-  // Key of the captured graph: batch geometry, schedule and every scalar baked into kernel arguments.
-  std::vector<long long> key;
-  key.reserve((size_t)B + 8 * (size_t)T + 16);
-  key.push_back(B); key.push_back(N); key.push_back(T); key.push_back(resample_steps); key.push_back(h->precision);
-  auto bits = [](float f) { int32_t i; memcpy(&i, &f, 4); return (long long)i; };
-  key.push_back(bits(sigma_0)); key.push_back(bits(alpha_0)); key.push_back(bits(sigma_x));
-  for (int b = 0; b < B; ++b) key.push_back(n_nodes_host[b]);
-  for (int s = 0; s < T; ++s) {
-    key.push_back(bits(steps[s].t)); key.push_back(bits(steps[s].alpha_ts)); key.push_back(bits(steps[s].c_eps));
-    key.push_back(bits(steps[s].c_sigma));
-  }
   const bool same = (key == h->gen_key);
   if (!same) {
     int rc = mlcg_set_batch(h, n_nodes_host, B, N);  // also drops any previously captured graph
     if (rc) return rc;
+    // set_batch drained the device: plan 1 may be rewritten too (outside any capture)
+    if (plan1_n_nodes && (rc = build_plan(h, h->plans[1], plan1_n_nodes, B, plan1_N))) return rc;
     h->gen_key = key;
   }
   h->gen_key_hits++;
@@ -1356,15 +1400,16 @@ extern "C" int mlcg_generate(mlcg_handle* h, const int32_t* n_nodes_host, int B,
   CK(cudaMemcpyAsync(h->g_ids.p, h->ids_stage.data(), (size_t)B * sizeof(int64_t), cudaMemcpyHostToDevice, st));
   const unsigned long long ctl[2] = {(unsigned long long)seed, (unsigned long long)sample_offset};
   CK(cudaMemcpyAsync(h->noise_ctl.p, ctl, sizeof(ctl), cudaMemcpyHostToDevice, st));
-  int rc = MLCG_OK;
+  int rc = upload(st);
+  if (rc) return rc;
   h->use_noise_ctl = true;  // the noise kernels read {seed, sample_offset} from device memory (graph-replayable)
   if (graphs_enabled && h->gen_graph == nullptr && h->gen_key_hits >= 2) {
-    // second call with this geometry: all workspaces exist and every kernel attribute has been set by the eager
-    // first call, so the launch sequence can be captured
+    // second call with this key: all workspaces exist and every kernel attribute has been set by the eager first call,
+    // so the launch sequence can be captured
     cudaGraph_t graph = nullptr;
     const long long launches0 = h->launches;
     CK(cudaStreamBeginCapture(st, cudaStreamCaptureModeThreadLocal));
-    rc = generate_device(h, T, steps, resample_steps, sigma_0, alpha_0, sigma_x, seed, sample_offset, stream);
+    rc = device(stream);
     cudaError_t ce = cudaStreamEndCapture(st, &graph);
     if (rc == MLCG_OK && ce == cudaSuccess && graph != nullptr) {
       ce = cudaGraphInstantiate(&h->gen_graph, graph, 0);
@@ -1384,16 +1429,168 @@ extern "C" int mlcg_generate(mlcg_handle* h, const int32_t* n_nodes_host, int B,
     CK(cudaGraphLaunch(h->gen_graph, st));
     h->launches += h->gen_graph_launches;
   } else {
-    rc = generate_device(h, T, steps, resample_steps, sigma_0, alpha_0, sigma_x, seed, sample_offset, stream);
+    rc = device(stream);
   }
   h->use_noise_ctl = false;
   if (rc) return rc;
   // the outputs may be pinned host buffers or device buffers (multi-GPU driver: results stay on the device for the gather)
-  CK(cudaMemcpyAsync(x_host, h->g_x.p, bn * 3 * 4, cudaMemcpyDefault, st));
-  CK(cudaMemcpyAsync(atom_class_host, h->g_cls.p, bn * 4, cudaMemcpyDefault, st));
-  CK(cudaMemcpyAsync(bonds_host, h->g_bonds.p, dd, cudaMemcpyDefault, st));
+  CK(cudaMemcpyAsync(x_out, h->g_x.p, bn * 3 * 4, cudaMemcpyDefault, st));
+  CK(cudaMemcpyAsync(atom_class_out, h->g_cls.p, bn * 4, cudaMemcpyDefault, st));
+  CK(cudaMemcpyAsync(bonds_out, h->g_bonds.p, dd, cudaMemcpyDefault, st));
   CK(cudaStreamSynchronize(st));
   return MLCG_OK;
+}
+
+extern "C" int mlcg_generate(mlcg_handle* h, const int32_t* n_nodes_host, int B, int N, const float* ctx_host, int T,
+                             const mlcg_step_scalars* steps, int resample_steps, float sigma_0, float alpha_0, float sigma_x,
+                             uint64_t seed, int64_t sample_offset, const int64_t* sample_ids_host, float* x_host,
+                             int32_t* atom_class_host, int8_t* bonds_host, void* stream) {
+  if (!h) return MLCG_E_ARG;
+  if (!h->egnn_loaded || !h->seer_loaded) FAIL(MLCG_E_STATE, "generate: load both weight sets first");
+  if (!n_nodes_host || !ctx_host || !steps || !x_host || !atom_class_host || !bonds_host) FAIL(MLCG_E_ARG, "generate: null pointer");
+  // Key of the captured graph: batch geometry, schedule and every scalar baked into kernel arguments.
+  std::vector<long long> key;
+  key.reserve((size_t)B + 8 * (size_t)T + 16);
+  key.push_back(B); key.push_back(N); key.push_back(T); key.push_back(resample_steps); key.push_back(h->precision);
+  key.push_back(fbits(sigma_0)); key.push_back(fbits(alpha_0)); key.push_back(fbits(sigma_x));
+  for (int b = 0; b < B; ++b) key.push_back(n_nodes_host[b]);
+  for (int s = 0; s < T; ++s) {
+    key.push_back(fbits(steps[s].t)); key.push_back(fbits(steps[s].alpha_ts)); key.push_back(fbits(steps[s].c_eps));
+    key.push_back(fbits(steps[s].c_sigma));
+  }
+  return generate_graphed(
+      h, key, n_nodes_host, B, N, nullptr, 0, ctx_host, seed, sample_offset, sample_ids_host, x_host, atom_class_host,
+      bonds_host, stream, [](cudaStream_t) { return (int)MLCG_OK; },
+      [&](void* s) { return generate_device(h, T, steps, resample_steps, sigma_0, alpha_0, sigma_x, seed, sample_offset, s); });
+}
+
+// Draw numbering of the merge loop of inertial fragment matching.  It starts at 0 like the first loop's, so both loops
+// draw the same normals per (sample, atom, draw) -- exactly what the eager composition
+// (MLConformerGenerator.edm_sample_tensors: two mlcg_sample calls) does, which this path reproduces bit for bit.
+static const uint64_t kMergeDrawBase = 0;
+
+// The device part of mlcg_generate_fragment (see mlcg.h): the launch sequence of the eager composition, on plan 0 (whole
+// molecules) and -- mode 2 -- plan 1 (the atoms still to be generated).  The plan switches happen on the host between
+// launches; each launch bakes in the pointers of its plan, so one captured graph holds both loops.
+static int generate_fragment_device(mlcg_handle* h, int mode, int n_ff, const IfmArgs& ifm, int T,
+                                    const mlcg_step_scalars* steps, int resample_steps, int diffusion_level, float merge_alpha,
+                                    float merge_sigma, float sigma_0, float alpha_0, float sigma_x, uint64_t seed,
+                                    int64_t sample_offset, void* stream) {
+  cudaStream_t st = (cudaStream_t)stream;
+  const int B = h->plans[0].B, N = h->plans[0].N;
+  const int64_t* ids = h->g_ids.as<int64_t>();
+  float* zk = h->f_zk.as<float>();
+  float* fm = h->f_fm.as<float>();
+  int rc;
+  if (mode == 1) {
+    // z_known / fixed_mask of EquivariantDiffusion.inpaint (prepare_fragment): the merge-input kernel with no generated atoms
+    k_ifm_merge_inputs<<<B, 64, 0, st>>>(nullptr, nullptr, nullptr, nullptr, h->f_ffx.as<float>(), h->f_ffh.as<float>(), n_ff,
+                                         0, N, zk, fm);
+    KCHECK();
+    rc = sample_loop(h, 1, T, steps, resample_steps, diffusion_level, 0.f, 0.f, sigma_0, alpha_0, sigma_x, h->g_ctx.as<float>(),
+                     zk, fm, nullptr, seed, sample_offset, ids, h->g_z.as<float>(), h->g_x.as<float>(), h->g_cls.as<int32_t>(),
+                     nullptr, nullptr, 0, stream);
+    if (rc) return rc;
+    return seer_device(h, stream);
+  }
+  // inertial fragment matching: per-sample context of the atoms still to be generated ...
+  k_ifm_context<<<(B + 127) / 128, 128, 0, st>>>(h->plans[0].d_n_nodes.as<int>(), B, ifm, h->f_ctx.as<float>(),
+                                                 h->f_shift.as<float>(), h->f_rot.as<float>(), h->f_ngen.as<int>());
+  KCHECK();
+  // ... generated on their own (plan 1) ...
+  h->pl = &h->plans[1];
+  rc = sample_loop(h, 0, T, steps, resample_steps, diffusion_level, 0.f, 0.f, sigma_0, alpha_0, sigma_x, h->f_ctx.as<float>(),
+                   nullptr, nullptr, nullptr, seed, sample_offset, ids, h->g_z.as<float>(), h->f_xg.as<float>(),
+                   h->f_clsg.as<int32_t>(), nullptr, nullptr, 0, stream);
+  h->pl = &h->plans[0];
+  if (rc) return rc;
+  // ... moved back to the reference frame next to the fixed fragment, and merged with it (plan 0)
+  k_ifm_merge_inputs<<<B, 64, 0, st>>>(h->f_xg.as<float>(), h->f_clsg.as<int32_t>(), h->f_shift.as<float>(), h->f_rot.as<float>(),
+                                       h->f_ffx.as<float>(), h->f_ffh.as<float>(), n_ff, N - n_ff, N, zk, fm);
+  KCHECK();
+  rc = sample_loop(h, 2, T, steps, resample_steps, diffusion_level, merge_alpha, merge_sigma, sigma_0, alpha_0, sigma_x,
+                   h->g_ctx.as<float>(), zk, fm, nullptr, seed, sample_offset, ids, h->g_z.as<float>(), h->g_x.as<float>(),
+                   h->g_cls.as<int32_t>(), nullptr, nullptr, kMergeDrawBase, stream);
+  if (rc) return rc;
+  return seer_device(h, stream);
+}
+
+extern "C" int mlcg_generate_fragment(mlcg_handle* h, const mlcg_fragment* frag, const int32_t* n_nodes_host, int B, int N,
+                                      const float* ctx_host, int T, const mlcg_step_scalars* steps, int resample_steps,
+                                      float sigma_0, float alpha_0, float sigma_x, uint64_t seed, int64_t sample_offset,
+                                      const int64_t* sample_ids_host, float* x_out, int32_t* atom_class_out, int8_t* bonds_out,
+                                      void* stream) {
+  if (!h) return MLCG_E_ARG;
+  if (!h->egnn_loaded || !h->seer_loaded) FAIL(MLCG_E_ARG, "generate_fragment: load both weight sets first");
+  if (!frag || !n_nodes_host || !ctx_host || !steps || !x_out || !atom_class_out || !bonds_out || !frag->ff_x_host ||
+      !frag->ff_h_host)
+    FAIL(MLCG_E_ARG, "generate_fragment: null pointer");
+  const int mode = frag->mode, n_ff = frag->n_ff;
+  if (mode != 1 && mode != 2) FAIL(MLCG_E_ARG, "generate_fragment: mode must be 1 (inpaint) or 2 (inertial fragment matching)");
+  if (mode == 2 && (!frag->moi_gen_origin_host || !frag->ff_weighted_com_host || !frag->norm_mean_host || !frag->norm_mad_host))
+    FAIL(MLCG_E_ARG, "generate_fragment: null pointer (inertial fragment matching needs the moment-of-inertia prologue)");
+  if (B <= 0 || N <= 0 || N > EDGE_MAXN || T <= 0 || resample_steps < 0)
+    FAIL(MLCG_E_ARG, "generate_fragment: need B > 0, 1 <= N <= 39, T > 0 and resample_steps >= 0");
+  if (n_ff < 1) FAIL(MLCG_E_ARG, "generate_fragment: the fragment needs at least one atom");
+  if (N - n_ff < 1) FAIL(MLCG_E_ARG, "generate_fragment: the fragment must have fewer atoms than N");
+  int min_n = N;
+  for (int b = 0; b < B; ++b) min_n = std::min(min_n, (int)n_nodes_host[b]);
+  if (n_ff >= min_n) FAIL(MLCG_E_ARG, "generate_fragment: the fragment must have fewer atoms than every sample");
+  IfmArgs ifm{};
+  std::vector<int32_t> n_gen;
+  if (mode == 2) {
+    memcpy(ifm.moi0, frag->moi_gen_origin_host, sizeof(ifm.moi0));
+    memcpy(ifm.ffsum, frag->ff_weighted_com_host, sizeof(ifm.ffsum));
+    memcpy(ifm.mean, frag->norm_mean_host, sizeof(ifm.mean));
+    memcpy(ifm.mad, frag->norm_mad_host, sizeof(ifm.mad));
+    ifm.n_ff = n_ff;
+    n_gen.resize(B);
+    for (int b = 0; b < B; ++b) n_gen[b] = n_nodes_host[b] - n_ff;
+  }
+  // Key of the captured graph.  It starts with -mode, so it never equals a key of mlcg_generate (which starts with B).
+  // Mode 2 adds what is baked into kernel arguments beyond mlcg_generate's key: the merge level and its scalars, and the
+  // moment-of-inertia prologue k_ifm_context takes by value.  The fragment itself is uploaded on every call.
+  std::vector<long long> key;
+  key.reserve((size_t)B + 8 * (size_t)T + 48);
+  key.push_back(-mode); key.push_back(B); key.push_back(N); key.push_back(T); key.push_back(resample_steps);
+  key.push_back(h->precision); key.push_back(n_ff);
+  key.push_back(fbits(sigma_0)); key.push_back(fbits(alpha_0)); key.push_back(fbits(sigma_x));
+  if (mode == 2) {
+    key.push_back(frag->diffusion_level); key.push_back(fbits(frag->merge_alpha)); key.push_back(fbits(frag->merge_sigma));
+    const float* pro = reinterpret_cast<const float*>(&ifm);
+    for (size_t k = 0; k < offsetof(IfmArgs, n_ff) / sizeof(float); ++k) key.push_back(fbits(pro[k]));
+  }
+  for (int b = 0; b < B; ++b) key.push_back(n_nodes_host[b]);
+  for (int s = 0; s < T; ++s) {
+    const mlcg_step_scalars& c = steps[s];
+    for (float v : {c.t, c.alpha_ts, c.c_eps, c.c_sigma, c.alpha_s, c.sigma_s, c.blend}) key.push_back(fbits(v));
+  }
+  const size_t bn = (size_t)B * N, bg = (size_t)B * (N - n_ff);
+  auto upload = [&](cudaStream_t st) -> int {
+    CK(h->f_ffx.ensure((size_t)n_ff * 3 * 4));
+    CK(h->f_ffh.ensure((size_t)n_ff * 8 * 4));
+    CK(h->f_zk.ensure(bn * ZC * 4));
+    CK(h->f_fm.ensure(bn * 4));
+    if (mode == 2) {
+      CK(h->f_ctx.ensure((size_t)B * 3 * 4));
+      CK(h->f_shift.ensure((size_t)B * 3 * 4));
+      CK(h->f_rot.ensure((size_t)B * 9 * 4));
+      CK(h->f_ngen.ensure((size_t)B * 4));
+      CK(h->f_xg.ensure(bg * 3 * 4));
+      CK(h->f_clsg.ensure(bg * 4));
+    }
+    CK(cudaMemcpyAsync(h->f_ffx.p, frag->ff_x_host, (size_t)n_ff * 3 * 4, cudaMemcpyHostToDevice, st));
+    CK(cudaMemcpyAsync(h->f_ffh.p, frag->ff_h_host, (size_t)n_ff * 8 * 4, cudaMemcpyHostToDevice, st));
+    return MLCG_OK;
+  };
+  const int diffusion_level = mode == 2 ? frag->diffusion_level : 0;
+  const float merge_alpha = mode == 2 ? frag->merge_alpha : 0.f, merge_sigma = mode == 2 ? frag->merge_sigma : 0.f;
+  return generate_graphed(h, key, n_nodes_host, B, N, mode == 2 ? n_gen.data() : nullptr, N - n_ff, ctx_host, seed,
+                          sample_offset, sample_ids_host, x_out, atom_class_out, bonds_out, stream, upload, [&](void* s) {
+                            return generate_fragment_device(h, mode, n_ff, ifm, T, steps, resample_steps, diffusion_level,
+                                                            merge_alpha, merge_sigma, sigma_0, alpha_0, sigma_x, seed,
+                                                            sample_offset, s);
+                          });
 }
 
 // ---------------------------------------------------------------------------------------------------------------
@@ -1548,13 +1745,13 @@ extern "C" int mlcg_gemm_phase_profile(mlcg_handle* h, int which, double* out, v
   cudaStream_t st = (cudaStream_t)stream;
   const int mode = h->precision, kc = h->kc448();
   const LayerW& L = h->layers[0];
-  const int grid = std::min(h->n_mtiles * (which == 0 ? 2 : 1), h->num_sms);
+  const int grid = std::min(h->pl->n_mtiles * (which == 0 ? 2 : 1), h->num_sms);
   DevBuf buf;
   CK(buf.ensure((size_t)grid * 8 * sizeof(long long)));
   CK(cudaMemsetAsync(buf.p, 0, (size_t)grid * 8 * sizeof(long long), st));
   GemmArgs a{};
   a.prof = buf.as<long long>();
-  a.m_rows = h->M;
+  a.m_rows = h->pl->M;
   a.out_scale = (which == 0) ? act_scale(mode) : op_scale(mode);
   cudaEvent_t e0, e1;
   CK(cudaEventCreate(&e0));
@@ -1564,20 +1761,20 @@ extern "C" int mlcg_gemm_phase_profile(mlcg_handle* h, int which, double* out, v
     a.a0 = h->h_op.as<uint8_t>(); a.a0_chunks = kc; a.a0_per_tile = kc; a.n_kc = kc;
     a.w = L.w1ab_op.as<uint8_t>(); a.bias = L.bias_pq.as<float>();
     a.out_f32 = h->pq.as<float>(); a.ldo = 2 * HP; a.n_valid = 2 * HP;
-    if (mode == PREC_FP16) CK((launch_gemm<PREC_FP16, HP, EPI_BF16>(a, h->n_mtiles, 2, st)));
-    else if (mode == PREC_BF16) CK((launch_gemm<PREC_BF16, HP, EPI_BF16>(a, h->n_mtiles, 2, st)));
-    else CK((launch_gemm<PREC_TF32, HP, EPI_F32>(a, h->n_mtiles, 2, st)));
+    if (mode == PREC_FP16) CK((launch_gemm<PREC_FP16, HP, EPI_BF16>(a, h->pl->n_mtiles, 2, st)));
+    else if (mode == PREC_BF16) CK((launch_gemm<PREC_BF16, HP, EPI_BF16>(a, h->pl->n_mtiles, 2, st)));
+    else CK((launch_gemm<PREC_TF32, HP, EPI_F32>(a, h->pl->n_mtiles, 2, st)));
   } else if (which == 1) {
     a.a0 = h->h_op.as<uint8_t>(); a.a0_chunks = kc; a.a0_per_tile = kc;
     a.a1 = h->agg_op.as<uint8_t>(); a.a1_per_tile = kc; a.n_kc = 2 * kc;
     a.w = L.w3_op.as<uint8_t>(); a.bias = L.b3p.as<float>();
     a.out_op = h->t_op.as<uint8_t>(); a.out_op_chunks = kc;
-    CK((launch_gemm_mode<HP, EPI_SILU_OP>(mode, a, h->n_mtiles, 1, st)));
+    CK((launch_gemm_mode<HP, EPI_SILU_OP>(mode, a, h->pl->n_mtiles, 1, st)));
   } else {
     a.a0 = h->t_op.as<uint8_t>(); a.a0_chunks = kc; a.a0_per_tile = kc; a.n_kc = kc;
     a.w = L.w4_op.as<uint8_t>(); a.bias = L.b4p.as<float>();
     a.out_op = h->h_op.as<uint8_t>(); a.out_op_chunks = kc; a.resid = h->h_res.as<float>(); a.ldr = 0;
-    CK((launch_gemm_mode<HP, EPI_RESID_OP>(mode, a, h->n_mtiles, 1, st)));
+    CK((launch_gemm_mode<HP, EPI_RESID_OP>(mode, a, h->pl->n_mtiles, 1, st)));
   }
   CK(cudaEventRecord(e1, st));
   h->launches++;

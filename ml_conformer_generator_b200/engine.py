@@ -217,12 +217,9 @@ class Engine:
                     n_nodes: torch.Tensor):
         """Device version of ifm_prepare_gen_fragment_context after its batch-independent prologue.  n_nodes: (B) total
         atoms per sample.  Returns device tensors (ctx (B,3) normalised, shift (B,3), rotation (B,3,3), n_gen (B) i32)."""
-        from .mol_utils import get_moment_of_inertia_tensor
-        ffx = fixed_fragment_x.detach().to("cpu", torch.float32)
-        n_ff = int(ffx.size(0))
-        moi0 = (torch.diag(torch.as_tensor(reference_context, dtype=torch.float32).cpu())
-                - get_moment_of_inertia_tensor(ffx, torch.ones(n_ff))).contiguous()
-        com = (n_ff * ffx.mean(dim=0)).to(torch.float32).contiguous()
+        from .mol_utils import ifm_moi_prologue
+        n_ff = int(fixed_fragment_x.size(0))
+        moi0, com = ifm_moi_prologue(fixed_fragment_x, reference_context)
         mean = torch.as_tensor(context_norms["mean"], dtype=torch.float32).contiguous()
         mad = torch.as_tensor(context_norms["mad"], dtype=torch.float32).contiguous()
         nn = n_nodes.to(self.device, torch.int32).contiguous()
@@ -268,21 +265,8 @@ class Engine:
         """End-to-end with host inputs: returns (x (B,N,3) f32, atom_class (B,N) i32, bonds (B,42,42) i8) in pinned host
         buffers, or -- `device_out=True`, used by the multi-GPU driver whose gather runs on the device -- in device
         tensors.  `sample_ids` (B int64): global ids keying the device noise (default `sample_offset + b`)."""
-        nn = np.ascontiguousarray(np.asarray(n_nodes, dtype=np.int32).reshape(-1))
+        nn, ctxh, ids, out = self._host_call_inputs("generate_host", n_nodes, max_n_nodes, ctx, sample_ids, out, device_out)
         B, N = int(nn.size), int(max_n_nodes)
-        ctxh = torch.from_numpy(np.ascontiguousarray(ctx, dtype=np.float32).reshape(B, 3)).pin_memory()
-        ids = None
-        if sample_ids is not None:
-            ids = np.ascontiguousarray(np.asarray(sample_ids, dtype=np.int64).reshape(-1))
-            if ids.size != B:
-                raise ValueError("generate_host: sample_ids must hold one id per sample")
-        if out is None:
-            if device_out:
-                out = (torch.empty(B, N, 3, device=self.device), torch.empty(B, N, dtype=torch.int32, device=self.device),
-                       torch.empty(B, 42, 42, dtype=torch.int8, device=self.device))
-            else:
-                out = (torch.empty(B, N, 3).pin_memory(), torch.empty(B, N, dtype=torch.int32).pin_memory(),
-                       torch.empty(B, 42, 42, dtype=torch.int8).pin_memory())
         gamma, steps = self._steps_cached(T, 3)
         dec = decode_scalars(gamma)
         rc = self.lib.mlcg_generate(self.h, nn.ctypes.data_as(C.c_void_p), B, N, _ptr(ctxh), T, steps, resample_steps,
@@ -291,6 +275,72 @@ class Engine:
                                     _ptr(out[1]), _ptr(out[2]), self._stream())
         self._check(rc, "generate")
         self.check_finite("generate")
+        self.B, self.N = B, N
+        self.n_nodes = torch.from_numpy(nn.copy())
+        return out
+
+    def _host_call_inputs(self, what, n_nodes, max_n_nodes, ctx, sample_ids, out, device_out):
+        """Host inputs of generate_host / generate_fragment_host: atom counts (int32), pinned (B,3) context, sample ids
+        (int64 or None) and the output buffers (`out`, or new pinned host / device tensors)."""
+        nn = np.ascontiguousarray(np.asarray(n_nodes, dtype=np.int32).reshape(-1))
+        B, N = int(nn.size), int(max_n_nodes)
+        ctxh = torch.from_numpy(np.ascontiguousarray(ctx, dtype=np.float32).reshape(B, 3)).pin_memory()
+        ids = None
+        if sample_ids is not None:
+            ids = np.ascontiguousarray(np.asarray(sample_ids, dtype=np.int64).reshape(-1))
+            if ids.size != B:
+                raise ValueError("%s: sample_ids must hold one id per sample" % what)
+        if out is None:
+            if device_out:
+                out = (torch.empty(B, N, 3, device=self.device), torch.empty(B, N, dtype=torch.int32, device=self.device),
+                       torch.empty(B, 42, 42, dtype=torch.int8, device=self.device))
+            else:
+                out = (torch.empty(B, N, 3).pin_memory(), torch.empty(B, N, dtype=torch.int32).pin_memory(),
+                       torch.empty(B, 42, 42, dtype=torch.int8).pin_memory())
+        return nn, ctxh, ids, out
+
+    def generate_fragment_host(self, n_nodes: np.ndarray, max_n_nodes: int, ctx: np.ndarray, fragment_x, fragment_h,
+                               inertial_fragment_matching: bool = True, reference_context=None, context_norms=None,
+                               T: int = 100, resample_steps: int = 0, blend_power: int = 3, diffusion_level: int = 50,
+                               seed: int = 0, sample_offset: int = 0, sample_ids=None, out=None, device_out: bool = False):
+        """generate_host around a fixed fragment (the reference's `fixed_fragment=`): fragment_x (n_ff,3) coordinates in
+        the frame centred on the reference's centre of mass, fragment_h (n_ff,8) raw 0/1 one-hot.  With
+        inertial_fragment_matching (the reference's default) the atoms still to be generated are sampled on their own in
+        the frame of their inertia tensor -- which needs the raw `reference_context` (principal moments) and
+        `context_norms` (default CONTEXT_NORMS) -- and merged with the fragment in a second loop at `diffusion_level`;
+        otherwise the fragment is inpainted.  `ctx` (B,3) is the normalised reference context of every sample.  Same
+        outputs, noise keys and graph replay as generate_host; the result equals the eager composition of
+        MLConformerGenerator.edm_sample_tensors + the GCN bit for bit."""
+        nn, ctxh, ids, out = self._host_call_inputs("generate_fragment_host", n_nodes, max_n_nodes, ctx, sample_ids, out,
+                                                    device_out)
+        B, N = int(nn.size), int(max_n_nodes)
+        ffx = np.ascontiguousarray(torch.as_tensor(fragment_x).detach().cpu().numpy(), dtype=np.float32)
+        ffh = np.ascontiguousarray(torch.as_tensor(fragment_h).detach().cpu().numpy(), dtype=np.float32)
+        if ffx.ndim != 2 or ffx.shape[1] != 3 or ffh.shape != (ffx.shape[0], 8):
+            raise ValueError("generate_fragment_host: the fragment must be coordinates (n,3) and a one-hot (n,8)")
+        gamma, steps = self._steps_cached(T, blend_power)
+        dec = decode_scalars(gamma)
+        frag = _lib.Fragment(2 if inertial_fragment_matching else 1, int(ffx.shape[0]), ffx.ctypes.data, ffh.ctypes.data)
+        keep = []
+        if inertial_fragment_matching:
+            if reference_context is None:
+                raise ValueError("generate_fragment_host: inertial fragment matching needs the raw reference_context")
+            from .config import CONTEXT_NORMS
+            from .mol_utils import ifm_moi_prologue
+            norms = CONTEXT_NORMS if context_norms is None else context_norms
+            moi0, com = ifm_moi_prologue(torch.from_numpy(ffx), reference_context)
+            keep = [moi0, com] + [torch.as_tensor(norms[k], dtype=torch.float32).contiguous() for k in ("mean", "mad")]
+            lvl = forward_level_scalars(gamma, diffusion_level)
+            frag.diffusion_level, frag.merge_alpha, frag.merge_sigma = int(diffusion_level), lvl["alpha"], lvl["sigma"]
+            frag.moi_gen_origin_host, frag.ff_weighted_com_host, frag.norm_mean_host, frag.norm_mad_host = (
+                t.data_ptr() for t in keep)
+        rc = self.lib.mlcg_generate_fragment(self.h, C.byref(frag), nn.ctypes.data_as(C.c_void_p), B, N, _ptr(ctxh), T,
+                                             steps, resample_steps, dec["sigma_0"], dec["alpha_0"], dec["sigma_x"], seed,
+                                             sample_offset, None if ids is None else ids.ctypes.data_as(C.c_void_p),
+                                             _ptr(out[0]), _ptr(out[1]), _ptr(out[2]), self._stream())
+        del keep
+        self._check(rc, "generate_fragment")
+        self.check_finite("generate_fragment")
         self.B, self.N = B, N
         self.n_nodes = torch.from_numpy(nn.copy())
         return out

@@ -165,6 +165,19 @@ def ifm_prepare_gen_fragment_context(fixed_fragment_x: torch.Tensor, reference_c
     return node_mask, edge_mask, ctx, shift.to(device), rotation.to(device)
 
 
+def ifm_moi_prologue(fixed_fragment_x: torch.Tensor, reference_context: torch.Tensor
+                     ) -> Tuple[torch.Tensor, torch.Tensor]:
+    """Batch-independent prologue of ifm_prepare_gen_fragment_context, in float32 as there (reference mol_utils.py:396-411):
+    moi_gen_origin (3,3) = diag(reference_context) - MOI(fixed fragment), and ff_weighted_com (3) = n_ff * mean(fixed
+    fragment coordinates).  The host inputs of mlcg_ifm_context / mlcg_generate_fragment."""
+    ffx = fixed_fragment_x.detach().to("cpu", torch.float32)
+    n_ff = int(ffx.size(0))
+    moi0 = (torch.diag(torch.as_tensor(reference_context, dtype=torch.float32).cpu())
+            - get_moment_of_inertia_tensor(ffx, torch.ones(n_ff))).contiguous()
+    com = (n_ff * ffx.mean(dim=0)).to(torch.float32).contiguous()
+    return moi0, com
+
+
 def ifm_prepare_fragments_for_merge(fixed_fragment_x: torch.Tensor, fixed_fragment_h: torch.Tensor,
                                     gen_fragments_x: torch.Tensor, gen_fragments_h: torch.Tensor, max_n_nodes: int,
                                     device: torch.device = torch.device("cpu")):

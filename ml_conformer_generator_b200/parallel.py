@@ -111,12 +111,20 @@ def generate_sharded(run_shard: Callable[[np.ndarray, np.ndarray], Sequence[torc
 
 def generate_sharded_engine(engine, n_nodes: Sequence[int], max_n_nodes: int, ctx: np.ndarray, T: int = 100,
                             resample_steps: int = 0, seed: int = 0, group=None, max_batch: int = 8192,
-                            stats: Optional[dict] = None):
+                            stats: Optional[dict] = None, fixed_fragment=None, inertial_fragment_matching: bool = True,
+                            reference_context=None, blend_power: int = 3, ifm_diffusion_level: int = 50):
     """`generate_sharded` driving `Engine.generate_host` (device outputs): the multi-GPU product path.  ctx: (B,3)
-    normalised context of every sample."""
+    normalised context of every sample.  With `fixed_fragment` = (coordinates (n,3), one-hot (n,8)) every shard runs
+    `Engine.generate_fragment_host` instead (inertial fragment matching needs the raw `reference_context`); the cost of a
+    sample still rises with its atom count, so the same size-balanced shards apply."""
     ctx = np.asarray(ctx, dtype=np.float32).reshape(-1, 3)
 
     def run_shard(ids, nn):
+        if fixed_fragment is not None:
+            return engine.generate_fragment_host(nn, max_n_nodes, ctx[ids], fixed_fragment[0], fixed_fragment[1],
+                                                 inertial_fragment_matching, reference_context, None, T, resample_steps,
+                                                 blend_power, ifm_diffusion_level, seed=seed, sample_ids=ids,
+                                                 device_out=True)
         return engine.generate_host(nn, max_n_nodes, ctx[ids], T, resample_steps, seed=seed, sample_ids=ids, device_out=True)
 
     return generate_sharded(run_shard, n_nodes, max_n_nodes, group, max_batch, engine.device, stats)

@@ -106,9 +106,12 @@ def sdf_postprocess(x, cls, bonds, n, index) -> str:
 
 
 def engine_batches(engine, n_nodes_per_batch: Sequence[np.ndarray], max_n_nodes: int, ctx_per_batch: Sequence[np.ndarray],
-                   T: int = 100, seed: int = 0) -> Callable:
+                   T: int = 100, seed: int = 0, fixed_fragment=None, inertial_fragment_matching: bool = True,
+                   reference_context=None, context_norms=None, blend_power: int = 3,
+                   ifm_diffusion_level: int = 50) -> Callable:
     """`generate` callable over `Engine.generate_host`: batch k gets global sample ids following the previous batches (so the
-    whole run equals one big batch, bit for bit) and reuses the pinned output buffers of its ring slot."""
+    whole run equals one big batch, bit for bit) and reuses the pinned output buffers of its ring slot.  With
+    `fixed_fragment` = (coordinates (n,3), one-hot (n,8)) it calls `Engine.generate_fragment_host` instead."""
     offsets = np.concatenate([[0], np.cumsum([len(n) for n in n_nodes_per_batch])])
 
     def generate(k, out):
@@ -116,8 +119,15 @@ def engine_batches(engine, n_nodes_per_batch: Sequence[np.ndarray], max_n_nodes:
         reuse = None
         if out is not None and tuple(out[0].shape) == (len(nn), max_n_nodes, 3):
             reuse = out[:3]
-        x, cls, bonds = engine.generate_host(nn, max_n_nodes, ctx_per_batch[k], T, 0, seed=seed,
-                                             sample_ids=np.arange(offsets[k], offsets[k + 1]), out=reuse)
+        ids = np.arange(offsets[k], offsets[k + 1])
+        if fixed_fragment is not None:
+            x, cls, bonds = engine.generate_fragment_host(nn, max_n_nodes, ctx_per_batch[k], fixed_fragment[0],
+                                                          fixed_fragment[1], inertial_fragment_matching, reference_context,
+                                                          context_norms, T, 0, blend_power, ifm_diffusion_level, seed=seed,
+                                                          sample_ids=ids, out=reuse)
+        else:
+            x, cls, bonds = engine.generate_host(nn, max_n_nodes, ctx_per_batch[k], T, 0, seed=seed, sample_ids=ids,
+                                                 out=reuse)
         return x, cls, bonds, nn
 
     return generate
