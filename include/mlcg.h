@@ -9,7 +9,7 @@
  *  - plain pointers and sizes only; no torch types.  Unless a parameter says "host", pointers are DEVICE pointers
  *    owned by the caller; the library never frees caller memory.
  *  - every call enqueues its work on `stream` (a cudaStream_t passed as void*) and returns without synchronising,
- *    except mlcg_generate / mlcg_generate_fragment / mlcg_load_* / mlcg_set_batch which are synchronous.
+ *    except mlcg_generate / mlcg_generate_fragment(_jobs) / mlcg_load_* / mlcg_set_batch which are synchronous.
  *  - return value: 0 = ok, < 0 = argument / state error (see mlcg_last_error), > 0 = cudaError_t.
  *  - one handle per (device, stream); a handle is thread-compatible, not thread-safe.
  *  - layouts are the reference's: z / eps / noise are (B, N, 11) float32 row-major with N = the call's max_n_nodes
@@ -181,15 +181,49 @@ typedef struct {
  * mlcg_sample(mode 1); mode 2: mlcg_ifm_context on the whole atom counts, mlcg_sample(mode 0) on the atoms still to be
  * generated with the context it wrote, mlcg_ifm_merge_inputs, mlcg_sample(mode 2) -- then mlcg_seer_inputs +
  * mlcg_seer_forward, with the same noise keys and draw numbers; the results equal that composition bit for bit.  The
- * fragment, context, sample ids and {seed, sample_offset} are uploaded on every call, so a replay never sees a previous
- * call's inputs; a different mode-2 prologue (another fragment or reference context) is a new key.  A call of
- * mlcg_generate and one of mlcg_generate_fragment invalidate each other's graph.  Returns MLCG_E_ARG for a mode other
- * than 1 or 2, n_ff < 1, n_ff >= min(n_nodes), N - n_ff < 1, a null pointer or weights not loaded. */
+ * fragment, its prologue, context, sample ids and {seed, sample_offset} are uploaded on every call, so a replay never sees
+ * a previous call's inputs, and another fragment or reference context of the same size replays the captured graph.  A
+ * call of mlcg_generate and one of mlcg_generate_fragment(_jobs) invalidate each other's graph.  This is the one-job case
+ * of mlcg_generate_fragment_jobs.  Returns MLCG_E_ARG for a mode other than 1 or 2, n_ff < 1, n_ff >= min(n_nodes),
+ * N - n_ff < 1, a null pointer or weights not loaded. */
 int mlcg_generate_fragment(mlcg_handle* h, const mlcg_fragment* frag, const int32_t* n_nodes_host, int B, int N,
                            const float* ctx_host, int T, const mlcg_step_scalars* steps, int resample_steps, float sigma_0,
                            float alpha_0, float sigma_x, uint64_t seed, int64_t sample_offset,
                            const int64_t* sample_ids_host, float* x_out, int32_t* atom_class_out, int8_t* bonds_out,
                            void* stream);
+
+/* Many fragment jobs of one mode in one call of mlcg_generate_fragment_jobs: every job has its own fixed fragment (and,
+ * mode 2, its own reference context); the loop settings are shared.  All HOST pointers. */
+typedef struct {
+  int mode;                          /* 1 = inpainting, 2 = inertial fragment matching (as mlcg_fragment.mode) */
+  int n_jobs;                        /* >= 1 */
+  const int32_t* job_of_sample_host; /* (B) the job of every sample, 0 <= job < n_jobs */
+  const int32_t* n_ff_host;          /* (n_jobs) fixed atoms of every job, 1 <= n_ff[job[b]] < n_nodes[b] */
+  const float* ff_x_host;            /* (sum n_ff,3) the jobs' fragment coordinates back to back, in job order */
+  const float* ff_h_host;            /* (sum n_ff,8) their raw 0/1 one-hot atom classes, in the same order */
+  int diffusion_level;               /* mode 2: merge_fragments' diffusion_level, shared */
+  float merge_alpha, merge_sigma;    /* mode 2: alpha / sigma of that level, shared */
+  const float* moi_gen_origin_host;  /* mode 2: (n_jobs,3,3), per job as mlcg_ifm_context takes it */
+  const float* ff_weighted_com_host; /* mode 2: (n_jobs,3), per job as mlcg_ifm_context takes it */
+  const float* norm_mean_host;       /* mode 2: 3, CONTEXT_NORMS mean, shared */
+  const float* norm_mad_host;        /* mode 2: 3, CONTEXT_NORMS mad, shared */
+} mlcg_fragment_jobs;
+
+/* mlcg_generate_fragment for many jobs at once: sample b runs with the fragment (and, mode 2, the prologue) of job
+ * job_of_sample[b]; every other input and output is that of mlcg_generate_fragment.  Mode 2 generates the atoms still to
+ * be generated, n_nodes[b] - n_ff[job[b]], padded to N - min(n_ff over the samples).  Every kernel works on each sample
+ * alone and the noise is keyed by the global sample id, so a sample's result equals that of a call holding only its own
+ * job with the same id, bit for bit.  The graph key is the geometry (mode, B, N, per-sample n_nodes and n_ff, the job
+ * count and the packed fragment length) and the shared scalars; the fragments, the job table, the job of every sample,
+ * the context, the ids and the seed are uploaded on every call, so other references or fragments of the same sizes
+ * replay the captured graph.  Returns MLCG_E_ARG for a mode other than 1 or 2, n_jobs < 1, a job index out of range,
+ * n_ff < 1 or N - n_ff < 1 for any job, n_ff[job[b]] >= n_nodes[b] for any sample, a null pointer or weights not
+ * loaded. */
+int mlcg_generate_fragment_jobs(mlcg_handle* h, const mlcg_fragment_jobs* jobs, const int32_t* n_nodes_host, int B, int N,
+                                const float* ctx_host, int T, const mlcg_step_scalars* steps, int resample_steps,
+                                float sigma_0, float alpha_0, float sigma_x, uint64_t seed, int64_t sample_offset,
+                                const int64_t* sample_ids_host, float* x_out, int32_t* atom_class_out, int8_t* bonds_out,
+                                void* stream);
 
 /* ---- Inertial fragment matching (the default fragment mode) between the two reverse loops ---------------------------
  * Replaces: ifm_prepare_gen_fragment_context (utils/mol_utils.py:373-457) after its batch-independent prologue.  The
@@ -262,6 +296,8 @@ int mlcg_nonfinite(mlcg_handle* h, void* stream);
 int mlcg_num_edge_tiles(mlcg_handle* h);
 int64_t mlcg_num_edges(mlcg_handle* h);          /* sum_b n_b (n_b - 1) */
 int64_t mlcg_kernel_launches(mlcg_handle* h);    /* kernels launched by this handle since creation */
+int64_t mlcg_graph_captures(mlcg_handle* h);     /* CUDA graphs captured by mlcg_generate / mlcg_generate_fragment(_jobs)
+                                                    since creation: a replay leaves it unchanged */
 /* Times the dominant kernel (the fused edge kernel) with CUDA events on `stream`: runs one sub-layer launch `iters`
  * times on the current batch state and returns the mean milliseconds per launch (< 0 on error). */
 float mlcg_time_edge_kernel(mlcg_handle* h, int layer, int iters, void* stream);

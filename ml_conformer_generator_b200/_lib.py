@@ -20,7 +20,7 @@ EXPORTS = [
     "mlcg_num_edges", "mlcg_kernel_launches", "mlcg_time_edge_kernel", "mlcg_edge_phase_profile", "mlcg_test_gemm",
     "mlcg_shape_moments", "mlcg_shape_tanimoto", "mlcg_gemm_phase_profile", "mlcg_plan_edge_tiles",
     "mlcg_egnn_forward_breakdown", "mlcg_ifm_context", "mlcg_ifm_merge_inputs", "mlcg_nonfinite", "mlcg_edge_block_order",
-    "mlcg_generate_fragment",
+    "mlcg_generate_fragment", "mlcg_generate_fragment_jobs", "mlcg_graph_captures",
 ]
 
 
@@ -43,6 +43,13 @@ class Fragment(C.Structure):
                 ("diffusion_level", C.c_int), ("merge_alpha", C.c_float), ("merge_sigma", C.c_float),
                 ("moi_gen_origin_host", C.c_void_p), ("ff_weighted_com_host", C.c_void_p), ("norm_mean_host", C.c_void_p),
                 ("norm_mad_host", C.c_void_p)]
+
+
+class FragmentJobs(C.Structure):
+    _fields_ = [("mode", C.c_int), ("n_jobs", C.c_int), ("job_of_sample_host", C.c_void_p), ("n_ff_host", C.c_void_p),
+                ("ff_x_host", C.c_void_p), ("ff_h_host", C.c_void_p), ("diffusion_level", C.c_int),
+                ("merge_alpha", C.c_float), ("merge_sigma", C.c_float), ("moi_gen_origin_host", C.c_void_p),
+                ("ff_weighted_com_host", C.c_void_p), ("norm_mean_host", C.c_void_p), ("norm_mad_host", C.c_void_p)]
 
 
 STAMP_PATH = LIB_PATH + ".stamp"
@@ -118,12 +125,16 @@ def load() -> C.CDLL:
                                   C.c_int64, vp, vp, vp, vp, vp]
     lib.mlcg_generate_fragment.argtypes = [vp, C.POINTER(Fragment), vp, ci, ci, vp, ci, C.POINTER(StepScalars), ci, cf, cf,
                                            cf, C.c_uint64, C.c_int64, vp, vp, vp, vp, vp]
+    lib.mlcg_generate_fragment_jobs.argtypes = [vp, C.POINTER(FragmentJobs), vp, ci, ci, vp, ci, C.POINTER(StepScalars), ci,
+                                                cf, cf, cf, C.c_uint64, C.c_int64, vp, vp, vp, vp, vp]
     lib.mlcg_nonfinite.argtypes = [vp, vp]
     lib.mlcg_num_edge_tiles.argtypes = [vp]
     lib.mlcg_num_edges.argtypes = [vp]
     lib.mlcg_num_edges.restype = C.c_int64
     lib.mlcg_kernel_launches.argtypes = [vp]
     lib.mlcg_kernel_launches.restype = C.c_int64
+    lib.mlcg_graph_captures.argtypes = [vp]
+    lib.mlcg_graph_captures.restype = C.c_int64
     lib.mlcg_time_edge_kernel.argtypes = [vp, ci, ci, vp]
     lib.mlcg_time_edge_kernel.restype = cf
     lib.mlcg_edge_phase_profile.argtypes = [vp, ci, C.POINTER(C.c_double), vp]

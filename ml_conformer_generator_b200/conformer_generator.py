@@ -9,6 +9,7 @@ entry points `edm_sample_tensors` / `generate_tensors` cover the accelerated pat
 import os
 from typing import Dict, List, Optional, Tuple
 
+import numpy as np
 import torch
 
 from .config import (ATOM_DECODER, CONTEXT_NORMS, DIMENSION, MAX_N_NODES, MIN_N_NODES, NUM_BOND_TYPES)
@@ -227,6 +228,30 @@ class MLConformerGenerator:
                              ifm_diffusion_level)
         pipe = GenerationPipeline(gen, postprocess or sdf_postprocess, n_workers=n_workers)
         yield from pipe.run(len(nn))
+
+    @torch.no_grad()
+    def generate_jobs(self, jobs: List[Dict], resample_steps: int = 0, blend_power: int = 3, ifm_diffusion_level: int = 50,
+                      seed: int = 0, max_batch: int = 8192) -> List[Dict[str, torch.Tensor]]:
+        """Many small generation jobs -- different references, atom counts and fixed fragments -- in few packed device
+        calls (the GPU reaches its rate only with thousands of molecules per call).  A job is a dict:
+          reference_context   raw principal moments (3)
+          n_atoms, variance   atom counts uniform in [n_atoms - variance, n_atoms + variance] (variance default 2, clipped
+                              to [min_n_nodes, max_n_nodes]), or
+          n_nodes             explicit atom count of every sample
+          n_samples           number of molecules (implied by n_nodes)
+          fixed_fragment      optional (coordinates (n,3), one-hot (n,8)), as in edm_sample_tensors
+          inertial_fragment_matching   default True
+          job_id              default: the job's position in the list
+        Jobs are grouped by kind (plain / inpainting / inertial fragment matching) and cut into calls of at most
+        `max_batch` samples; the loop settings are shared.  A job's molecules depend only on `seed`, its job_id, its own
+        fields and the shared settings (jobs.py), never on the other jobs or their order.  Returns one dict per job, in
+        input order, of host tensors: x (n,N,3), atom_class (n,N) (-1 = padding), n_nodes (n,), bonds (n,42,42) (the
+        provisional bond orders of generate_tensors), with N the job's own max atom count."""
+        from .jobs import flatten_jobs, run_packed, split_jobs
+        packed = flatten_jobs(jobs, seed, self.context_norms, self.min_n_nodes, self.max_n_nodes)
+        out = run_packed(self.engine, packed, np.arange(packed.ids.size), self.generative_model.T, resample_steps,
+                         blend_power, ifm_diffusion_level, seed, max_batch, context_norms=self.context_norms)
+        return split_jobs(packed, *out)
 
     # ------------------------------------------------------------------------------------------------------------
     # RDKit-facing path, same signatures as the reference

@@ -102,8 +102,10 @@ struct mlcg_handle {
   DevBuf s_ld, s_la, s_rowd, s_rowa, s_x64, s_y_op, s_x, s_emb, s_add, s_raw, s_y_f32;
   // mlcg_generate device buffers
   DevBuf g_ctx, g_z, g_x, g_cls, g_el, g_dist, g_adj, g_bonds, g_ids;
-  // mlcg_generate_fragment device buffers: fragment, z_known / fixed_mask, and the first IFM loop's context and outputs
-  DevBuf f_ffx, f_ffh, f_zk, f_fm, f_ctx, f_shift, f_rot, f_ngen, f_xg, f_clsg;
+  // mlcg_generate_fragment(_jobs) device buffers: packed fragments, job table, job of every sample, z_known / fixed_mask,
+  // and the first IFM loop's context and outputs
+  DevBuf f_ffx, f_ffh, f_jobs, f_job, f_zk, f_fm, f_ctx, f_shift, f_rot, f_ngen, f_xg, f_clsg;
+  DevBuf hook_job;  // the one-job table of the eager hooks mlcg_ifm_context / mlcg_ifm_merge_inputs
   DevBuf nf_flag;  // set by k_decode when a generated coordinate is not finite (mlcg_nonfinite)
   std::vector<int64_t> ids_stage;
   // test gemm
@@ -115,6 +117,7 @@ struct mlcg_handle {
   std::vector<long long> gen_key;  // geometry / schedule the graph was captured for
   int gen_key_hits = 0;            // calls seen with the current key (1st runs eagerly, 2nd captures)
   long long gen_graph_launches = 0;
+  long long graph_captures = 0;    // CUDA graphs captured by mlcg_generate / mlcg_generate_fragment(_jobs)
   cudaStream_t own_stream = nullptr;  // used by mlcg_generate when the caller passes the NULL stream (not capturable)
   // mlcg_egnn_forward_breakdown: events recorded after every launch of one forward, tagged with a kernel class
   bool bd_on = false;
@@ -448,7 +451,7 @@ extern "C" void mlcg_destroy(mlcg_handle* h) {
                     &h->h_res, &h->pq, &h->h_op, &h->agg_op, &h->t_op, &h->agg_f32, &h->t_f32, &h->a1, &h->m2, &h->t_dev,
                     &h->eps_dev, &h->s_ld, &h->s_la, &h->s_rowd, &h->s_rowa, &h->s_x64, &h->s_y_op, &h->s_x, &h->s_emb,
                     &h->s_add, &h->s_raw, &h->s_y_f32, &h->g_ctx, &h->g_z, &h->g_x, &h->g_cls, &h->g_el, &h->g_dist,
-                    &h->g_adj, &h->g_bonds, &h->g_ids, &h->f_ffx, &h->f_ffh, &h->f_zk, &h->f_fm, &h->f_ctx, &h->f_shift,
+                    &h->g_adj, &h->g_bonds, &h->g_ids, &h->f_ffx, &h->f_ffh, &h->f_jobs, &h->f_job, &h->hook_job, &h->f_zk, &h->f_fm, &h->f_ctx, &h->f_shift,
                     &h->f_rot, &h->f_ngen, &h->f_xg, &h->f_clsg, &h->nf_flag, &h->tg_a, &h->tg_w, &h->tg_b, &h->tg_c})
     b->release();
   delete h;
@@ -840,6 +843,7 @@ extern "C" int mlcg_nonfinite(mlcg_handle* h, void* stream) {
 extern "C" int mlcg_num_edge_tiles(mlcg_handle* h) { return h ? h->pl->n_etiles : -1; }
 extern "C" int64_t mlcg_num_edges(mlcg_handle* h) { return h ? h->pl->n_edges : -1; }
 extern "C" int64_t mlcg_kernel_launches(mlcg_handle* h) { return h ? h->launches : -1; }
+extern "C" int64_t mlcg_graph_captures(mlcg_handle* h) { return h ? h->graph_captures : -1; }
 
 // ---------------------------------------------------------------------------------------------------------------
 // EGNN forward
@@ -1416,6 +1420,7 @@ static int generate_graphed(mlcg_handle* h, const std::vector<long long>& key, c
       if (ce != cudaSuccess) h->gen_graph = nullptr;
     }
     if (graph) cudaGraphDestroy(graph);
+    if (h->gen_graph != nullptr) h->graph_captures++;
     h->gen_graph_launches = h->launches - launches0;
     h->launches = launches0;  // nothing has run yet
     if (rc != MLCG_OK || h->gen_graph == nullptr) {
@@ -1469,23 +1474,25 @@ extern "C" int mlcg_generate(mlcg_handle* h, const int32_t* n_nodes_host, int B,
 // (MLConformerGenerator.edm_sample_tensors: two mlcg_sample calls) does, which this path reproduces bit for bit.
 static const uint64_t kMergeDrawBase = 0;
 
-// The device part of mlcg_generate_fragment (see mlcg.h): the launch sequence of the eager composition, on plan 0 (whole
-// molecules) and -- mode 2 -- plan 1 (the atoms still to be generated).  The plan switches happen on the host between
-// launches; each launch bakes in the pointers of its plan, so one captured graph holds both loops.
-static int generate_fragment_device(mlcg_handle* h, int mode, int n_ff, const IfmArgs& ifm, int T,
+// The device part of mlcg_generate_fragment_jobs (see mlcg.h): the launch sequence of the eager composition, on plan 0
+// (whole molecules) and -- mode 2 -- plan 1 (the atoms still to be generated, stride Ng).  The plan switches happen on the
+// host between launches; each launch bakes in the pointers of its plan, so one captured graph holds both loops.
+static int generate_fragment_device(mlcg_handle* h, int mode, int Ng, const IfmNorms& nrm, int T,
                                     const mlcg_step_scalars* steps, int resample_steps, int diffusion_level, float merge_alpha,
                                     float merge_sigma, float sigma_0, float alpha_0, float sigma_x, uint64_t seed,
                                     int64_t sample_offset, void* stream) {
   cudaStream_t st = (cudaStream_t)stream;
   const int B = h->plans[0].B, N = h->plans[0].N;
   const int64_t* ids = h->g_ids.as<int64_t>();
+  const int* job = h->f_job.as<int>();
+  const FragJob* jobs = h->f_jobs.as<FragJob>();
   float* zk = h->f_zk.as<float>();
   float* fm = h->f_fm.as<float>();
   int rc;
   if (mode == 1) {
     // z_known / fixed_mask of EquivariantDiffusion.inpaint (prepare_fragment): the merge-input kernel with no generated atoms
-    k_ifm_merge_inputs<<<B, 64, 0, st>>>(nullptr, nullptr, nullptr, nullptr, h->f_ffx.as<float>(), h->f_ffh.as<float>(), n_ff,
-                                         0, N, zk, fm);
+    k_ifm_merge_inputs<<<B, 64, 0, st>>>(nullptr, nullptr, nullptr, nullptr, h->f_ffx.as<float>(), h->f_ffh.as<float>(), job,
+                                         jobs, 0, N, zk, fm);
     KCHECK();
     rc = sample_loop(h, 1, T, steps, resample_steps, diffusion_level, 0.f, 0.f, sigma_0, alpha_0, sigma_x, h->g_ctx.as<float>(),
                      zk, fm, nullptr, seed, sample_offset, ids, h->g_z.as<float>(), h->g_x.as<float>(), h->g_cls.as<int32_t>(),
@@ -1494,7 +1501,7 @@ static int generate_fragment_device(mlcg_handle* h, int mode, int n_ff, const If
     return seer_device(h, stream);
   }
   // inertial fragment matching: per-sample context of the atoms still to be generated ...
-  k_ifm_context<<<(B + 127) / 128, 128, 0, st>>>(h->plans[0].d_n_nodes.as<int>(), B, ifm, h->f_ctx.as<float>(),
+  k_ifm_context<<<(B + 127) / 128, 128, 0, st>>>(h->plans[0].d_n_nodes.as<int>(), job, jobs, B, nrm, h->f_ctx.as<float>(),
                                                  h->f_shift.as<float>(), h->f_rot.as<float>(), h->f_ngen.as<int>());
   KCHECK();
   // ... generated on their own (plan 1) ...
@@ -1506,7 +1513,7 @@ static int generate_fragment_device(mlcg_handle* h, int mode, int n_ff, const If
   if (rc) return rc;
   // ... moved back to the reference frame next to the fixed fragment, and merged with it (plan 0)
   k_ifm_merge_inputs<<<B, 64, 0, st>>>(h->f_xg.as<float>(), h->f_clsg.as<int32_t>(), h->f_shift.as<float>(), h->f_rot.as<float>(),
-                                       h->f_ffx.as<float>(), h->f_ffh.as<float>(), n_ff, N - n_ff, N, zk, fm);
+                                       h->f_ffx.as<float>(), h->f_ffh.as<float>(), job, jobs, Ng, N, zk, fm);
   KCHECK();
   rc = sample_loop(h, 2, T, steps, resample_steps, diffusion_level, merge_alpha, merge_sigma, sigma_0, alpha_0, sigma_x,
                    h->g_ctx.as<float>(), zk, fm, nullptr, seed, sample_offset, ids, h->g_z.as<float>(), h->g_x.as<float>(),
@@ -1515,60 +1522,84 @@ static int generate_fragment_device(mlcg_handle* h, int mode, int n_ff, const If
   return seer_device(h, stream);
 }
 
-extern "C" int mlcg_generate_fragment(mlcg_handle* h, const mlcg_fragment* frag, const int32_t* n_nodes_host, int B, int N,
-                                      const float* ctx_host, int T, const mlcg_step_scalars* steps, int resample_steps,
-                                      float sigma_0, float alpha_0, float sigma_x, uint64_t seed, int64_t sample_offset,
-                                      const int64_t* sample_ids_host, float* x_out, int32_t* atom_class_out, int8_t* bonds_out,
-                                      void* stream) {
+extern "C" int mlcg_generate_fragment_jobs(mlcg_handle* h, const mlcg_fragment_jobs* fj, const int32_t* n_nodes_host, int B,
+                                           int N, const float* ctx_host, int T, const mlcg_step_scalars* steps,
+                                           int resample_steps, float sigma_0, float alpha_0, float sigma_x, uint64_t seed,
+                                           int64_t sample_offset, const int64_t* sample_ids_host, float* x_out,
+                                           int32_t* atom_class_out, int8_t* bonds_out, void* stream) {
   if (!h) return MLCG_E_ARG;
   if (!h->egnn_loaded || !h->seer_loaded) FAIL(MLCG_E_ARG, "generate_fragment: load both weight sets first");
-  if (!frag || !n_nodes_host || !ctx_host || !steps || !x_out || !atom_class_out || !bonds_out || !frag->ff_x_host ||
-      !frag->ff_h_host)
+  if (!fj || !n_nodes_host || !ctx_host || !steps || !x_out || !atom_class_out || !bonds_out || !fj->job_of_sample_host ||
+      !fj->n_ff_host || !fj->ff_x_host || !fj->ff_h_host)
     FAIL(MLCG_E_ARG, "generate_fragment: null pointer");
-  const int mode = frag->mode, n_ff = frag->n_ff;
+  const int mode = fj->mode, n_jobs = fj->n_jobs;
   if (mode != 1 && mode != 2) FAIL(MLCG_E_ARG, "generate_fragment: mode must be 1 (inpaint) or 2 (inertial fragment matching)");
-  if (mode == 2 && (!frag->moi_gen_origin_host || !frag->ff_weighted_com_host || !frag->norm_mean_host || !frag->norm_mad_host))
+  if (mode == 2 && (!fj->moi_gen_origin_host || !fj->ff_weighted_com_host || !fj->norm_mean_host || !fj->norm_mad_host))
     FAIL(MLCG_E_ARG, "generate_fragment: null pointer (inertial fragment matching needs the moment-of-inertia prologue)");
-  if (B <= 0 || N <= 0 || N > EDGE_MAXN || T <= 0 || resample_steps < 0)
-    FAIL(MLCG_E_ARG, "generate_fragment: need B > 0, 1 <= N <= 39, T > 0 and resample_steps >= 0");
-  if (n_ff < 1) FAIL(MLCG_E_ARG, "generate_fragment: the fragment needs at least one atom");
-  if (N - n_ff < 1) FAIL(MLCG_E_ARG, "generate_fragment: the fragment must have fewer atoms than N");
-  int min_n = N;
-  for (int b = 0; b < B; ++b) min_n = std::min(min_n, (int)n_nodes_host[b]);
-  if (n_ff >= min_n) FAIL(MLCG_E_ARG, "generate_fragment: the fragment must have fewer atoms than every sample");
-  IfmArgs ifm{};
-  std::vector<int32_t> n_gen;
-  if (mode == 2) {
-    memcpy(ifm.moi0, frag->moi_gen_origin_host, sizeof(ifm.moi0));
-    memcpy(ifm.ffsum, frag->ff_weighted_com_host, sizeof(ifm.ffsum));
-    memcpy(ifm.mean, frag->norm_mean_host, sizeof(ifm.mean));
-    memcpy(ifm.mad, frag->norm_mad_host, sizeof(ifm.mad));
-    ifm.n_ff = n_ff;
-    n_gen.resize(B);
-    for (int b = 0; b < B; ++b) n_gen[b] = n_nodes_host[b] - n_ff;
+  if (B <= 0 || N <= 0 || N > EDGE_MAXN || T <= 0 || resample_steps < 0 || n_jobs < 1)
+    FAIL(MLCG_E_ARG, "generate_fragment: need B > 0, 1 <= N <= 39, T > 0, resample_steps >= 0 and n_jobs >= 1");
+  // the job table: each job's fragment rows in the packed ff_x / ff_h and its prologue
+  std::vector<FragJob> jobs((size_t)n_jobs);
+  int n_ff_total = 0;
+  for (int j = 0; j < n_jobs; ++j) {
+    const int n_ff = fj->n_ff_host[j];
+    if (n_ff < 1) FAIL(MLCG_E_ARG, "generate_fragment: the fragment needs at least one atom (job " + std::to_string(j) + ")");
+    if (N - n_ff < 1) FAIL(MLCG_E_ARG, "generate_fragment: the fragment must have fewer atoms than N (job " + std::to_string(j) + ")");
+    FragJob& q = jobs[j];
+    q.n_ff = n_ff;
+    q.ff_off = n_ff_total;
+    n_ff_total += n_ff;
+    if (mode == 2) {
+      memcpy(q.moi0, fj->moi_gen_origin_host + (size_t)j * 9, sizeof(q.moi0));
+      memcpy(q.ffsum, fj->ff_weighted_com_host + (size_t)j * 3, sizeof(q.ffsum));
+    }
   }
-  // Key of the captured graph.  It starts with -mode, so it never equals a key of mlcg_generate (which starts with B).
-  // Mode 2 adds what is baked into kernel arguments beyond mlcg_generate's key: the merge level and its scalars, and the
-  // moment-of-inertia prologue k_ifm_context takes by value.  The fragment itself is uploaded on every call.
+  // per sample: its job's fragment size, which must leave at least one atom to generate
+  std::vector<int32_t> n_ff_of((size_t)B), n_gen;
+  int min_n_ff = N;
+  for (int b = 0; b < B; ++b) {
+    const int j = fj->job_of_sample_host[b];
+    if (j < 0 || j >= n_jobs) FAIL(MLCG_E_ARG, "generate_fragment: job index out of range (sample " + std::to_string(b) + ")");
+    n_ff_of[b] = jobs[j].n_ff;
+    if (n_ff_of[b] >= n_nodes_host[b])
+      FAIL(MLCG_E_ARG, "generate_fragment: the fragment must have fewer atoms than every sample (sample " + std::to_string(b) + ")");
+    min_n_ff = std::min(min_n_ff, (int)n_ff_of[b]);
+  }
+  // first IFM loop: the atoms still to be generated, padded to the longest of them
+  const int Ng = N - min_n_ff;
+  IfmNorms nrm{};
+  if (mode == 2) {
+    memcpy(nrm.mean, fj->norm_mean_host, sizeof(nrm.mean));
+    memcpy(nrm.mad, fj->norm_mad_host, sizeof(nrm.mad));
+    n_gen.resize(B);
+    for (int b = 0; b < B; ++b) n_gen[b] = n_nodes_host[b] - n_ff_of[b];
+  }
+  // Key of the captured graph: the geometry and every scalar baked into kernel arguments.  It starts with -mode, so it
+  // never equals a key of mlcg_generate (which starts with B).  The job count and the packed fragment length fix the sizes
+  // of the buffers the graph reads.  The fragments, the job table, the job of every sample, the context, the ids and
+  // {seed, sample_offset} are uploaded on every call, so a replay with other references or fragments of the same sizes
+  // reuses the graph and never sees a previous call's inputs.
   std::vector<long long> key;
-  key.reserve((size_t)B + 8 * (size_t)T + 48);
+  key.reserve(2 * (size_t)B + 7 * (size_t)T + 32);
   key.push_back(-mode); key.push_back(B); key.push_back(N); key.push_back(T); key.push_back(resample_steps);
-  key.push_back(h->precision); key.push_back(n_ff);
+  key.push_back(h->precision); key.push_back(n_jobs); key.push_back(n_ff_total);
   key.push_back(fbits(sigma_0)); key.push_back(fbits(alpha_0)); key.push_back(fbits(sigma_x));
   if (mode == 2) {
-    key.push_back(frag->diffusion_level); key.push_back(fbits(frag->merge_alpha)); key.push_back(fbits(frag->merge_sigma));
-    const float* pro = reinterpret_cast<const float*>(&ifm);
-    for (size_t k = 0; k < offsetof(IfmArgs, n_ff) / sizeof(float); ++k) key.push_back(fbits(pro[k]));
+    key.push_back(fj->diffusion_level); key.push_back(fbits(fj->merge_alpha)); key.push_back(fbits(fj->merge_sigma));
+    for (int c = 0; c < 3; ++c) { key.push_back(fbits(nrm.mean[c])); key.push_back(fbits(nrm.mad[c])); }
   }
   for (int b = 0; b < B; ++b) key.push_back(n_nodes_host[b]);
+  for (int b = 0; b < B; ++b) key.push_back(n_ff_of[b]);
   for (int s = 0; s < T; ++s) {
     const mlcg_step_scalars& c = steps[s];
     for (float v : {c.t, c.alpha_ts, c.c_eps, c.c_sigma, c.alpha_s, c.sigma_s, c.blend}) key.push_back(fbits(v));
   }
-  const size_t bn = (size_t)B * N, bg = (size_t)B * (N - n_ff);
+  const size_t bn = (size_t)B * N, bg = (size_t)B * Ng;
   auto upload = [&](cudaStream_t st) -> int {
-    CK(h->f_ffx.ensure((size_t)n_ff * 3 * 4));
-    CK(h->f_ffh.ensure((size_t)n_ff * 8 * 4));
+    CK(h->f_ffx.ensure((size_t)n_ff_total * 3 * 4));
+    CK(h->f_ffh.ensure((size_t)n_ff_total * 8 * 4));
+    CK(h->f_jobs.ensure((size_t)n_jobs * sizeof(FragJob)));
+    CK(h->f_job.ensure((size_t)B * 4));
     CK(h->f_zk.ensure(bn * ZC * 4));
     CK(h->f_fm.ensure(bn * 4));
     if (mode == 2) {
@@ -1579,18 +1610,47 @@ extern "C" int mlcg_generate_fragment(mlcg_handle* h, const mlcg_fragment* frag,
       CK(h->f_xg.ensure(bg * 3 * 4));
       CK(h->f_clsg.ensure(bg * 4));
     }
-    CK(cudaMemcpyAsync(h->f_ffx.p, frag->ff_x_host, (size_t)n_ff * 3 * 4, cudaMemcpyHostToDevice, st));
-    CK(cudaMemcpyAsync(h->f_ffh.p, frag->ff_h_host, (size_t)n_ff * 8 * 4, cudaMemcpyHostToDevice, st));
+    CK(cudaMemcpyAsync(h->f_ffx.p, fj->ff_x_host, (size_t)n_ff_total * 3 * 4, cudaMemcpyHostToDevice, st));
+    CK(cudaMemcpyAsync(h->f_ffh.p, fj->ff_h_host, (size_t)n_ff_total * 8 * 4, cudaMemcpyHostToDevice, st));
+    CK(cudaMemcpyAsync(h->f_jobs.p, jobs.data(), (size_t)n_jobs * sizeof(FragJob), cudaMemcpyHostToDevice, st));
+    CK(cudaMemcpyAsync(h->f_job.p, fj->job_of_sample_host, (size_t)B * 4, cudaMemcpyHostToDevice, st));
     return MLCG_OK;
   };
-  const int diffusion_level = mode == 2 ? frag->diffusion_level : 0;
-  const float merge_alpha = mode == 2 ? frag->merge_alpha : 0.f, merge_sigma = mode == 2 ? frag->merge_sigma : 0.f;
-  return generate_graphed(h, key, n_nodes_host, B, N, mode == 2 ? n_gen.data() : nullptr, N - n_ff, ctx_host, seed,
-                          sample_offset, sample_ids_host, x_out, atom_class_out, bonds_out, stream, upload, [&](void* s) {
-                            return generate_fragment_device(h, mode, n_ff, ifm, T, steps, resample_steps, diffusion_level,
+  const int diffusion_level = mode == 2 ? fj->diffusion_level : 0;
+  const float merge_alpha = mode == 2 ? fj->merge_alpha : 0.f, merge_sigma = mode == 2 ? fj->merge_sigma : 0.f;
+  return generate_graphed(h, key, n_nodes_host, B, N, mode == 2 ? n_gen.data() : nullptr, Ng, ctx_host, seed, sample_offset,
+                          sample_ids_host, x_out, atom_class_out, bonds_out, stream, upload, [&](void* s) {
+                            return generate_fragment_device(h, mode, Ng, nrm, T, steps, resample_steps, diffusion_level,
                                                             merge_alpha, merge_sigma, sigma_0, alpha_0, sigma_x, seed,
                                                             sample_offset, s);
                           });
+}
+
+// One fragment for every sample: the one-job case of mlcg_generate_fragment_jobs.
+extern "C" int mlcg_generate_fragment(mlcg_handle* h, const mlcg_fragment* frag, const int32_t* n_nodes_host, int B, int N,
+                                      const float* ctx_host, int T, const mlcg_step_scalars* steps, int resample_steps,
+                                      float sigma_0, float alpha_0, float sigma_x, uint64_t seed, int64_t sample_offset,
+                                      const int64_t* sample_ids_host, float* x_out, int32_t* atom_class_out, int8_t* bonds_out,
+                                      void* stream) {
+  if (!h) return MLCG_E_ARG;
+  if (!frag) FAIL(MLCG_E_ARG, "generate_fragment: null pointer");
+  std::vector<int32_t> job_of_sample((size_t)std::max(B, 1), 0);  // never empty: B <= 0 fails the B check
+  mlcg_fragment_jobs fj{};
+  fj.mode = frag->mode;
+  fj.n_jobs = 1;
+  fj.job_of_sample_host = job_of_sample.data();
+  fj.n_ff_host = &frag->n_ff;
+  fj.ff_x_host = frag->ff_x_host;
+  fj.ff_h_host = frag->ff_h_host;
+  fj.diffusion_level = frag->diffusion_level;
+  fj.merge_alpha = frag->merge_alpha;
+  fj.merge_sigma = frag->merge_sigma;
+  fj.moi_gen_origin_host = frag->moi_gen_origin_host;
+  fj.ff_weighted_com_host = frag->ff_weighted_com_host;
+  fj.norm_mean_host = frag->norm_mean_host;
+  fj.norm_mad_host = frag->norm_mad_host;
+  return mlcg_generate_fragment_jobs(h, &fj, n_nodes_host, B, N, ctx_host, T, steps, resample_steps, sigma_0, alpha_0,
+                                     sigma_x, seed, sample_offset, sample_ids_host, x_out, atom_class_out, bonds_out, stream);
 }
 
 // ---------------------------------------------------------------------------------------------------------------
@@ -1715,13 +1775,18 @@ extern "C" int mlcg_ifm_context(mlcg_handle* h, const float* moi_gen_origin_host
   if (!moi_gen_origin_host || !ff_weighted_com_host || !norm_mean_host || !norm_mad_host || !n_nodes || !ctx_out || !shift_out ||
       !rot_out || !n_gen_out || B <= 0 || n_ff <= 0)
     FAIL(MLCG_E_ARG, "ifm_context: bad argument");
-  IfmArgs a{};
-  memcpy(a.moi0, moi_gen_origin_host, sizeof(a.moi0));
-  memcpy(a.ffsum, ff_weighted_com_host, sizeof(a.ffsum));
-  memcpy(a.mean, norm_mean_host, sizeof(a.mean));
-  memcpy(a.mad, norm_mad_host, sizeof(a.mad));
-  a.n_ff = n_ff;
-  k_ifm_context<<<(B + 127) / 128, 128, 0, (cudaStream_t)stream>>>(n_nodes, B, a, ctx_out, shift_out, rot_out, n_gen_out);
+  FragJob q{};
+  memcpy(q.moi0, moi_gen_origin_host, sizeof(q.moi0));
+  memcpy(q.ffsum, ff_weighted_com_host, sizeof(q.ffsum));
+  q.n_ff = n_ff;
+  IfmNorms nrm{};
+  memcpy(nrm.mean, norm_mean_host, sizeof(nrm.mean));
+  memcpy(nrm.mad, norm_mad_host, sizeof(nrm.mad));
+  cudaStream_t st = (cudaStream_t)stream;
+  CK(h->hook_job.ensure(sizeof(FragJob)));
+  CK(cudaMemcpyAsync(h->hook_job.p, &q, sizeof(q), cudaMemcpyHostToDevice, st));
+  k_ifm_context<<<(B + 127) / 128, 128, 0, st>>>(n_nodes, nullptr, h->hook_job.as<FragJob>(), B, nrm, ctx_out, shift_out,
+                                                 rot_out, n_gen_out);
   KCHECK();
   return MLCG_OK;
 }
@@ -1733,7 +1798,13 @@ extern "C" int mlcg_ifm_merge_inputs(mlcg_handle* h, const float* x_gen, const i
   if (!x_gen || !cls_gen || !shift || !rot || !ff_x || !ff_h || !z_known || !fixed_mask || B <= 0 || n_ff <= 0 || Ng <= 0 ||
       N < n_ff || N > 64)
     FAIL(MLCG_E_ARG, "ifm_merge_inputs: bad argument");
-  k_ifm_merge_inputs<<<B, 64, 0, (cudaStream_t)stream>>>(x_gen, cls_gen, shift, rot, ff_x, ff_h, n_ff, Ng, N, z_known, fixed_mask);
+  FragJob q{};
+  q.n_ff = n_ff;
+  cudaStream_t st = (cudaStream_t)stream;
+  CK(h->hook_job.ensure(sizeof(FragJob)));
+  CK(cudaMemcpyAsync(h->hook_job.p, &q, sizeof(q), cudaMemcpyHostToDevice, st));
+  k_ifm_merge_inputs<<<B, 64, 0, st>>>(x_gen, cls_gen, shift, rot, ff_x, ff_h, nullptr, h->hook_job.as<FragJob>(), Ng, N, z_known,
+                                       fixed_mask);
   KCHECK();
   return MLCG_OK;
 }

@@ -10,11 +10,17 @@
 
 namespace mlcg {
 
-struct IfmArgs {
+// One job of a fragment call (mlcg_generate_fragment_jobs): its fixed fragment's rows in the packed ff_x / ff_h and,
+// for inertial fragment matching, the per-job part of the moment-of-inertia prologue.  Sample b reads jobs[job[b]].
+struct FragJob {
   float moi0[9];   // diag(reference context) - MOI(fixed fragment): the generated fragment's MOI about the origin
   float ffsum[3];  // n_ff * mean(fixed fragment coordinates)
-  float mean[3], mad[3];  // context normalisation (utils/config.py CONTEXT_NORMS)
-  int n_ff;
+  int n_ff;        // fixed atoms
+  int ff_off;      // row of the fragment's first atom in the packed ff_x / ff_h
+};
+
+struct IfmNorms {
+  float mean[3], mad[3];  // context normalisation (utils/config.py CONTEXT_NORMS), shared by all jobs
 };
 
 // Symmetric 3x3 eigen-decomposition, cyclic Jacobi in double precision (converges to machine precision in <= 6 sweeps
@@ -69,11 +75,14 @@ __device__ inline void eigh3(const double a_in[3][3], double w[3], double v[3][3
     for (int j = 0; j < 3; ++j) v[i][j] = vs[i][j];
 }
 
-// one thread per sample.  n_nodes: total atoms of the sample (fixed + generated).
-__global__ void k_ifm_context(const int* __restrict__ n_nodes, int B, IfmArgs p, float* __restrict__ ctx_out,
-                              float* __restrict__ shift_out, float* __restrict__ rot_out, int* __restrict__ n_gen_out) {
+// one thread per sample.  n_nodes: total atoms of the sample (fixed + generated); job (B): the sample's entry of `jobs`
+// (nullptr: every sample reads jobs[0]).
+__global__ void k_ifm_context(const int* __restrict__ n_nodes, const int* __restrict__ job, const FragJob* __restrict__ jobs,
+                              int B, IfmNorms nrm, float* __restrict__ ctx_out, float* __restrict__ shift_out,
+                              float* __restrict__ rot_out, int* __restrict__ n_gen_out) {
   const int b = blockIdx.x * blockDim.x + threadIdx.x;
   if (b >= B) return;
+  const FragJob p = jobs[job ? job[b] : 0];
   const float n_gen = (float)(n_nodes[b] - p.n_ff);
   // shift = (n_ff * mean(ff_x)) / n_gen   (reference :411-412; fp32 as there)
   float s[3];
@@ -89,27 +98,32 @@ __global__ void k_ifm_context(const int* __restrict__ n_nodes, int B, IfmArgs p,
   double w[3], v[3][3];
   eigh3(m, w, v);
   for (int c = 0; c < 3; ++c) {
-    ctx_out[b * 3 + c] = __fdiv_rn(__fsub_rn((float)w[c], p.mean[c]), p.mad[c]);
+    ctx_out[b * 3 + c] = __fdiv_rn(__fsub_rn((float)w[c], nrm.mean[c]), nrm.mad[c]);
     shift_out[b * 3 + c] = s[c];
     for (int k = 0; k < 3; ++k) rot_out[b * 9 + k * 3 + c] = (float)v[k][c];
   }
   n_gen_out[b] = n_nodes[b] - p.n_ff;
 }
 
-// z_known (B,N,11) and fixed_mask (B,N) of the merge loop.  Atom i < n_ff: the fixed fragment (coordinates + raw 0/1
-// one-hot).  Atom n_ff + j: generated atom j of the first loop moved back to the reference frame, x R^T - shift, with the
-// one-hot of its class.  As in the reference, padded generated rows (x = 0) come out as -shift with an all-zero one-hot.
+// z_known (B,N,11) and fixed_mask (B,N) of the merge loop.  Sample b has the fixed fragment of jobs[job[b]] (nullptr: of
+// jobs[0]): n_ff atoms at rows ff_off.. of the packed ff_x / ff_h.  Atom i < n_ff: the fixed fragment (coordinates + raw
+// 0/1 one-hot).  Atom n_ff + j (j < Ng, the packed stride of x_gen / cls_gen): generated atom j of the first loop moved
+// back to the reference frame, x R^T - shift, with the one-hot of its class.  As in the reference, padded generated rows
+// (x = 0) come out as -shift with an all-zero one-hot.
 __global__ void k_ifm_merge_inputs(const float* __restrict__ x_gen, const int* __restrict__ cls_gen, const float* __restrict__ shift,
                                    const float* __restrict__ rot, const float* __restrict__ ff_x, const float* __restrict__ ff_h,
-                                   int n_ff, int Ng, int N, float* __restrict__ z_known, float* __restrict__ fixed_mask) {
+                                   const int* __restrict__ job, const FragJob* __restrict__ jobs, int Ng, int N,
+                                   float* __restrict__ z_known, float* __restrict__ fixed_mask) {
   const int b = blockIdx.x;
+  const int jb = job ? job[b] : 0;
+  const int n_ff = jobs[jb].n_ff, ff_off = jobs[jb].ff_off;
   for (int i = threadIdx.x; i < N; i += blockDim.x) {
     float out[ZC];
 #pragma unroll
     for (int c = 0; c < ZC; ++c) out[c] = 0.f;
     if (i < n_ff) {
-      for (int c = 0; c < 3; ++c) out[c] = ff_x[i * 3 + c];
-      for (int c = 0; c < 8; ++c) out[3 + c] = ff_h[i * 8 + c];
+      for (int c = 0; c < 3; ++c) out[c] = ff_x[(size_t)(ff_off + i) * 3 + c];
+      for (int c = 0; c < 8; ++c) out[3 + c] = ff_h[(size_t)(ff_off + i) * 8 + c];
     } else if (i - n_ff < Ng) {
       const int j = i - n_ff;
       const float* xg = x_gen + ((size_t)b * Ng + j) * 3;

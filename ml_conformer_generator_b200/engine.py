@@ -311,33 +311,68 @@ class Engine:
         otherwise the fragment is inpainted.  `ctx` (B,3) is the normalised reference context of every sample.  Same
         outputs, noise keys and graph replay as generate_host; the result equals the eager composition of
         MLConformerGenerator.edm_sample_tensors + the GCN bit for bit."""
-        nn, ctxh, ids, out = self._host_call_inputs("generate_fragment_host", n_nodes, max_n_nodes, ctx, sample_ids, out,
-                                                    device_out)
+        return self._fragment_jobs_call("generate_fragment_host", n_nodes, max_n_nodes, ctx, np.zeros(np.size(n_nodes), np.int32),
+                                        [(fragment_x, fragment_h)], inertial_fragment_matching,
+                                        None if reference_context is None else [reference_context], context_norms, T,
+                                        resample_steps, blend_power, diffusion_level, seed, sample_offset, sample_ids, out,
+                                        device_out)
+
+    def generate_fragment_jobs_host(self, n_nodes: np.ndarray, max_n_nodes: int, ctx: np.ndarray, job_of_sample,
+                                    fragments, inertial_fragment_matching: bool = True, reference_contexts=None,
+                                    context_norms=None, T: int = 100, resample_steps: int = 0, blend_power: int = 3,
+                                    diffusion_level: int = 50, seed: int = 0, sample_offset: int = 0, sample_ids=None,
+                                    out=None, device_out: bool = False):
+        """generate_fragment_host for many fragment jobs of one mode in one call: sample b runs with the fragment
+        fragments[job_of_sample[b]] = (coordinates (n,3), one-hot (n,8)) and -- inertial fragment matching -- the raw
+        reference context reference_contexts[job_of_sample[b]].  `ctx` (B,3) is every sample's normalised context; the
+        loop settings are shared.  Same outputs, noise keys and graph replay as generate_fragment_host, and every sample
+        equals a call holding only its own job with the same sample id, bit for bit."""
+        return self._fragment_jobs_call("generate_fragment_jobs_host", n_nodes, max_n_nodes, ctx, job_of_sample, fragments,
+                                        inertial_fragment_matching, reference_contexts, context_norms, T, resample_steps,
+                                        blend_power, diffusion_level, seed, sample_offset, sample_ids, out, device_out)
+
+    def _fragment_jobs_call(self, what, n_nodes, max_n_nodes, ctx, job_of_sample, fragments, inertial_fragment_matching,
+                            reference_contexts, context_norms, T, resample_steps, blend_power, diffusion_level, seed,
+                            sample_offset, sample_ids, out, device_out):
+        nn, ctxh, ids, out = self._host_call_inputs(what, n_nodes, max_n_nodes, ctx, sample_ids, out, device_out)
         B, N = int(nn.size), int(max_n_nodes)
-        ffx = np.ascontiguousarray(torch.as_tensor(fragment_x).detach().cpu().numpy(), dtype=np.float32)
-        ffh = np.ascontiguousarray(torch.as_tensor(fragment_h).detach().cpu().numpy(), dtype=np.float32)
-        if ffx.ndim != 2 or ffx.shape[1] != 3 or ffh.shape != (ffx.shape[0], 8):
-            raise ValueError("generate_fragment_host: the fragment must be coordinates (n,3) and a one-hot (n,8)")
+        job = np.ascontiguousarray(np.asarray(job_of_sample, dtype=np.int32).reshape(-1))
+        if job.size != B:
+            raise ValueError("%s: job_of_sample must hold one job per sample" % what)
+        ffx, ffh = [], []
+        for fx, fh in fragments:
+            fx = np.asarray(torch.as_tensor(fx).detach().cpu().numpy(), dtype=np.float32)
+            fh = np.asarray(torch.as_tensor(fh).detach().cpu().numpy(), dtype=np.float32)
+            if fx.ndim != 2 or fx.shape[1] != 3 or fh.shape != (fx.shape[0], 8):
+                raise ValueError("%s: the fragment must be coordinates (n,3) and a one-hot (n,8)" % what)
+            ffx.append(fx)
+            ffh.append(fh)
+        n_ff = np.array([f.shape[0] for f in ffx], dtype=np.int32)
+        packed_x = np.ascontiguousarray(np.concatenate(ffx, axis=0).reshape(-1, 3), dtype=np.float32)
+        packed_h = np.ascontiguousarray(np.concatenate(ffh, axis=0).reshape(-1, 8), dtype=np.float32)
         gamma, steps = self._steps_cached(T, blend_power)
         dec = decode_scalars(gamma)
-        frag = _lib.Fragment(2 if inertial_fragment_matching else 1, int(ffx.shape[0]), ffx.ctypes.data, ffh.ctypes.data)
+        fj = _lib.FragmentJobs(2 if inertial_fragment_matching else 1, len(ffx), job.ctypes.data, n_ff.ctypes.data,
+                               packed_x.ctypes.data, packed_h.ctypes.data)
         keep = []
         if inertial_fragment_matching:
-            if reference_context is None:
-                raise ValueError("generate_fragment_host: inertial fragment matching needs the raw reference_context")
+            if reference_contexts is None or len(reference_contexts) != len(ffx):
+                raise ValueError("%s: inertial fragment matching needs the raw reference_context of every job" % what)
             from .config import CONTEXT_NORMS
             from .mol_utils import ifm_moi_prologue
             norms = CONTEXT_NORMS if context_norms is None else context_norms
-            moi0, com = ifm_moi_prologue(torch.from_numpy(ffx), reference_context)
-            keep = [moi0, com] + [torch.as_tensor(norms[k], dtype=torch.float32).contiguous() for k in ("mean", "mad")]
+            pro = [ifm_moi_prologue(torch.from_numpy(fx), ref) for fx, ref in zip(ffx, reference_contexts)]
+            keep = [torch.stack([p[0] for p in pro]).contiguous(), torch.stack([p[1] for p in pro]).contiguous()] + \
+                [torch.as_tensor(norms[k], dtype=torch.float32).contiguous() for k in ("mean", "mad")]
             lvl = forward_level_scalars(gamma, diffusion_level)
-            frag.diffusion_level, frag.merge_alpha, frag.merge_sigma = int(diffusion_level), lvl["alpha"], lvl["sigma"]
-            frag.moi_gen_origin_host, frag.ff_weighted_com_host, frag.norm_mean_host, frag.norm_mad_host = (
+            fj.diffusion_level, fj.merge_alpha, fj.merge_sigma = int(diffusion_level), lvl["alpha"], lvl["sigma"]
+            fj.moi_gen_origin_host, fj.ff_weighted_com_host, fj.norm_mean_host, fj.norm_mad_host = (
                 t.data_ptr() for t in keep)
-        rc = self.lib.mlcg_generate_fragment(self.h, C.byref(frag), nn.ctypes.data_as(C.c_void_p), B, N, _ptr(ctxh), T,
-                                             steps, resample_steps, dec["sigma_0"], dec["alpha_0"], dec["sigma_x"], seed,
-                                             sample_offset, None if ids is None else ids.ctypes.data_as(C.c_void_p),
-                                             _ptr(out[0]), _ptr(out[1]), _ptr(out[2]), self._stream())
+        rc = self.lib.mlcg_generate_fragment_jobs(self.h, C.byref(fj), nn.ctypes.data_as(C.c_void_p), B, N, _ptr(ctxh), T,
+                                                  steps, resample_steps, dec["sigma_0"], dec["alpha_0"], dec["sigma_x"],
+                                                  seed, sample_offset,
+                                                  None if ids is None else ids.ctypes.data_as(C.c_void_p), _ptr(out[0]),
+                                                  _ptr(out[1]), _ptr(out[2]), self._stream())
         del keep
         self._check(rc, "generate_fragment")
         self.check_finite("generate_fragment")
@@ -354,6 +389,10 @@ class Engine:
 
     def kernel_launches(self) -> int:
         return int(self.lib.mlcg_kernel_launches(self.h))
+
+    def graph_captures(self) -> int:
+        """CUDA graphs captured by the host calls since the engine was created (a replay leaves it unchanged)."""
+        return int(self.lib.mlcg_graph_captures(self.h))
 
     def time_edge_kernel(self, layer: int = 0, iters: int = 10) -> float:
         return float(self.lib.mlcg_time_edge_kernel(self.h, layer, iters, self._stream()))

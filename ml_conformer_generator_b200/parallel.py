@@ -128,3 +128,25 @@ def generate_sharded_engine(engine, n_nodes: Sequence[int], max_n_nodes: int, ct
         return engine.generate_host(nn, max_n_nodes, ctx[ids], T, resample_steps, seed=seed, sample_ids=ids, device_out=True)
 
     return generate_sharded(run_shard, n_nodes, max_n_nodes, group, max_batch, engine.device, stats)
+
+
+def generate_jobs_sharded(engine, jobs, T: int = 100, resample_steps: int = 0, blend_power: int = 3,
+                          ifm_diffusion_level: int = 50, seed: int = 0, group=None, max_batch: int = 8192,
+                          stats: Optional[dict] = None, context_norms=None, min_n_nodes: Optional[int] = None,
+                          max_n_nodes: Optional[int] = None):
+    """MLConformerGenerator.generate_jobs over the ranks of `group`: the jobs are flattened as there (jobs.flatten_jobs),
+    the flat samples dealt with `shard_indices`, and each rank runs the per-kind packed calls of its samples
+    (jobs.run_packed, device outputs).  One packed all-gather, then the split per job: every rank returns one dict per
+    job, equal bit for bit to the single-GPU result."""
+    from .config import CONTEXT_NORMS, MAX_N_NODES, MIN_N_NODES
+    from .jobs import flatten_jobs, run_packed, split_jobs
+    norms = CONTEXT_NORMS if context_norms is None else context_norms
+    packed = flatten_jobs(jobs, seed, norms, MIN_N_NODES if min_n_nodes is None else min_n_nodes,
+                          MAX_N_NODES if max_n_nodes is None else max_n_nodes)
+
+    def run_shard(ids, nn):
+        return run_packed(engine, packed, ids, T, resample_steps, blend_power, ifm_diffusion_level, seed, max_batch,
+                          device_out=True, context_norms=norms)
+
+    x, cls, bonds = generate_sharded(run_shard, packed.n_nodes, packed.N, group, max_batch, engine.device, stats)
+    return split_jobs(packed, x, cls, bonds)
