@@ -270,6 +270,18 @@ int mlcg_shape_tanimoto(mlcg_handle* h, const float* ref_pts, int n_ref, const f
                         int N, const float* frames, const float* orient, int n_orient, const float* axes, int G,
                         float amplitude, float atom_radius, float* workspace, float* scores, float* aligned, void* stream);
 
+/* mlcg_shape_tanimoto for many references in one call: sample b is scored against reference job[b].
+ * ref_pts (J,64,3): reference j's atoms in its principal frame in rows 0..n_ref[j]-1; n_ref (J) int32; axes (J,3,G): the
+ * grid of each reference; coords / n_nodes / frames / orient / scores / aligned as mlcg_shape_tanimoto; job (B) int32.
+ * workspace: J * (G^3 + 1) floats, reference j's density and squared sum at j * (G^3 + 1).  A sample's scores are
+ * bit-identical to mlcg_shape_tanimoto with its own reference, whatever else shares the call.  The kernels do not check
+ * job[b] in [0, J) or n_ref[j] in [1, 64]: the caller must.  MLCG_E_ARG for a null pointer (aligned may be NULL), J < 1,
+ * B < 1, N outside [1, 64], n_orient outside [1, 65535] or G outside [2, 48].  All device pointers. */
+int mlcg_shape_tanimoto_jobs(mlcg_handle* h, const float* ref_pts, const int32_t* n_ref, const float* axes, int J,
+                             const float* coords, const int32_t* n_nodes, const int32_t* job, int B, int N,
+                             const float* frames, const float* orient, int n_orient, int G, float amplitude,
+                             float atom_radius, float* workspace, float* scores, float* aligned, void* stream);
+
 /* Host-only (no device, no handle): the plan of the fused edge kernel for a batch.  tiles_out receives 8 int32 per tile
  * {molecule, rows of the first target that precede the tile, rows, atoms, first target, targets touched, state of the
  * first target, state of the last target} with state -1 = whole, -2 = carried in shared memory between two consecutive

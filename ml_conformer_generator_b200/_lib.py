@@ -20,7 +20,7 @@ EXPORTS = [
     "mlcg_num_edges", "mlcg_kernel_launches", "mlcg_time_edge_kernel", "mlcg_edge_phase_profile", "mlcg_test_gemm",
     "mlcg_shape_moments", "mlcg_shape_tanimoto", "mlcg_gemm_phase_profile", "mlcg_plan_edge_tiles",
     "mlcg_egnn_forward_breakdown", "mlcg_ifm_context", "mlcg_ifm_merge_inputs", "mlcg_nonfinite", "mlcg_edge_block_order",
-    "mlcg_generate_fragment", "mlcg_generate_fragment_jobs", "mlcg_graph_captures",
+    "mlcg_generate_fragment", "mlcg_generate_fragment_jobs", "mlcg_graph_captures", "mlcg_shape_tanimoto_jobs",
 ]
 
 
@@ -146,5 +146,7 @@ def load() -> C.CDLL:
     lib.mlcg_edge_block_order.argtypes = [ci, vp]
     lib.mlcg_shape_moments.argtypes = [vp, vp, vp, ci, ci, C.c_float, C.c_float, ci, vp, vp]
     lib.mlcg_shape_tanimoto.argtypes = [vp, vp, ci, vp, vp, ci, ci, vp, vp, ci, vp, ci, C.c_float, C.c_float, vp, vp, vp, vp]
+    lib.mlcg_shape_tanimoto_jobs.argtypes = [vp, vp, vp, vp, ci, vp, vp, vp, ci, ci, vp, vp, ci, ci, C.c_float, C.c_float, vp,
+                                             vp, vp, vp]
     _lib = lib
     return lib

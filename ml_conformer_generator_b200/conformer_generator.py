@@ -231,7 +231,7 @@ class MLConformerGenerator:
 
     @torch.no_grad()
     def generate_jobs(self, jobs: List[Dict], resample_steps: int = 0, blend_power: int = 3, ifm_diffusion_level: int = 50,
-                      seed: int = 0, max_batch: int = 8192) -> List[Dict[str, torch.Tensor]]:
+                      seed: int = 0, max_batch: int = 8192, keep_best: Optional[int] = None) -> List[Dict[str, torch.Tensor]]:
         """Many small generation jobs -- different references, atom counts and fixed fragments -- in few packed device
         calls (the GPU reaches its rate only with thousands of molecules per call).  A job is a dict:
           reference_context   raw principal moments (3)
@@ -242,16 +242,32 @@ class MLConformerGenerator:
           fixed_fragment      optional (coordinates (n,3), one-hot (n,8)), as in edm_sample_tensors
           inertial_fragment_matching   default True
           job_id              default: the job's position in the list
+          reference_conformer optional heavy-atom coordinates (n_ref,3), 3 <= n_ref <= 64, to score the molecules against
         Jobs are grouped by kind (plain / inpainting / inertial fragment matching) and cut into calls of at most
         `max_batch` samples; the loop settings are shared.  A job's molecules depend only on `seed`, its job_id, its own
         fields and the shared settings (jobs.py), never on the other jobs or their order.  Returns one dict per job, in
         input order, of host tensors: x (n,N,3), atom_class (n,N) (-1 = padding), n_nodes (n,), bonds (n,42,42) (the
-        provisional bond orders of generate_tensors), with N the job's own max atom count."""
-        from .jobs import flatten_jobs, run_packed, split_jobs
+        provisional bond orders of generate_tensors), with N the job's own max atom count.
+
+        The molecules of all jobs with a reference_conformer are scored on the GPU in one pass (ShapeScorer.evaluate_jobs,
+        the tensor part of the reference's evaluate_samples), and their dicts gain shape_tanimoto (n,), best_orientation
+        (n,), aligned_coords (n,N,3) and reference_coords (n_ref,3), each bit-identical to ShapeScorer.evaluate on that job.
+        With `keep_best` = k (every job then needs a reference_conformer) each job keeps only its min(k, n) best molecules
+        by shape_tanimoto, descending (NaN last, ties to the lower index), and gains sample_index: each row's position in
+        the unfiltered job."""
+        from .jobs import attach_scores, check_keep_best, flatten_jobs, run_packed, score_packed, split_jobs
         packed = flatten_jobs(jobs, seed, self.context_norms, self.min_n_nodes, self.max_n_nodes)
-        out = run_packed(self.engine, packed, np.arange(packed.ids.size), self.generative_model.T, resample_steps,
-                         blend_power, ifm_diffusion_level, seed, max_batch, context_norms=self.context_norms)
-        return split_jobs(packed, *out)
+        check_keep_best(packed, keep_best)
+        idx = np.arange(packed.ids.size)
+        args = (self.engine, packed, idx, self.generative_model.T, resample_steps, blend_power, ifm_diffusion_level, seed,
+                max_batch)
+        if not packed.scored:
+            return split_jobs(packed, *run_packed(*args, context_norms=self.context_norms))
+        from .shape_similarity import ShapeScorer
+        x, cls, bonds = run_packed(*args, device_out=True, context_norms=self.context_norms)
+        scores = score_packed(ShapeScorer(self.engine), packed, idx, x)
+        res = attach_scores(packed, split_jobs(packed, x, cls, bonds), *scores, keep_best)
+        return [{k: v.cpu() for k, v in r.items()} for r in res]
 
     # ------------------------------------------------------------------------------------------------------------
     # RDKit-facing path, same signatures as the reference

@@ -1765,6 +1765,28 @@ extern "C" int mlcg_shape_tanimoto(mlcg_handle* h, const float* ref_pts, int n_r
   return MLCG_OK;
 }
 
+extern "C" int mlcg_shape_tanimoto_jobs(mlcg_handle* h, const float* ref_pts, const int32_t* n_ref, const float* axes, int J,
+                                        const float* coords, const int32_t* n_nodes, const int32_t* job, int B, int N,
+                                        const float* frames, const float* orient, int n_orient, int G, float amplitude,
+                                        float atom_radius, float* workspace, float* scores, float* aligned, void* stream) {
+  if (!h) return MLCG_E_ARG;
+  if (!ref_pts || !n_ref || !axes || !coords || !n_nodes || !job || !frames || !orient || !workspace || !scores || J < 1 ||
+      B < 1 || N < 1 || N > SHAPE_MAX_ATOMS || n_orient < 1 || n_orient > 65535 || G < 2 || G > SHAPE_MAX_GRID)
+    FAIL(MLCG_E_ARG, "shape_tanimoto_jobs: need non-null pointers, J >= 1, B >= 1, 1 <= N <= 64, 1 <= n_orient <= 65535, "
+                     "2 <= G <= 48");
+  CK(cudaSetDevice(h->device));
+  cudaStream_t st = (cudaStream_t)stream;
+  const float alpha = (float)shape_alpha(amplitude, atom_radius);
+  k_shape_grid<true, true><<<dim3(J, 1), 256, 0, st>>>(ref_pts, n_ref, 0, SHAPE_MAX_ATOMS, nullptr, nullptr, 1, axes, G,
+                                                       amplitude, alpha, workspace, nullptr, nullptr, nullptr);
+  KCHECK();
+  k_shape_grid<false, true><<<dim3(B, n_orient), 256, 0, st>>>(coords, n_nodes, 0, N, frames, orient, n_orient, axes, G,
+                                                               amplitude, alpha, workspace, scores, aligned, job);
+  KCHECK();
+  h->launches += 2;
+  return MLCG_OK;
+}
+
 // ---------------------------------------------------------------------------------------------------------------
 // inertial fragment matching between the two reverse loops (reference utils/mol_utils.py:373-550)
 // ---------------------------------------------------------------------------------------------------------------

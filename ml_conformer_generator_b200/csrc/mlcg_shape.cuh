@@ -150,17 +150,25 @@ __global__ void __launch_bounds__(128) k_shape_moments(const float* __restrict__
 // Density overlap on the grid.  block = (sample b, orientation o); final coordinates = ((x - shift_b) . R_b) . O_o.
 //  kRef = true : one block, writes the density of the reference molecule to dens[G^3] and sum f^2 to dens[G^3].
 //  kRef = false: reads them, writes scores[b][o] = fg / (f2 + gg - fg) and (optionally) the final coordinates.
-template <bool kRef>
+//  kJobs = true: many references in one launch.  Reference j owns axes + j*3*G and dens + j*(G^3+1).  The reference pass
+//  runs one block per reference (b = j, its points at coords + j*N*3, its atom count n_nodes[j]); the sample pass scores
+//  sample b against reference job[b].  Everything else -- and so every bit of a score -- is the single-reference code.
+template <bool kRef, bool kJobs = false>
 __global__ void __launch_bounds__(256) k_shape_grid(const float* __restrict__ coords, const int* __restrict__ n_nodes, int n_fixed,
                                                     int N, const float* __restrict__ frames, const float* __restrict__ orient,
                                                     int n_orient, const float* __restrict__ axes, int G, float amplitude,
                                                     float alpha, float* dens, float* __restrict__ scores,
-                                                    float* __restrict__ aligned) {
+                                                    float* __restrict__ aligned, const int* __restrict__ job = nullptr) {
   __shared__ float tx[SHAPE_MAX_ATOMS][SHAPE_MAX_GRID], ty[SHAPE_MAX_ATOMS][SHAPE_MAX_GRID], tz[SHAPE_MAX_ATOMS][SHAPE_MAX_GRID];
   __shared__ float px[SHAPE_MAX_ATOMS], py[SHAPE_MAX_ATOMS], pz[SHAPE_MAX_ATOMS];
   __shared__ float red[2][8];
   const int b = blockIdx.x, o = blockIdx.y, tid = threadIdx.x;
-  const int n = kRef ? n_fixed : n_nodes[b];
+  const int n = (kRef && !kJobs) ? n_fixed : n_nodes[b];
+  if (kJobs) {
+    const size_t j = kRef ? (size_t)b : (size_t)job[b];
+    axes += j * 3 * G;
+    dens += j * ((size_t)G * G * G + 1);
+  }
   if (tid < n) {
     const float* x = coords + ((size_t)b * N + tid) * 3;
     float v[3] = {x[0], x[1], x[2]};

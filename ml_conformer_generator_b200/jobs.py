@@ -8,9 +8,13 @@ call) and cut into calls of at most `max_batch` samples; a job may straddle two 
 Determinism: sample k of a job has the global id `job_id * 2**32 + k`, which keys its device noise, and the job's atom
 counts are drawn from a generator seeded by `(seed, job_id)`.  Every kernel works on each sample alone, so a job's
 molecules depend only on `seed`, its `job_id`, its own fields and the shared loop settings -- never on the other jobs,
-their order or how the samples are cut into calls or shards."""
+their order or how the samples are cut into calls or shards.
+
+A job with a `reference_conformer` also has its molecules scored by Gaussian shape Tanimoto against that conformer
+(`score_packed`, one `ShapeScorer.evaluate_jobs` pass over the samples of all scored jobs) and may keep only its best ones
+(`attach_scores`).  Scoring works on each sample alone too, so the same independence holds for the scores."""
 from dataclasses import dataclass
-from typing import Dict, List, Optional, Sequence
+from typing import Dict, List, Optional, Sequence, Tuple
 
 import numpy as np
 import torch
@@ -21,7 +25,8 @@ from .mol_utils import _check_fragment_size, normalise_context
 KINDS = ("plain", "inpaint", "ifm")
 JOB_ID_SHIFT = 32
 _JOB_KEYS = {"reference_context", "n_atoms", "variance", "n_nodes", "n_samples", "fixed_fragment",
-             "inertial_fragment_matching", "job_id"}
+             "inertial_fragment_matching", "job_id", "reference_conformer"}
+SHAPE_MAX_ATOMS = 64  # atoms of a reference conformer (the shape kernels' limit)
 
 
 @dataclass
@@ -37,6 +42,12 @@ class PackedJobs:
     ctx: np.ndarray          # (S,3) f32 normalised context
     job: np.ndarray          # (S,) int32 job index
     ids: np.ndarray          # (S,) int64 global sample id (the noise key)
+    conformers: Optional[List[Optional[torch.Tensor]]] = None  # (J) heavy-atom reference conformer (n_ref,3) f32 or None
+
+    @property
+    def scored(self) -> bool:
+        """Whether any job has a reference conformer to score its molecules against."""
+        return self.conformers is not None and any(c is not None for c in self.conformers)
 
     @property
     def N(self) -> int:
@@ -55,7 +66,7 @@ def flatten_jobs(jobs: Sequence[Dict], seed: int = 0, context_norms: Dict = CONT
         raise ValueError("seed must be non-negative")
     if len(jobs) == 0:
         raise ValueError("generate_jobs: no jobs")
-    kind, job_ids, tops, fragments, refs = [], [], [], [], []
+    kind, job_ids, tops, fragments, refs, confs = [], [], [], [], [], []
     n_nodes, ctx = [], []
     for p, job in enumerate(jobs):
         unknown = set(job) - _JOB_KEYS
@@ -95,6 +106,14 @@ def flatten_jobs(jobs: Sequence[Dict], seed: int = 0, context_norms: Dict = CONT
             _check_fragment_size(int(fx.shape[0]), lo, hi)
             kind.append(2 if job.get("inertial_fragment_matching", True) else 1)
             fragments.append((fx, fh))
+        conf = job.get("reference_conformer")
+        if conf is not None:
+            conf = torch.as_tensor(conf).detach().cpu().to(torch.float32)
+            if conf.dim() != 2 or conf.shape[1] != 3:
+                raise ValueError("job %d: reference_conformer must be heavy-atom coordinates (n, 3)" % p)
+            if not 3 <= conf.shape[0] <= SHAPE_MAX_ATOMS:
+                raise ValueError("job %d: reference_conformer must have 3 <= n <= %d atoms" % (p, SHAPE_MAX_ATOMS))
+        confs.append(conf)
         job_ids.append(job_id)
         tops.append(hi)
         refs.append(ref)
@@ -108,7 +127,7 @@ def flatten_jobs(jobs: Sequence[Dict], seed: int = 0, context_norms: Dict = CONT
     job = np.repeat(np.arange(len(jobs), dtype=np.int32), sizes)
     ids = (job_ids[job] << JOB_ID_SHIFT) + (np.arange(starts[-1], dtype=np.int64) - starts[job])
     return PackedJobs(np.asarray(kind, dtype=np.int32), job_ids, np.asarray(tops, dtype=np.int32), starts, fragments, refs,
-                      np.concatenate(n_nodes).astype(np.int32), np.concatenate(ctx).astype(np.float32), job, ids)
+                      np.concatenate(n_nodes).astype(np.int32), np.concatenate(ctx).astype(np.float32), job, ids, confs)
 
 
 def run_packed(engine, packed: PackedJobs, idx: np.ndarray, T: int = 100, resample_steps: int = 0, blend_power: int = 3,
@@ -155,4 +174,66 @@ def split_jobs(packed: PackedJobs, x: torch.Tensor, cls: torch.Tensor, bonds: to
         a, b, nj = int(packed.starts[j]), int(packed.starts[j + 1]), int(packed.max_n_nodes[j])
         res.append({"x": x[a:b, :nj].clone(), "atom_class": cls[a:b, :nj].clone(),
                     "n_nodes": torch.from_numpy(packed.n_nodes[a:b].astype(np.int64)), "bonds": bonds[a:b].clone()})
+    return res
+
+
+def check_keep_best(packed: PackedJobs, keep_best: Optional[int]) -> None:
+    if keep_best is None:
+        return
+    if int(keep_best) < 1:
+        raise ValueError("keep_best must be at least 1")
+    if packed.conformers is None or any(c is None for c in packed.conformers):
+        raise ValueError("keep_best ranks by shape: every job needs a reference_conformer")
+
+
+def score_row_spec(N: int) -> Tuple[Tuple[torch.dtype, tuple], ...]:
+    """dtype and per-sample shape of score_packed's per-sample outputs, for packing them next to the molecules."""
+    return ((torch.float32, ()), (torch.int64, ()), (torch.float32, (N, 3)))
+
+
+def score_packed(scorer, packed: PackedJobs, idx: np.ndarray, x: torch.Tensor):
+    """Scores the flat samples `idx` (x (n,N,3) in the order of `idx`, N = packed.N) of the jobs with a reference conformer
+    in one `scorer.evaluate_jobs` pass.  Returns (shape_tanimoto (n,) f32, best_orientation (n,) i64, aligned_coords
+    (n,N,3) f32) on x's device -- rows of jobs without a conformer are 0 -- and the list over the jobs of each reference in
+    its principal frame (None for jobs without one)."""
+    idx = np.asarray(idx, dtype=np.int64).reshape(-1)
+    has = np.array([c is not None for c in packed.conformers])
+    scored_jobs = np.nonzero(has)[0]
+    rows = np.nonzero(has[packed.job[idx]])[0]
+    dev, n = x.device, idx.size
+    rr = torch.as_tensor(rows, device=dev)
+    out = scorer.evaluate_jobs([packed.conformers[j] for j in scored_jobs], x[rr],
+                               torch.from_numpy(packed.n_nodes[idx[rows]]),
+                               torch.from_numpy(np.searchsorted(scored_jobs, packed.job[idx[rows]]).astype(np.int64)))
+    score = torch.zeros(n, device=dev)
+    orient = torch.zeros(n, dtype=torch.int64, device=dev)
+    aligned = torch.zeros(n, x.shape[1], 3, device=dev)
+    score[rr], orient[rr], aligned[rr] = (out[k].to(dev) for k in ("shape_tanimoto", "best_orientation", "aligned_coords"))
+    ref_coords = [None] * len(packed.conformers)
+    for k, j in enumerate(scored_jobs):
+        ref_coords[j] = out["reference_coords"][k]
+    return score, orient, aligned, ref_coords
+
+
+def attach_scores(packed: PackedJobs, res: List[Dict[str, torch.Tensor]], score: torch.Tensor, orient: torch.Tensor,
+                  aligned: torch.Tensor, ref_coords: List[Optional[torch.Tensor]],
+                  keep_best: Optional[int] = None) -> List[Dict[str, torch.Tensor]]:
+    """Adds shape_tanimoto, best_orientation, aligned_coords and reference_coords to the dict (split_jobs) of every job
+    with a reference conformer; `score` etc. hold all samples in flat order.  With `keep_best` = k each such job keeps its
+    min(k, n) best molecules, by shape_tanimoto descending (NaN last), ties to the lower sample index, with
+    `sample_index` the row of each in the unfiltered job.  Jobs without a conformer are left as they are."""
+    for j, r in enumerate(res):
+        if packed.conformers[j] is None:
+            continue
+        a, b, nj = int(packed.starts[j]), int(packed.starts[j + 1]), int(packed.max_n_nodes[j])
+        r.update(shape_tanimoto=score[a:b].clone(), best_orientation=orient[a:b].clone(),
+                 aligned_coords=aligned[a:b, :nj].clone())
+        if keep_best is not None:
+            s = r["shape_tanimoto"]
+            key = torch.where(torch.isnan(s), torch.full_like(s, -float("inf")), s)
+            keep = torch.sort(key, descending=True, stable=True).indices[:int(keep_best)]
+            for k in list(r):
+                r[k] = r[k][keep.to(r[k].device)]
+            r["sample_index"] = keep
+        r["reference_coords"] = ref_coords[j]
     return res

@@ -38,20 +38,31 @@ def result_bytes(max_n_nodes: int) -> int:
     return max_n_nodes * 3 * 4 + max_n_nodes * 4 + SEER_D * SEER_D
 
 
-def pack_results(x: torch.Tensor, cls: torch.Tensor, bonds: torch.Tensor) -> torch.Tensor:
-    """(n,N,3) f32, (n,N) i32, (n,42,42) i8 -> (n, result_bytes(N)) uint8: one buffer, one collective."""
+def _extra_bytes(extra) -> int:
+    return sum(int(np.prod(shape)) * torch.empty(0, dtype=dtype).element_size() for dtype, shape in extra)
+
+
+def pack_results(x: torch.Tensor, cls: torch.Tensor, bonds: torch.Tensor, *extra: torch.Tensor) -> torch.Tensor:
+    """(n,N,3) f32, (n,N) i32, (n,42,42) i8 -> (n, result_bytes(N)) uint8: one buffer, one collective.  `extra` per-sample
+    tensors (n, ...) are appended to each row in order."""
     n = x.shape[0]
-    return torch.cat([x.contiguous().view(torch.uint8).reshape(n, -1), cls.contiguous().view(torch.uint8).reshape(n, -1),
-                      bonds.contiguous().view(torch.uint8).reshape(n, -1)], dim=1)
+    return torch.cat([t.contiguous().view(torch.uint8).reshape(n, -1) for t in (x, cls, bonds) + extra], dim=1)
 
 
-def unpack_results(buf: torch.Tensor, max_n_nodes: int) -> Tuple[torch.Tensor, torch.Tensor, torch.Tensor]:
+def unpack_results(buf: torch.Tensor, max_n_nodes: int, extra=()) -> Tuple[torch.Tensor, ...]:
+    """Inverse of pack_results; `extra` lists the (dtype, per-sample shape) of the appended tensors."""
     n, N = buf.shape[0], max_n_nodes
     a, b = N * 12, N * 16
     x = buf[:, :a].clone().view(torch.float32).reshape(n, N, 3)
     cls = buf[:, a:b].clone().view(torch.int32).reshape(n, N)
-    bonds = buf[:, b:].clone().view(torch.int8).reshape(n, SEER_D, SEER_D)
-    return x, cls, bonds
+    c = result_bytes(N)
+    bonds = buf[:, b:c].clone().view(torch.int8).reshape(n, SEER_D, SEER_D)
+    out = [x, cls, bonds]
+    for dtype, shape in extra:
+        w = _extra_bytes([(dtype, shape)])
+        out.append(buf[:, c:c + w].clone().view(dtype).reshape(n, *shape))
+        c += w
+    return tuple(out)
 
 
 def gather_packed(local: torch.Tensor, shards: List[np.ndarray], total: int, group=None) -> torch.Tensor:
@@ -83,11 +94,12 @@ def gather_packed(local: torch.Tensor, shards: List[np.ndarray], total: int, gro
 
 def generate_sharded(run_shard: Callable[[np.ndarray, np.ndarray], Sequence[torch.Tensor]], n_nodes: Sequence[int],
                      max_n_nodes: int, group=None, max_batch: int = 8192, device: Optional[torch.device] = None,
-                     stats: Optional[dict] = None) -> Tuple[torch.Tensor, torch.Tensor, torch.Tensor]:
+                     stats: Optional[dict] = None, extra=()) -> Tuple[torch.Tensor, ...]:
     """Shards `n_nodes` over the ranks of `group`; this rank calls `run_shard(ids, n_nodes[ids])` -- the per-GPU hot path,
     e.g. `Engine.generate_host(..., sample_ids=ids, device_out=True)` -- once per sub-batch of at most `max_batch` of its
     samples (one call for a shard that fits), packs the results and runs the one all-gather.  Returns
-    (x (B,N,3) f32, atom_class (B,N) i32, bonds (B,42,42) i8) for ALL samples in global order, on every rank."""
+    (x (B,N,3) f32, atom_class (B,N) i32, bonds (B,42,42) i8) for ALL samples in global order, on every rank, followed by
+    the further per-sample tensors run_shard returns after bonds, described by `extra` as in unpack_results."""
     world = dist.get_world_size(group) if dist.is_initialized() else 1
     rank = dist.get_rank(group) if dist.is_initialized() else 0
     n_nodes = np.asarray(n_nodes)
@@ -96,17 +108,17 @@ def generate_sharded(run_shard: Callable[[np.ndarray, np.ndarray], Sequence[torc
     pieces = []
     for s in range(0, len(mine), max_batch):
         ids = mine[s:s + max_batch]
-        x, cls, bonds = run_shard(ids, n_nodes[ids])
-        pieces.append(pack_results(x, cls, bonds))
+        pieces.append(pack_results(*run_shard(ids, n_nodes[ids])))
     if stats is not None:
         stats["calls"] = len(pieces)
         stats["shard"] = len(mine)
     if pieces:
         local = torch.cat(pieces, dim=0) if len(pieces) > 1 else pieces[0]
     else:
-        local = torch.zeros((0, result_bytes(max_n_nodes)), dtype=torch.uint8, device=device or torch.device("cpu"))
+        local = torch.zeros((0, result_bytes(max_n_nodes) + _extra_bytes(extra)), dtype=torch.uint8,
+                            device=device or torch.device("cpu"))
     full = gather_packed(local, shards, len(n_nodes), group)
-    return unpack_results(full, max_n_nodes)
+    return unpack_results(full, max_n_nodes, extra)
 
 
 def generate_sharded_engine(engine, n_nodes: Sequence[int], max_n_nodes: int, ctx: np.ndarray, T: int = 100,
@@ -133,20 +145,38 @@ def generate_sharded_engine(engine, n_nodes: Sequence[int], max_n_nodes: int, ct
 def generate_jobs_sharded(engine, jobs, T: int = 100, resample_steps: int = 0, blend_power: int = 3,
                           ifm_diffusion_level: int = 50, seed: int = 0, group=None, max_batch: int = 8192,
                           stats: Optional[dict] = None, context_norms=None, min_n_nodes: Optional[int] = None,
-                          max_n_nodes: Optional[int] = None):
+                          max_n_nodes: Optional[int] = None, keep_best: Optional[int] = None, scorer=None):
     """MLConformerGenerator.generate_jobs over the ranks of `group`: the jobs are flattened as there (jobs.flatten_jobs),
     the flat samples dealt with `shard_indices`, and each rank runs the per-kind packed calls of its samples
     (jobs.run_packed, device outputs).  One packed all-gather, then the split per job: every rank returns one dict per
-    job, equal bit for bit to the single-GPU result."""
+    job, equal bit for bit to the single-GPU result.  Jobs with a `reference_conformer` are scored by each rank on its
+    own shard (jobs.score_packed with `scorer`, default a ShapeScorer on the engine); the scores travel in the same
+    all-gather, and the `keep_best` selection runs after it, identically on every rank."""
     from .config import CONTEXT_NORMS, MAX_N_NODES, MIN_N_NODES
-    from .jobs import flatten_jobs, run_packed, split_jobs
+    from .jobs import attach_scores, check_keep_best, flatten_jobs, run_packed, score_packed, score_row_spec, split_jobs
     norms = CONTEXT_NORMS if context_norms is None else context_norms
     packed = flatten_jobs(jobs, seed, norms, MIN_N_NODES if min_n_nodes is None else min_n_nodes,
                           MAX_N_NODES if max_n_nodes is None else max_n_nodes)
+    check_keep_best(packed, keep_best)
+    if packed.scored and scorer is None:
+        from .shape_similarity import ShapeScorer
+        scorer = ShapeScorer(engine)
+    ref_coords = []
 
     def run_shard(ids, nn):
-        return run_packed(engine, packed, ids, T, resample_steps, blend_power, ifm_diffusion_level, seed, max_batch,
-                          device_out=True, context_norms=norms)
+        out = run_packed(engine, packed, ids, T, resample_steps, blend_power, ifm_diffusion_level, seed, max_batch,
+                         device_out=True, context_norms=norms)
+        if not packed.scored:
+            return out
+        *scores, ref_coords[:] = score_packed(scorer, packed, ids, out[0])
+        return (*out, *scores)
 
-    x, cls, bonds = generate_sharded(run_shard, packed.n_nodes, packed.N, group, max_batch, engine.device, stats)
-    return split_jobs(packed, x, cls, bonds)
+    extra = score_row_spec(packed.N) if packed.scored else ()
+    x, cls, bonds, *scores = generate_sharded(run_shard, packed.n_nodes, packed.N, group, max_batch, engine.device, stats,
+                                              extra)
+    res = split_jobs(packed, x, cls, bonds)
+    if not packed.scored:
+        return res
+    if not ref_coords:  # an empty shard: the references alone
+        ref_coords = score_packed(scorer, packed, np.zeros(0, np.int64), x[:0])[3]
+    return attach_scores(packed, res, *scores, ref_coords, keep_best)

@@ -2,11 +2,11 @@
 
 Mirrors the tensor part of the reference's `evaluate_samples` (cheminformatics/pipeline.py:37-86) and the functions of
 cheminformatics/shape_similarity.py it calls, with the same names where a counterpart exists.  The clique series and the
-grid overlap run in `libmlcg_b200.so` (`mlcg_shape_moments`, `mlcg_shape_tanimoto`); the 3x3 eigen-decomposition stays on
-the host in torch, exactly as the reference does it (`torch.linalg.eigh`, shape_similarity.py:139), so the principal-frame
-sign / order conventions are the reference's.  There is no CPU fallback.
+grid overlap run in `libmlcg_b200.so` (`mlcg_shape_moments`, `mlcg_shape_tanimoto`, `mlcg_shape_tanimoto_jobs`); the 3x3
+eigen-decomposition stays on the host in torch, exactly as the reference does it (`torch.linalg.eigh`,
+shape_similarity.py:139), so the principal-frame sign / order conventions are the reference's.  There is no CPU fallback.
 """
-from typing import Dict, Optional
+from typing import Dict, Optional, Sequence
 
 import numpy as np
 import torch
@@ -17,6 +17,7 @@ ATOM_RADIUS = 1.60   # reference shape_similarity.py:14
 AMPLITUDE = 2.70     # reference shape_similarity.py:15
 GRID_POINTS = 40     # tanimoto_score default, :470
 MAX_ATOMS = 64
+MAX_JOB_REFERENCES = 256  # references per mlcg_shape_tanimoto_jobs call: 64 MB of density workspace at 40^3
 
 
 def get_alpha(atom_radius: float = ATOM_RADIUS, gaussian_amplitude: float = AMPLITUDE) -> float:
@@ -140,3 +141,85 @@ class ShapeScorer:
         idx = best.view(-1, 1, 1, 1).expand(-1, 1, aligned.size(2), 3)
         return {"shape_tanimoto": best_score, "best_orientation": best, "aligned_coords": aligned.gather(1, idx).squeeze(1),
                 "scores": scores, "reference_coords": ref_pts, "moments": sf["moments"], "reference_moments": rf["moments"][0]}
+
+    # -- evaluate for many references at once ------------------------------------------------------------------------
+    def evaluate_jobs(self, references: Sequence[torch.Tensor], coords: torch.Tensor, n_nodes: torch.Tensor,
+                      job: torch.Tensor, n: int = GRID_POINTS) -> Dict[str, object]:
+        """`evaluate` of every sample against its own reference: sample b (coords (B,N,3), n_nodes (B)) is scored against
+        references[job[b]] (heavy-atom coordinates (n_ref,3), 3 <= n_ref <= 64).  Returns device tensors
+        `shape_tanimoto` (B,), `best_orientation` (B,), `aligned_coords` (B,N,3), `scores` (B,4), `moments` (B,3), and
+        per reference the lists `reference_coords` (n_ref,3) and `reference_moments` (3,).  Every value is bit-identical
+        to `evaluate(references[j], samples of job j)`: the references go through evaluate's own host code one at a time,
+        the kernels score each sample alone, and the best orientation uses evaluate's rule on the device.  B may be 0
+        (the reference outputs only).  Calls hold at most MAX_JOB_REFERENCES references each, which bounds the density
+        workspace (256 KB per reference at n = 40)."""
+        e = self.engine
+        refs = [torch.as_tensor(r).detach().to(torch.float32) for r in references]
+        J = len(refs)
+        for j, r in enumerate(refs):
+            if r.dim() != 2 or r.size(1) != 3 or not 3 <= r.size(0) <= MAX_ATOMS:
+                raise ValueError("reference %d must be (n_ref, 3) with 3 <= n_ref <= %d" % (j, MAX_ATOMS))
+        coords = coords.to(self.device, torch.float32).contiguous()
+        if coords.dim() != 3 or coords.size(2) != 3:
+            raise ValueError("coords must be (B, N, 3)")
+        B, N = coords.size(0), coords.size(1)
+        n_nodes = torch.as_tensor(n_nodes).reshape(-1)
+        job = torch.as_tensor(job).reshape(-1).to(torch.int64).cpu()
+        if n_nodes.numel() != B or job.numel() != B:
+            raise ValueError("coords, n_nodes and job must have the same length B")
+        if B and (J == 0 or int(job.min()) < 0 or int(job.max()) >= J):
+            raise ValueError("job indices must lie in [0, %d)" % J)
+        # the references exactly as evaluate computes them (principal_frames of that one reference, then grid_axes)
+        ref_pts = torch.zeros(J, MAX_ATOMS, 3)
+        axes = torch.empty(J, 3, n)
+        ref_coords, ref_moments = [], []
+        for j, r in enumerate(refs):
+            rf = self.principal_frames(r.unsqueeze(0), torch.tensor([r.size(0)]))
+            pts = rf["points"][0]
+            ref_pts[j, :pts.size(0)] = pts
+            axes[j] = grid_axes(pts, n)
+            ref_coords.append(pts.to(self.device))
+            ref_moments.append(rf["moments"][0].to(self.device))
+        out = {"reference_coords": ref_coords, "reference_moments": ref_moments}
+        n_orient = self._orient.size(0)
+        if B == 0:
+            out.update(shape_tanimoto=torch.empty(0, device=self.device),
+                       best_orientation=torch.empty(0, dtype=torch.long, device=self.device),
+                       aligned_coords=torch.empty(0, N, 3, device=self.device),
+                       scores=torch.empty(0, n_orient, device=self.device), moments=torch.empty(0, 3, device=self.device))
+            return out
+        sf = self.principal_frames(coords, n_nodes)
+        frames = sf["frames"].to(self.device)
+        nn_dev = n_nodes.to(torch.int32).to(self.device)
+        job_dev = job.to(self.device)
+        ref_pts, axes = ref_pts.to(self.device), axes.to(self.device)
+        n_ref = torch.tensor([r.size(0) for r in refs], dtype=torch.int32, device=self.device)
+        orient = self._orient.reshape(-1, 9).to(self.device).contiguous()
+        work = torch.empty(min(J, MAX_JOB_REFERENCES) * (n ** 3 + 1), device=self.device)
+        scores = torch.empty(B, n_orient, device=self.device)
+        aligned = torch.zeros(B, n_orient, N, 3, device=self.device)
+        for j0 in range(0, J, MAX_JOB_REFERENCES):
+            j1 = min(J, j0 + MAX_JOB_REFERENCES)
+            rows = torch.nonzero((job_dev >= j0) & (job_dev < j1)).view(-1)
+            if rows.numel() == 0:
+                continue
+            c, nn, fr = coords[rows].contiguous(), nn_dev[rows].contiguous(), frames[rows].contiguous()
+            jb = (job_dev[rows] - j0).to(torch.int32).contiguous()
+            sc = torch.empty(rows.numel(), n_orient, device=self.device)
+            al = torch.zeros(rows.numel(), n_orient, N, 3, device=self.device)
+            e._check(e.lib.mlcg_shape_tanimoto_jobs(
+                e.h, _ptr(ref_pts[j0:j1]), _ptr(n_ref[j0:j1]), _ptr(axes[j0:j1]), j1 - j0, _ptr(c), _ptr(nn), _ptr(jb),
+                rows.numel(), N, _ptr(fr), _ptr(orient), n_orient, n, self.amplitude, self.atom_radius, _ptr(work),
+                _ptr(sc), _ptr(al), e._stream()), "shape_tanimoto_jobs")
+            scores[rows], aligned[rows] = sc, al
+        # evaluate's rule: the first strict maximum over the orientations (a NaN never wins)
+        best = torch.zeros(B, dtype=torch.long, device=self.device)
+        best_score = scores[:, 0].clone()
+        for k in range(1, n_orient):
+            better = scores[:, k] > best_score
+            best = torch.where(better, torch.full_like(best, k), best)
+            best_score = torch.where(better, scores[:, k], best_score)
+        idx = best.view(-1, 1, 1, 1).expand(-1, 1, N, 3)
+        out.update(shape_tanimoto=best_score, best_orientation=best, aligned_coords=aligned.gather(1, idx).squeeze(1),
+                   scores=scores, moments=sf["moments"].to(self.device))
+        return out
