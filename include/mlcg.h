@@ -9,7 +9,8 @@
  *  - plain pointers and sizes only; no torch types.  Unless a parameter says "host", pointers are DEVICE pointers
  *    owned by the caller; the library never frees caller memory.
  *  - every call enqueues its work on `stream` (a cudaStream_t passed as void*) and returns without synchronising,
- *    except mlcg_generate / mlcg_generate_fragment(_jobs) / mlcg_load_* / mlcg_set_batch which are synchronous.
+ *    except mlcg_generate / mlcg_generate_fragment(_jobs) / mlcg_generate_analogue_jobs / mlcg_load_* / mlcg_set_batch
+ *    which are synchronous.
  *  - return value: 0 = ok, < 0 = argument / state error (see mlcg_last_error), > 0 = cudaError_t.
  *  - one handle per (device, stream); a handle is thread-compatible, not thread-safe.
  *  - layouts are the reference's: z / eps / noise are (B, N, 11) float32 row-major with N = the call's max_n_nodes
@@ -122,8 +123,11 @@ int mlcg_decode(mlcg_handle* h, const float* z0, const float* eps0, float sigma_
                 const mlcg_noise* noise, float* x, int32_t* atom_class, void* stream);
 
 /* Whole reverse loop on the device.  mode 0 = EquivariantDiffusion.forward (equivariant_diffusion.py:365-421),
- * 1 = .inpaint (:423-513), 2 = .merge_fragments (:515-607).  steps: HOST array of T entries, steps[s] for integer
- * step s (s = T-1 .. 0 are executed; merge skips s > diffusion_level).  ctx: (B,3).  noise_tape: NULL (device
+ * 1 = .inpaint (:423-513), 2 = .merge_fragments (:515-607), 3 = analogue: the merge_fragments loop without any
+ * re-injection (forward diffusion of z_known to diffusion_level, max(resample_steps, 1) denoises per level, decode; no
+ * re-injection launch and no re-injection noise draw; fixed_mask is not read and may be NULL) -- with nothing fixed,
+ * merge_fragments' fixed-atom centre of mass is 0/0.  steps: HOST array of T entries, steps[s] for integer
+ * step s (s = T-1 .. 0 are executed; modes 2 and 3 skip s > diffusion_level).  ctx: (B,3).  noise_tape: NULL (device
  * Philox, seed; sample_ids: NULL or a DEVICE array of B global sample ids, see mlcg_noise) or (n_draws, B, N, 11) raw
  * draws consumed in the reference's order.  z_work: (B,N,11) scratch that
  * holds z_0 on return.  trace_z / trace_eps: optional (n_forwards, B, N, 11) outputs recording every denoiser
@@ -225,6 +229,50 @@ int mlcg_generate_fragment_jobs(mlcg_handle* h, const mlcg_fragment_jobs* jobs, 
                                 const int64_t* sample_ids_host, float* x_out, int32_t* atom_class_out, int8_t* bonds_out,
                                 void* stream);
 
+/* Analogue jobs of mlcg_generate_analogue_jobs: every job has a parent molecule, whose atoms are all kept (the samples of
+ * a job have exactly the parent's atom count), and optionally some of them fixed.  All HOST pointers. */
+typedef struct {
+  int n_jobs;                        /* >= 1 */
+  const int32_t* job_of_sample_host; /* (B) the job of every sample, 0 <= job < n_jobs */
+  const int32_t* n_atoms_host;       /* (n_jobs) atoms of every parent, 1 <= n_atoms <= N, = n_nodes of its samples */
+  const float* coords_host;          /* (sum n_atoms,3) the parents' coordinates, centred on their heavy-atom mean, back to
+                                        back in job order */
+  const float* one_hot_host;         /* (sum n_atoms,8) their raw 0/1 one-hot atom classes, in the same order */
+  const int32_t* fixed_host;         /* (sum n_atoms) 1 = the atom is re-injected at every step, 0 = free; in one call
+                                        either every job has a fixed atom or none has, and no job has all atoms fixed */
+  int diffusion_level;               /* L in [1, T]: the parents are forward-diffused to level L, shared */
+  float merge_alpha, merge_sigma;    /* alpha / sigma of that level (mlcg_sample's merge_alpha / merge_sigma), shared */
+} mlcg_analogue_jobs;
+
+/* Analogues of given molecules: each sample starts from its job's parent forward-diffused to diffusion_level and is
+ * denoised from there to 0 (L = 1 returns the parent up to the last steps' noise, L = T is a fresh sample).  With fixed
+ * atoms the loop is merge_fragments' (equivariant_diffusion.py:515-607, mlcg_sample mode 2): the fixed atoms are
+ * re-injected at every step with the blend (1 - s/T)^blend_power (in steps) and the fixed-atom centre-of-mass
+ * alignment.  With none it is mlcg_sample mode 3.  Inputs, outputs, synchronous behaviour and CUDA-graph replay (from the
+ * second call with the same key on) as mlcg_generate_fragment_jobs; the device sequence is mlcg_analogue_inputs,
+ * mlcg_sample (mode 2 or 3, draws numbered from 0) and mlcg_seer_inputs + mlcg_seer_forward, and the results equal that
+ * eager composition bit for bit.  Every kernel works on each sample alone and the noise is keyed by the global sample id,
+ * so a sample's result equals that of a call holding only its own job with the same id.  The graph key is the geometry
+ * (B, N, per-sample n_nodes, the job count and the packed parent length), the mode and the shared scalars; the parents,
+ * flags, job of every sample, context, ids and seed are uploaded on every call, so new parents of the same sizes replay
+ * the captured graph.  ctx_host (B,3) is the normalised context of every sample.  Atom class 7 (Br) is never decoded (the
+ * argmax reads 7 channels), fixed atoms included.  Returns MLCG_E_ARG for a job index out of range,
+ * n_nodes[b] != n_atoms[job[b]], a call mixing jobs with and without fixed atoms, a job with every atom fixed,
+ * n_atoms outside [1, N], N outside [1, 39], diffusion_level outside [1, T], n_jobs < 1, a null pointer or weights not
+ * loaded. */
+int mlcg_generate_analogue_jobs(mlcg_handle* h, const mlcg_analogue_jobs* jobs, const int32_t* n_nodes_host, int B, int N,
+                                const float* ctx_host, int T, const mlcg_step_scalars* steps, int resample_steps,
+                                float sigma_0, float alpha_0, float sigma_x, uint64_t seed, int64_t sample_offset,
+                                const int64_t* sample_ids_host, float* x_out, int32_t* atom_class_out, int8_t* bonds_out,
+                                void* stream);
+/* The first step of mlcg_generate_analogue_jobs on its own (eager composition, tests): z_known (B,N,11) and fixed_mask
+ * (B,N) float from the parent table.  Sample b gets the parent of job job_of_sample[b] in rows 0..n_atoms-1 (centred
+ * coordinates, raw one-hot; fixed_mask = its flag) and zeros beyond.  `jobs` holds HOST pointers as above
+ * (diffusion_level and the merge scalars are not read); z_known / fixed_mask are DEVICE pointers.  MLCG_E_ARG as
+ * mlcg_generate_analogue_jobs, without the checks that need n_nodes or T. */
+int mlcg_analogue_inputs(mlcg_handle* h, const mlcg_analogue_jobs* jobs, int B, int N, float* z_known, float* fixed_mask,
+                         void* stream);
+
 /* ---- Inertial fragment matching (the default fragment mode) between the two reverse loops ---------------------------
  * Replaces: ifm_prepare_gen_fragment_context (utils/mol_utils.py:373-457) after its batch-independent prologue.  The
  * caller computes once, on the host and in float32 as the reference does, moi_gen_origin_host (3x3 row-major) =
@@ -309,7 +357,8 @@ int mlcg_num_edge_tiles(mlcg_handle* h);
 int64_t mlcg_num_edges(mlcg_handle* h);          /* sum_b n_b (n_b - 1) */
 int64_t mlcg_kernel_launches(mlcg_handle* h);    /* kernels launched by this handle since creation */
 int64_t mlcg_graph_captures(mlcg_handle* h);     /* CUDA graphs captured by mlcg_generate / mlcg_generate_fragment(_jobs)
-                                                    since creation: a replay leaves it unchanged */
+                                                    / mlcg_generate_analogue_jobs since creation: a replay leaves it
+                                                    unchanged */
 /* Times the dominant kernel (the fused edge kernel) with CUDA events on `stream`: runs one sub-layer launch `iters`
  * times on the current batch state and returns the mean milliseconds per launch (< 0 on error). */
 float mlcg_time_edge_kernel(mlcg_handle* h, int layer, int iters, void* stream);

@@ -21,6 +21,7 @@ EXPORTS = [
     "mlcg_shape_moments", "mlcg_shape_tanimoto", "mlcg_gemm_phase_profile", "mlcg_plan_edge_tiles",
     "mlcg_egnn_forward_breakdown", "mlcg_ifm_context", "mlcg_ifm_merge_inputs", "mlcg_nonfinite", "mlcg_edge_block_order",
     "mlcg_generate_fragment", "mlcg_generate_fragment_jobs", "mlcg_graph_captures", "mlcg_shape_tanimoto_jobs",
+    "mlcg_generate_analogue_jobs", "mlcg_analogue_inputs",
 ]
 
 
@@ -50,6 +51,12 @@ class FragmentJobs(C.Structure):
                 ("ff_x_host", C.c_void_p), ("ff_h_host", C.c_void_p), ("diffusion_level", C.c_int),
                 ("merge_alpha", C.c_float), ("merge_sigma", C.c_float), ("moi_gen_origin_host", C.c_void_p),
                 ("ff_weighted_com_host", C.c_void_p), ("norm_mean_host", C.c_void_p), ("norm_mad_host", C.c_void_p)]
+
+
+class AnalogueJobs(C.Structure):
+    _fields_ = [("n_jobs", C.c_int), ("job_of_sample_host", C.c_void_p), ("n_atoms_host", C.c_void_p),
+                ("coords_host", C.c_void_p), ("one_hot_host", C.c_void_p), ("fixed_host", C.c_void_p),
+                ("diffusion_level", C.c_int), ("merge_alpha", C.c_float), ("merge_sigma", C.c_float)]
 
 
 STAMP_PATH = LIB_PATH + ".stamp"
@@ -127,6 +134,9 @@ def load() -> C.CDLL:
                                            cf, C.c_uint64, C.c_int64, vp, vp, vp, vp, vp]
     lib.mlcg_generate_fragment_jobs.argtypes = [vp, C.POINTER(FragmentJobs), vp, ci, ci, vp, ci, C.POINTER(StepScalars), ci,
                                                 cf, cf, cf, C.c_uint64, C.c_int64, vp, vp, vp, vp, vp]
+    lib.mlcg_generate_analogue_jobs.argtypes = [vp, C.POINTER(AnalogueJobs), vp, ci, ci, vp, ci, C.POINTER(StepScalars), ci,
+                                                cf, cf, cf, C.c_uint64, C.c_int64, vp, vp, vp, vp, vp]
+    lib.mlcg_analogue_inputs.argtypes = [vp, C.POINTER(AnalogueJobs), ci, ci, vp, vp, vp]
     lib.mlcg_nonfinite.argtypes = [vp, vp]
     lib.mlcg_num_edge_tiles.argtypes = [vp]
     lib.mlcg_num_edges.argtypes = [vp]

@@ -243,8 +243,22 @@ class MLConformerGenerator:
           inertial_fragment_matching   default True
           job_id              default: the job's position in the list
           reference_conformer optional heavy-atom coordinates (n_ref,3), 3 <= n_ref <= 64, to score the molecules against
-        Jobs are grouped by kind (plain / inpainting / inertial fragment matching) and cut into calls of at most
-        `max_batch` samples; the loop settings are shared.  A job's molecules depend only on `seed`, its job_id, its own
+        An analogue job asks for molecules like a given one instead:
+          parent_molecule     (coordinates (n,3), raw 0/1 one-hot (n,8)), the parent's n heavy atoms, 3 <= n <=
+                              max_n_nodes; every sample has exactly these n atoms.  n_samples is required; n_atoms,
+                              variance, n_nodes, fixed_fragment and inertial_fragment_matching cannot go with it
+          fixed_atoms         optional distinct indices of at most n - 1 parent atoms, re-injected at every step as
+                              merge_fragments re-injects a fragment (blend (1 - s/T)^blend_power, centre-of-mass alignment)
+          diffusion_level     optional L in [1, T] (default `ifm_diffusion_level`): the parent is forward-diffused to level
+                              L and denoised from there -- L = 1 gives the parent back, L = T a fresh sample
+          reference_context   optional here: default the parent's own principal moments, get_context_shape of the centred
+                              coordinates (as generate_conformers takes them from a reference conformer); another context
+                              steers the analogues toward another shape
+        The parent is centred on its mean before noising and the results are returned in its input frame.  Atom class 7
+        (Br) is never emitted -- the decode reads 7 class channels -- and that holds for fixed atoms too.  Rows that
+        keep_best returned can be fed back as parents: (x[k, :n], one_hot(atom_class[k, :n], 8)).
+        Jobs are grouped by kind (plain / inpainting / inertial fragment matching / analogue, the last by (has fixed
+        atoms, diffusion level)) and cut into calls of at most `max_batch` samples; the loop settings are shared.  A job's molecules depend only on `seed`, its job_id, its own
         fields and the shared settings (jobs.py), never on the other jobs or their order.  Returns one dict per job, in
         input order, of host tensors: x (n,N,3), atom_class (n,N) (-1 = padding), n_nodes (n,), bonds (n,42,42) (the
         provisional bond orders of generate_tensors), with N the job's own max atom count.

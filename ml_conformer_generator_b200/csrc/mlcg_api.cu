@@ -106,6 +106,9 @@ struct mlcg_handle {
   // and the first IFM loop's context and outputs
   DevBuf f_ffx, f_ffh, f_jobs, f_job, f_zk, f_fm, f_ctx, f_shift, f_rot, f_ngen, f_xg, f_clsg;
   DevBuf hook_job;  // the one-job table of the eager hooks mlcg_ifm_context / mlcg_ifm_merge_inputs
+  // mlcg_generate_analogue_jobs: the parent table (AnalogueTable's blob); z_known / fixed_mask go to f_zk / f_fm.  The
+  // eager hook mlcg_analogue_inputs has a buffer of its own, so it never moves one a captured graph reads.
+  DevBuf a_tab, hook_parents;
   DevBuf nf_flag;  // set by k_decode when a generated coordinate is not finite (mlcg_nonfinite)
   std::vector<int64_t> ids_stage;
   // test gemm
@@ -1132,9 +1135,10 @@ static int sample_loop(mlcg_handle* h, int mode, int T, const mlcg_step_scalars*
                        float* trace_z, float* trace_eps, uint64_t draw0, void* stream) {
   STEP_PROLOGUE("sample");
   if (!h->egnn_loaded) FAIL(MLCG_E_STATE, "sample: load the EGNN weights first");
-  if (mode < 0 || mode > 2 || T <= 0 || !steps || !ctx || !z || !x_out || !atom_class_out || resample_steps < 0)
+  if (mode < 0 || mode > 3 || T <= 0 || !steps || !ctx || !z || !x_out || !atom_class_out || resample_steps < 0)
     FAIL(MLCG_E_ARG, "sample: bad argument");
-  if (mode != 0 && (!z_known || !fixed_mask)) FAIL(MLCG_E_ARG, "sample: inpaint / merge need z_known and fixed_mask");
+  if ((mode == 1 || mode == 2) && (!z_known || !fixed_mask)) FAIL(MLCG_E_ARG, "sample: inpaint / merge need z_known and fixed_mask");
+  if (mode == 3 && !z_known) FAIL(MLCG_E_ARG, "sample: analogue needs z_known");
   const size_t zsz = (size_t)h->pl->B * h->pl->N * ZC;
   float* eps = h->eps_dev.as<float>();
   float* tdev = h->t_dev.as<float>();
@@ -1171,7 +1175,9 @@ static int sample_loop(mlcg_handle* h, int mode, int T, const mlcg_step_scalars*
     return mlcg_reinject(h, z, z_known, fixed_mask, &steps[s], &n, stream);
   };
   int rc;
-  if (mode == 2) {
+  // modes 2 and 3 start from the known molecule forward-diffused to diffusion_level
+  const bool from_known = (mode == 2 || mode == 3);
+  if (from_known) {
     mlcg_noise n = next_noise();
     if ((rc = mlcg_forward_diffuse(h, z, z_known, merge_alpha, merge_sigma, &n, stream))) return rc;
   } else {
@@ -1180,14 +1186,15 @@ static int sample_loop(mlcg_handle* h, int mode, int T, const mlcg_step_scalars*
   }
   const int r_eff = (mode == 0) ? resample_steps : std::max(resample_steps, 1);
   for (int s = T - 1; s >= 0; --s) {
-    if (mode == 2 && s > diffusion_level) continue;
+    if (from_known && s > diffusion_level) continue;
     if (mode == 0) {
       for (int r = 0; r <= r_eff; ++r)
         if ((rc = denoise(s))) return rc;
     } else {
+      // mode 3 (analogue, nothing fixed) is the merge loop without the re-injection: no launch, no noise draw
       for (int r = 0; r < r_eff; ++r) {
         if ((rc = denoise(s))) return rc;
-        if ((rc = reinject(s))) return rc;
+        if (mode != 3 && (rc = reinject(s))) return rc;
       }
       if (mode == 1 && (rc = denoise(s))) return rc;
     }
@@ -1651,6 +1658,143 @@ extern "C" int mlcg_generate_fragment(mlcg_handle* h, const mlcg_fragment* frag,
   fj.norm_mad_host = frag->norm_mad_host;
   return mlcg_generate_fragment_jobs(h, &fj, n_nodes_host, B, N, ctx_host, T, steps, resample_steps, sigma_0, alpha_0,
                                      sigma_x, seed, sample_offset, sample_ids_host, x_out, atom_class_out, bonds_out, stream);
+}
+
+// The parent table of an analogue call, validated and packed into one host blob (one upload): the job table, the job of
+// every sample, then the parents' coordinates, one-hots and fixed flags back to back.  Every section is a multiple of 4
+// bytes, so every pointer into the device copy is aligned.
+struct AnalogueTable {
+  std::vector<unsigned char> blob;
+  size_t off_jobs = 0, off_job = 0, off_x = 0, off_h = 0, off_fix = 0;
+  int n_atoms_total = 0;
+  bool any_fixed = false;
+  template <class P>
+  P* at(const DevBuf& d, size_t off) const { return reinterpret_cast<P*>(d.as<unsigned char>() + off); }
+};
+
+// n_nodes_host may be null (the eager hook: no per-sample atom counts to check).
+static int analogue_table(mlcg_handle* h, const char* what, const mlcg_analogue_jobs* aj, const int32_t* n_nodes_host, int B,
+                          int N, AnalogueTable& t) {
+  const std::string w(what);
+  if (!aj || !aj->job_of_sample_host || !aj->n_atoms_host || !aj->coords_host || !aj->one_hot_host || !aj->fixed_host)
+    FAIL(MLCG_E_ARG, w + ": null pointer");
+  const int n_jobs = aj->n_jobs;
+  if (B <= 0 || N <= 0 || N > EDGE_MAXN || n_jobs < 1) FAIL(MLCG_E_ARG, w + ": need B > 0, 1 <= N <= 39 and n_jobs >= 1");
+  std::vector<AnalogueJob> jobs((size_t)n_jobs);
+  int total = 0, with_fixed = 0;
+  for (int j = 0; j < n_jobs; ++j) {
+    const int n = aj->n_atoms_host[j];
+    if (n < 1 || n > N) FAIL(MLCG_E_ARG, w + ": a parent needs 1 <= n_atoms <= N (job " + std::to_string(j) + ")");
+    jobs[j].n_atoms = n;
+    jobs[j].off = total;
+    int n_fixed = 0;
+    for (int i = 0; i < n; ++i) n_fixed += aj->fixed_host[total + i] != 0;
+    if (n_fixed == n) FAIL(MLCG_E_ARG, w + ": every atom of the parent is fixed (job " + std::to_string(j) + ")");
+    with_fixed += n_fixed > 0;
+    total += n;
+  }
+  if (with_fixed != 0 && with_fixed != n_jobs)
+    FAIL(MLCG_E_ARG, w + ": the jobs of one call must all have fixed atoms or all have none");
+  for (int b = 0; b < B; ++b) {
+    const int j = aj->job_of_sample_host[b];
+    if (j < 0 || j >= n_jobs) FAIL(MLCG_E_ARG, w + ": job index out of range (sample " + std::to_string(b) + ")");
+    if (n_nodes_host && n_nodes_host[b] != jobs[j].n_atoms)
+      FAIL(MLCG_E_ARG, w + ": n_nodes must equal the parent's atom count (sample " + std::to_string(b) + ")");
+  }
+  t.n_atoms_total = total;
+  t.any_fixed = with_fixed > 0;
+  t.off_jobs = 0;
+  t.off_job = t.off_jobs + (size_t)n_jobs * sizeof(AnalogueJob);
+  t.off_x = t.off_job + (size_t)B * 4;
+  t.off_h = t.off_x + (size_t)total * 3 * 4;
+  t.off_fix = t.off_h + (size_t)total * 8 * 4;
+  t.blob.resize(t.off_fix + (size_t)total * 4);
+  unsigned char* p = t.blob.data();
+  memcpy(p + t.off_jobs, jobs.data(), (size_t)n_jobs * sizeof(AnalogueJob));
+  memcpy(p + t.off_job, aj->job_of_sample_host, (size_t)B * 4);
+  memcpy(p + t.off_x, aj->coords_host, (size_t)total * 3 * 4);
+  memcpy(p + t.off_h, aj->one_hot_host, (size_t)total * 8 * 4);
+  memcpy(p + t.off_fix, aj->fixed_host, (size_t)total * 4);
+  return MLCG_OK;
+}
+
+static void launch_analogue_inputs(const AnalogueTable& t, const DevBuf& d, int B, int N, float* z_known, float* fixed_mask,
+                                   cudaStream_t st) {
+  k_analogue_inputs<<<warp_grid(B), 128, 0, st>>>(t.at<float>(d, t.off_x), t.at<float>(d, t.off_h), t.at<int>(d, t.off_fix),
+                                                  t.at<int>(d, t.off_job), t.at<AnalogueJob>(d, t.off_jobs), B, N, z_known,
+                                                  fixed_mask);
+}
+
+extern "C" int mlcg_analogue_inputs(mlcg_handle* h, const mlcg_analogue_jobs* aj, int B, int N, float* z_known,
+                                    float* fixed_mask, void* stream) {
+  if (!h) return MLCG_E_ARG;
+  if (!z_known || !fixed_mask) FAIL(MLCG_E_ARG, "analogue_inputs: null pointer");
+  AnalogueTable t;
+  int rc = analogue_table(h, "analogue_inputs", aj, nullptr, B, N, t);
+  if (rc) return rc;
+  cudaStream_t st = (cudaStream_t)stream;
+  CK(h->hook_parents.ensure(t.blob.size()));
+  CK(cudaMemcpyAsync(h->hook_parents.p, t.blob.data(), t.blob.size(), cudaMemcpyHostToDevice, st));
+  launch_analogue_inputs(t, h->hook_parents, B, N, z_known, fixed_mask, st);
+  KCHECK();
+  return MLCG_OK;
+}
+
+// Draw numbering of the analogue loop: from 0, as mlcg_sample numbers it, so the graphed call equals the eager composition.
+extern "C" int mlcg_generate_analogue_jobs(mlcg_handle* h, const mlcg_analogue_jobs* aj, const int32_t* n_nodes_host, int B,
+                                           int N, const float* ctx_host, int T, const mlcg_step_scalars* steps,
+                                           int resample_steps, float sigma_0, float alpha_0, float sigma_x, uint64_t seed,
+                                           int64_t sample_offset, const int64_t* sample_ids_host, float* x_out,
+                                           int32_t* atom_class_out, int8_t* bonds_out, void* stream) {
+  if (!h) return MLCG_E_ARG;
+  if (!h->egnn_loaded || !h->seer_loaded) FAIL(MLCG_E_ARG, "generate_analogue: load both weight sets first");
+  if (!n_nodes_host || !ctx_host || !steps || !x_out || !atom_class_out || !bonds_out)
+    FAIL(MLCG_E_ARG, "generate_analogue: null pointer");
+  if (T <= 0 || resample_steps < 0) FAIL(MLCG_E_ARG, "generate_analogue: need T > 0 and resample_steps >= 0");
+  AnalogueTable t;
+  int rc = analogue_table(h, "generate_analogue", aj, n_nodes_host, B, N, t);
+  if (rc) return rc;
+  const int L = aj->diffusion_level;
+  if (L < 1 || L > T) FAIL(MLCG_E_ARG, "generate_analogue: diffusion_level must lie in [1, T]");
+  // mode 2 (merge_fragments) re-injects the fixed atoms; mode 3 is the same loop with nothing to re-inject
+  const int mode = t.any_fixed ? 2 : 3;
+  // Key of the captured graph: the geometry and every scalar baked into kernel arguments.  It starts with -(10 + mode),
+  // so it never equals a key of mlcg_generate (B first) or mlcg_generate_fragment_jobs (-1 / -2).  The job count and the
+  // packed parent length fix the layout of the uploaded table; the parents, flags, context, ids and seed are uploaded on
+  // every call, so new parents of the same sizes replay the graph.
+  std::vector<long long> key;
+  key.reserve((size_t)B + 7 * (size_t)T + 32);
+  key.push_back(-(10 + mode)); key.push_back(B); key.push_back(N); key.push_back(T); key.push_back(resample_steps);
+  key.push_back(h->precision); key.push_back(aj->n_jobs); key.push_back(t.n_atoms_total);
+  key.push_back(fbits(sigma_0)); key.push_back(fbits(alpha_0)); key.push_back(fbits(sigma_x));
+  key.push_back(L); key.push_back(fbits(aj->merge_alpha)); key.push_back(fbits(aj->merge_sigma));
+  for (int b = 0; b < B; ++b) key.push_back(n_nodes_host[b]);
+  for (int s = 0; s < T; ++s) {
+    const mlcg_step_scalars& c = steps[s];
+    for (float v : {c.t, c.alpha_ts, c.c_eps, c.c_sigma, c.alpha_s, c.sigma_s, c.blend}) key.push_back(fbits(v));
+  }
+  const size_t bn = (size_t)B * N;
+  auto upload = [&](cudaStream_t st) -> int {
+    CK(h->a_tab.ensure(t.blob.size()));
+    CK(h->f_zk.ensure(bn * ZC * 4));
+    CK(h->f_fm.ensure(bn * 4));
+    CK(cudaMemcpyAsync(h->a_tab.p, t.blob.data(), t.blob.size(), cudaMemcpyHostToDevice, st));
+    return MLCG_OK;
+  };
+  auto device = [&](void* s) -> int {
+    cudaStream_t st = (cudaStream_t)s;
+    float* zk = h->f_zk.as<float>();
+    float* fm = h->f_fm.as<float>();
+    launch_analogue_inputs(t, h->a_tab, B, N, zk, fm, st);
+    KCHECK();
+    int rc2 = sample_loop(h, mode, T, steps, resample_steps, L, aj->merge_alpha, aj->merge_sigma, sigma_0, alpha_0, sigma_x,
+                          h->g_ctx.as<float>(), zk, fm, nullptr, seed, sample_offset, h->g_ids.as<int64_t>(),
+                          h->g_z.as<float>(), h->g_x.as<float>(), h->g_cls.as<int32_t>(), nullptr, nullptr, 0, s);
+    if (rc2) return rc2;
+    return seer_device(h, s);
+  };
+  return generate_graphed(h, key, n_nodes_host, B, N, nullptr, 0, ctx_host, seed, sample_offset, sample_ids_host, x_out,
+                          atom_class_out, bonds_out, stream, upload, device);
 }
 
 // ---------------------------------------------------------------------------------------------------------------

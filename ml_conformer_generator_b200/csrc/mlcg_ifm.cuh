@@ -5,6 +5,7 @@
 //                       eigen-decomposition (torch.linalg.eigh there; cyclic Jacobi here) and the normalised context
 //   k_ifm_merge_inputs  inverse_coord_transform (:508-524) + ifm_prepare_fragments_for_merge (:460-505): z_known and
 //                       fixed_mask of the merge loop, built straight from the first loop's device outputs
+//   k_analogue_inputs   z_known and fixed_mask of the analogue loop, from a per-job table of parent molecules
 #pragma once
 #include "mlcg_common.cuh"
 
@@ -142,6 +143,46 @@ __global__ void k_ifm_merge_inputs(const float* __restrict__ x_gen, const int* _
 #pragma unroll
     for (int c = 0; c < ZC; ++c) dst[c] = out[c];
     fixed_mask[(size_t)b * N + i] = (i < n_ff) ? 1.0f : 0.0f;
+  }
+}
+
+// One job of an analogue call (mlcg_generate_analogue_jobs): its parent's rows in the packed parent table.
+struct AnalogueJob {
+  int n_atoms;  // atoms of the parent (= n_nodes of every sample of the job)
+  int off;      // row of the parent's first atom in the packed p_x / p_h / p_fix
+};
+
+// z_known (B,N,11) and fixed_mask (B,N) of the analogue loop (merge_fragments run on a whole parent molecule).  Sample b
+// has the parent of jobs[job[b]]: atom i < n_atoms is the parent's atom i (centred coordinates + raw 0/1 one-hot) with
+// fixed_mask = its fixed flag; rows beyond n_atoms are zero.  One warp per sample, lanes own atoms (lane, lane + 32), as
+// the step kernels.  A separate kernel rather than a k_ifm_merge_inputs variant: its table (per-atom fixed flags, no
+// generated part) and launch shape differ, and k_ifm_merge_inputs stays exactly as it was.
+__global__ void k_analogue_inputs(const float* __restrict__ p_x, const float* __restrict__ p_h, const int* __restrict__ p_fix,
+                                  const int* __restrict__ job, const AnalogueJob* __restrict__ jobs, int B, int N,
+                                  float* __restrict__ z_known, float* __restrict__ fixed_mask) {
+  const int b = (blockIdx.x * blockDim.x + threadIdx.x) >> 5, lane = threadIdx.x & 31;
+  if (b >= B) return;
+  const AnalogueJob q = jobs[job[b]];
+#pragma unroll
+  for (int s = 0; s < 2; ++s) {
+    const int i = lane + 32 * s;
+    if (i >= N) continue;
+    float out[ZC];
+#pragma unroll
+    for (int c = 0; c < ZC; ++c) out[c] = 0.f;
+    float fm = 0.f;
+    if (i < q.n_atoms) {
+      const size_t r = (size_t)(q.off + i);
+#pragma unroll
+      for (int c = 0; c < 3; ++c) out[c] = p_x[r * 3 + c];
+#pragma unroll
+      for (int c = 0; c < 8; ++c) out[3 + c] = p_h[r * 8 + c];
+      fm = p_fix[r] ? 1.0f : 0.0f;
+    }
+    float* dst = z_known + ((size_t)b * N + i) * ZC;
+#pragma unroll
+    for (int c = 0; c < ZC; ++c) dst[c] = out[c];
+    fixed_mask[(size_t)b * N + i] = fm;
   }
 }
 

@@ -144,11 +144,14 @@ class Engine:
                diffusion_level: int = 50, blend_power: int = 3, noise_tape: Optional[torch.Tensor] = None,
                seed: int = 0, sample_offset: int = 0, trace: bool = False, sample_ids=None):
         """Runs the reverse loop for the batch set by set_batch.  Returns (x (B,N,3), atom_class (B,N) int32[, trace]).
-        Device noise is keyed by (seed, global sample id): `sample_ids` (B int64) or `sample_offset + b`."""
-        modes = {"forward": 0, "inpaint": 1, "merge": 2}
+        Device noise is keyed by (seed, global sample id): `sample_ids` (B int64) or `sample_offset + b`.  Modes:
+        "forward", "inpaint", "merge" (merge_fragments) and "analogue" (the merge loop with nothing re-injected: z_known
+        forward-diffused to `diffusion_level`, then denoised; fixed_mask is ignored)."""
+        modes = {"forward": 0, "inpaint": 1, "merge": 2, "analogue": 3}
         gamma, steps = self._steps(T, blend_power)
         dec = decode_scalars(gamma)
-        lvl = forward_level_scalars(gamma, diffusion_level) if mode == "merge" else {"alpha": 0.0, "sigma": 0.0}
+        from_known = mode in ("merge", "analogue")
+        lvl = forward_level_scalars(gamma, diffusion_level) if from_known else {"alpha": 0.0, "sigma": 0.0}
         B, N = self.B, self.N
         dev = self.device
         ctx = ctx.to(dev, torch.float32).contiguous()
@@ -163,13 +166,15 @@ class Engine:
             if ids.numel() != B:
                 raise ValueError("sample: sample_ids must hold one id per sample")
         r_eff = resample_steps if mode == "forward" else max(resample_steps, 1)
-        n_active = T if mode != "merge" else min(diffusion_level, T - 1) + 1
+        n_active = T if not from_known else min(diffusion_level, T - 1) + 1
         if mode == "forward":
             n_fwd, n_draw = T * (r_eff + 1) + 1, 1 + T * (r_eff + 1) + 1
         elif mode == "inpaint":
             n_fwd, n_draw = T * (r_eff + 1) + 1, 1 + T * (2 * r_eff + 1) + 1
-        else:
+        elif mode == "merge":
             n_fwd, n_draw = n_active * r_eff + 1, 1 + n_active * 2 * r_eff + 1
+        else:
+            n_fwd, n_draw = n_active * r_eff + 1, 1 + n_active * r_eff + 1
         if tape is not None and tuple(tape.shape) != (n_draw, B, N, 11):
             raise ValueError("sample: noise tape must be (%d,%d,%d,11), got %s" % (n_draw, B, N, tuple(tape.shape)))
         z = torch.empty(B, N, 11, device=dev)
@@ -376,6 +381,78 @@ class Engine:
         del keep
         self._check(rc, "generate_fragment")
         self.check_finite("generate_fragment")
+        self.B, self.N = B, N
+        self.n_nodes = torch.from_numpy(nn.copy())
+        return out
+
+    @staticmethod
+    def _analogue_table(what, job_of_sample, B, parents, fixed):
+        """mlcg_analogue_jobs (diffusion level unset) and the host arrays it points to, which must outlive the call."""
+        job = np.ascontiguousarray(np.asarray(job_of_sample, dtype=np.int32).reshape(-1))
+        if job.size != B:
+            raise ValueError("%s: job_of_sample must hold one job per sample" % what)
+        if fixed is not None and len(fixed) != len(parents):
+            raise ValueError("%s: fixed must hold one flag array per parent" % what)
+        px, ph, pf = [], [], []
+        for j, (x, h) in enumerate(parents):
+            x = np.asarray(torch.as_tensor(x).detach().cpu().numpy(), dtype=np.float32)
+            h = np.asarray(torch.as_tensor(h).detach().cpu().numpy(), dtype=np.float32)
+            if x.ndim != 2 or x.shape[1] != 3 or h.shape != (x.shape[0], 8):
+                raise ValueError("%s: a parent must be coordinates (n,3) and a one-hot (n,8)" % what)
+            f = np.zeros(x.shape[0], np.int32) if fixed is None or fixed[j] is None else \
+                np.asarray(fixed[j]).reshape(-1).astype(np.int32)
+            if f.size != x.shape[0]:
+                raise ValueError("%s: the fixed flags must hold one entry per parent atom" % what)
+            px.append(x)
+            ph.append(h)
+            pf.append(f)
+        keep = [job, np.array([x.shape[0] for x in px], dtype=np.int32),
+                np.ascontiguousarray(np.concatenate(px).reshape(-1, 3)), np.ascontiguousarray(np.concatenate(ph).reshape(-1, 8)),
+                np.ascontiguousarray(np.concatenate(pf))]
+        return _lib.AnalogueJobs(len(px), *(a.ctypes.data for a in keep)), keep
+
+    def analogue_inputs(self, job_of_sample, parents, fixed, max_n_nodes: int):
+        """Device version of the analogue jobs' first step (mlcg_analogue_inputs): (z_known (B,N,11), fixed_mask (B,N)) with
+        sample b holding parent job_of_sample[b] = (centred coordinates (n,3), one-hot (n,8)) and its fixed flags
+        (fixed[j]: (n,) 0/1, or None for none)."""
+        B, N = int(np.size(job_of_sample)), int(max_n_nodes)
+        aj, keep = self._analogue_table("analogue_inputs", job_of_sample, B, parents, fixed)
+        zk = torch.empty(B, N, 11, device=self.device)
+        fm = torch.empty(B, N, device=self.device)
+        self._check(self.lib.mlcg_analogue_inputs(self.h, C.byref(aj), B, N, _ptr(zk), _ptr(fm), self._stream()),
+                    "analogue_inputs")
+        del keep
+        return zk, fm
+
+    def generate_analogue_jobs_host(self, n_nodes: np.ndarray, max_n_nodes: int, ctx: np.ndarray, job_of_sample, parents,
+                                    fixed=None, T: int = 100, resample_steps: int = 0, blend_power: int = 3,
+                                    diffusion_level: int = 50, seed: int = 0, sample_offset: int = 0, sample_ids=None,
+                                    out=None, device_out: bool = False):
+        """Analogues of parent molecules in one call (mlcg_generate_analogue_jobs): sample b starts from parent
+        parents[job_of_sample[b]] = (coordinates (n,3) centred on their mean, raw 0/1 one-hot (n,8)) forward-diffused to
+        `diffusion_level` and is denoised from there; n_nodes[b] must be that parent's n.  fixed[j] ((n,) 0/1 or None)
+        marks atoms re-injected at every step as merge_fragments re-injects a fragment; in one call every job has a fixed
+        atom or none has.  `ctx` (B,3) is every sample's normalised context.  Same outputs, noise keys and graph replay as
+        generate_fragment_jobs_host; every sample equals a call holding only its own job with the same id, bit for bit,
+        and the result equals the eager composition analogue_inputs + sample + the GCN."""
+        nn, ctxh, ids, out = self._host_call_inputs("generate_analogue_jobs_host", n_nodes, max_n_nodes, ctx, sample_ids,
+                                                    out, device_out)
+        B, N = int(nn.size), int(max_n_nodes)
+        aj, keep = self._analogue_table("generate_analogue_jobs_host", job_of_sample, B, parents, fixed)
+        gamma, steps = self._steps_cached(T, blend_power)
+        dec = decode_scalars(gamma)
+        if not 1 <= int(diffusion_level) <= T:
+            raise ValueError("generate_analogue_jobs_host: diffusion_level must lie in [1, T=%d]" % T)
+        lvl = forward_level_scalars(gamma, int(diffusion_level))
+        aj.diffusion_level, aj.merge_alpha, aj.merge_sigma = int(diffusion_level), lvl["alpha"], lvl["sigma"]
+        rc = self.lib.mlcg_generate_analogue_jobs(self.h, C.byref(aj), nn.ctypes.data_as(C.c_void_p), B, N, _ptr(ctxh), T,
+                                                  steps, resample_steps, dec["sigma_0"], dec["alpha_0"], dec["sigma_x"],
+                                                  seed, sample_offset,
+                                                  None if ids is None else ids.ctypes.data_as(C.c_void_p), _ptr(out[0]),
+                                                  _ptr(out[1]), _ptr(out[2]), self._stream())
+        del keep
+        self._check(rc, "generate_analogue")
+        self.check_finite("generate_analogue")
         self.B, self.N = B, N
         self.n_nodes = torch.from_numpy(nn.copy())
         return out

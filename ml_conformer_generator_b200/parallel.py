@@ -60,7 +60,8 @@ def unpack_results(buf: torch.Tensor, max_n_nodes: int, extra=()) -> Tuple[torch
     out = [x, cls, bonds]
     for dtype, shape in extra:
         w = _extra_bytes([(dtype, shape)])
-        out.append(buf[:, c:c + w].clone().view(dtype).reshape(n, *shape))
+        # flattened before the copy: clone() keeps a single row's stride, which an 8-byte view cannot take
+        out.append(buf[:, c:c + w].reshape(-1).clone().view(dtype).reshape(n, *shape))
         c += w
     return tuple(out)
 
@@ -148,16 +149,18 @@ def generate_jobs_sharded(engine, jobs, T: int = 100, resample_steps: int = 0, b
                           max_n_nodes: Optional[int] = None, keep_best: Optional[int] = None, scorer=None):
     """MLConformerGenerator.generate_jobs over the ranks of `group`: the jobs are flattened as there (jobs.flatten_jobs),
     the flat samples dealt with `shard_indices`, and each rank runs the per-kind packed calls of its samples
-    (jobs.run_packed, device outputs).  One packed all-gather, then the split per job: every rank returns one dict per
+    (jobs.run_packed, device outputs; analogue jobs included).  One packed all-gather, then the split per job: every rank returns one dict per
     job, equal bit for bit to the single-GPU result.  Jobs with a `reference_conformer` are scored by each rank on its
     own shard (jobs.score_packed with `scorer`, default a ShapeScorer on the engine); the scores travel in the same
     all-gather, and the `keep_best` selection runs after it, identically on every rank."""
     from .config import CONTEXT_NORMS, MAX_N_NODES, MIN_N_NODES
-    from .jobs import attach_scores, check_keep_best, flatten_jobs, run_packed, score_packed, score_row_spec, split_jobs
+    from .jobs import (analogue_levels, attach_scores, check_keep_best, flatten_jobs, run_packed, score_packed,
+                       score_row_spec, split_jobs)
     norms = CONTEXT_NORMS if context_norms is None else context_norms
     packed = flatten_jobs(jobs, seed, norms, MIN_N_NODES if min_n_nodes is None else min_n_nodes,
                           MAX_N_NODES if max_n_nodes is None else max_n_nodes)
     check_keep_best(packed, keep_best)
+    analogue_levels(packed, ifm_diffusion_level, T)  # on every rank, also one with an empty shard
     if packed.scored and scorer is None:
         from .shape_similarity import ShapeScorer
         scorer = ShapeScorer(engine)
