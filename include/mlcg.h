@@ -148,12 +148,25 @@ int mlcg_seer_inputs(mlcg_handle* h, const float* x, const int32_t* atom_class, 
 int mlcg_seer_forward(mlcg_handle* h, const int32_t* elements, const float* dist, const float* adj, float* logits,
                       int8_t* bonds, int B, void* stream);
 
-/* End-to-end call with HOST inputs (what MLConformerGenerator.generate_tensors and the multi-GPU driver use): uploads
- * n_nodes / context / sample ids, runs mlcg_set_batch (only when the geometry changed) + mlcg_sample(mode 0) +
- * mlcg_seer_inputs + mlcg_seer_forward -- replayed as one CUDA graph from the second call with the same geometry on --
- * and copies the results out.  n_nodes_host (B), ctx_host (B,3), sample_ids_host (B int64 global ids, or NULL =
- * sample_offset + b) are HOST arrays.  x_out (B,N,3), atom_class_out (B,N) int32, bonds_out (B,42,42) int8 may be
- * pinned HOST or DEVICE buffers (copied with cudaMemcpyDefault).  Synchronous. */
+/* ---- Host generation calls: mlcg_generate, mlcg_generate_fragment(_jobs), mlcg_generate_analogue_jobs ---------------
+ * End-to-end calls with HOST inputs (what MLConformerGenerator.generate_tensors and the multi-GPU driver use).  They share
+ * these arguments and this behaviour:
+ *  - n_nodes_host (B), ctx_host (B,3) normalised context, steps (T) and sample_ids_host (B int64 global ids, or NULL =
+ *    sample_offset + b) are HOST arrays; x_out (B,N,3), atom_class_out (B,N) int32 and bonds_out (B,42,42) int8 may be
+ *    pinned HOST or DEVICE buffers (copied with cudaMemcpyDefault).
+ *  - synchronous: the call returns when the outputs are written.  A NULL stream runs the call on a private stream.
+ *  - the device sequence (the kind's reverse loops, then mlcg_seer_inputs + mlcg_seer_forward) runs eagerly on the first
+ *    call with a key, is captured into a CUDA graph on the second and replayed from then on.  The key is the kind, the
+ *    geometry (B, N, per-sample atom counts, the kind's table sizes) and every scalar baked into the sequence (precision,
+ *    schedule, decode scalars, the kind's loop settings).  A new key rebuilds the batch plan (mlcg_set_batch); calls of
+ *    different kinds therefore invalidate each other's graph.
+ *  - the context, the sample ids, {seed, sample_offset} and the kind's job table are uploaded on every call, so a replay
+ *    never sees a previous call's inputs, and new inputs of the same sizes replay the graph.
+ *  - the noise is keyed by (seed, global sample id), and every kernel works on each sample alone: a sample's result does
+ *    not depend on the others in the call.
+ * Each returns MLCG_E_ARG for a null pointer among the shared arguments. */
+
+/* Plain generation: mlcg_sample(mode 0) from noise.  Returns MLCG_E_STATE if either weight set is not loaded. */
 int mlcg_generate(mlcg_handle* h, const int32_t* n_nodes_host, int B, int N, const float* ctx_host, int T,
                   const mlcg_step_scalars* steps, int resample_steps, float sigma_0, float alpha_0, float sigma_x,
                   uint64_t seed, int64_t sample_offset, const int64_t* sample_ids_host, float* x_out,
@@ -178,18 +191,14 @@ typedef struct {
   const float* norm_mad_host;        /* mode 2: 3, CONTEXT_NORMS mad */
 } mlcg_fragment;
 
-/* Fragment-conditioned counterpart of mlcg_generate: same inputs, outputs, synchronous behaviour and CUDA-graph replay
- * (from the second call with the same key on), plus the fragment.  ctx_host (B,3) is the normalised reference context
- * of every sample.  The device sequence is the eager composition of MLConformerGenerator.edm_sample_tensors followed by
- * the GCN -- mode 1: z_known / fixed_mask from the fragment (prepare_fragment, utils/mol_utils.py:298-342),
- * mlcg_sample(mode 1); mode 2: mlcg_ifm_context on the whole atom counts, mlcg_sample(mode 0) on the atoms still to be
- * generated with the context it wrote, mlcg_ifm_merge_inputs, mlcg_sample(mode 2) -- then mlcg_seer_inputs +
- * mlcg_seer_forward, with the same noise keys and draw numbers; the results equal that composition bit for bit.  The
- * fragment, its prologue, context, sample ids and {seed, sample_offset} are uploaded on every call, so a replay never sees
- * a previous call's inputs, and another fragment or reference context of the same size replays the captured graph.  A
- * call of mlcg_generate and one of mlcg_generate_fragment(_jobs) invalidate each other's graph.  This is the one-job case
- * of mlcg_generate_fragment_jobs.  Returns MLCG_E_ARG for a mode other than 1 or 2, n_ff < 1, n_ff >= min(n_nodes),
- * N - n_ff < 1, a null pointer or weights not loaded. */
+/* Host generation around a fixed fragment.  The device sequence is the eager composition of
+ * MLConformerGenerator.edm_sample_tensors followed by the GCN -- mode 1: z_known / fixed_mask from the fragment
+ * (prepare_fragment, utils/mol_utils.py:298-342), mlcg_sample(mode 1); mode 2: mlcg_ifm_context on the whole atom
+ * counts, mlcg_sample(mode 0) on the atoms still to be generated with the context it wrote, mlcg_ifm_merge_inputs,
+ * mlcg_sample(mode 2) -- with the same noise keys and draw numbers; the results equal that composition bit for bit.  The
+ * fragment and its prologue are the job table.  This is the one-job case of mlcg_generate_fragment_jobs.  Returns
+ * MLCG_E_ARG for a mode other than 1 or 2, n_ff < 1, n_ff >= min(n_nodes), N - n_ff < 1, a null pointer or weights not
+ * loaded. */
 int mlcg_generate_fragment(mlcg_handle* h, const mlcg_fragment* frag, const int32_t* n_nodes_host, int B, int N,
                            const float* ctx_host, int T, const mlcg_step_scalars* steps, int resample_steps, float sigma_0,
                            float alpha_0, float sigma_x, uint64_t seed, int64_t sample_offset,
@@ -215,14 +224,11 @@ typedef struct {
 
 /* mlcg_generate_fragment for many jobs at once: sample b runs with the fragment (and, mode 2, the prologue) of job
  * job_of_sample[b]; every other input and output is that of mlcg_generate_fragment.  Mode 2 generates the atoms still to
- * be generated, n_nodes[b] - n_ff[job[b]], padded to N - min(n_ff over the samples).  Every kernel works on each sample
- * alone and the noise is keyed by the global sample id, so a sample's result equals that of a call holding only its own
- * job with the same id, bit for bit.  The graph key is the geometry (mode, B, N, per-sample n_nodes and n_ff, the job
- * count and the packed fragment length) and the shared scalars; the fragments, the job table, the job of every sample,
- * the context, the ids and the seed are uploaded on every call, so other references or fragments of the same sizes
- * replay the captured graph.  Returns MLCG_E_ARG for a mode other than 1 or 2, n_jobs < 1, a job index out of range,
- * n_ff < 1 or N - n_ff < 1 for any job, n_ff[job[b]] >= n_nodes[b] for any sample, a null pointer or weights not
- * loaded. */
+ * be generated, n_nodes[b] - n_ff[job[b]], padded to N - min(n_ff over the samples).  A sample's result equals that of a
+ * call holding only its own job with the same id, bit for bit.  The table sizes in the key are the per-sample n_ff, the
+ * job count and the packed fragment length, so other references or fragments of the same sizes replay the graph.
+ * Returns MLCG_E_ARG for a mode other than 1 or 2, n_jobs < 1, a job index out of range, n_ff < 1 or N - n_ff < 1 for
+ * any job, n_ff[job[b]] >= n_nodes[b] for any sample, a null pointer or weights not loaded. */
 int mlcg_generate_fragment_jobs(mlcg_handle* h, const mlcg_fragment_jobs* jobs, const int32_t* n_nodes_host, int B, int N,
                                 const float* ctx_host, int T, const mlcg_step_scalars* steps, int resample_steps,
                                 float sigma_0, float alpha_0, float sigma_x, uint64_t seed, int64_t sample_offset,
@@ -248,14 +254,10 @@ typedef struct {
  * denoised from there to 0 (L = 1 returns the parent up to the last steps' noise, L = T is a fresh sample).  With fixed
  * atoms the loop is merge_fragments' (equivariant_diffusion.py:515-607, mlcg_sample mode 2): the fixed atoms are
  * re-injected at every step with the blend (1 - s/T)^blend_power (in steps) and the fixed-atom centre-of-mass
- * alignment.  With none it is mlcg_sample mode 3.  Inputs, outputs, synchronous behaviour and CUDA-graph replay (from the
- * second call with the same key on) as mlcg_generate_fragment_jobs; the device sequence is mlcg_analogue_inputs,
- * mlcg_sample (mode 2 or 3, draws numbered from 0) and mlcg_seer_inputs + mlcg_seer_forward, and the results equal that
- * eager composition bit for bit.  Every kernel works on each sample alone and the noise is keyed by the global sample id,
- * so a sample's result equals that of a call holding only its own job with the same id.  The graph key is the geometry
- * (B, N, per-sample n_nodes, the job count and the packed parent length), the mode and the shared scalars; the parents,
- * flags, job of every sample, context, ids and seed are uploaded on every call, so new parents of the same sizes replay
- * the captured graph.  ctx_host (B,3) is the normalised context of every sample.  Atom class 7 (Br) is never decoded (the
+ * alignment.  With none it is mlcg_sample mode 3.  The device sequence is mlcg_analogue_inputs, mlcg_sample (mode 2 or 3,
+ * draws numbered from 0) and the GCN, and the results equal that eager composition bit for bit.  A sample's result
+ * equals that of a call holding only its own job with the same id.  The table sizes in the key are the job count and
+ * the packed parent length, so new parents of the same sizes replay the graph.  Atom class 7 (Br) is never decoded (the
  * argmax reads 7 channels), fixed atoms included.  Returns MLCG_E_ARG for a job index out of range,
  * n_nodes[b] != n_atoms[job[b]], a call mixing jobs with and without fixed atoms, a job with every atom fixed,
  * n_atoms outside [1, N], N outside [1, 39], diffusion_level outside [1, T], n_jobs < 1, a null pointer or weights not

@@ -128,14 +128,13 @@ def load() -> C.CDLL:
                                 C.c_uint64, C.c_int64, vp, vp, vp, vp, vp, vp, vp]
     lib.mlcg_seer_inputs.argtypes = [vp, vp, vp, vp, vp, vp, vp]
     lib.mlcg_seer_forward.argtypes = [vp, vp, vp, vp, vp, vp, ci, vp]
-    lib.mlcg_generate.argtypes = [vp, vp, ci, ci, vp, ci, C.POINTER(StepScalars), ci, cf, cf, cf, C.c_uint64,
-                                  C.c_int64, vp, vp, vp, vp, vp]
-    lib.mlcg_generate_fragment.argtypes = [vp, C.POINTER(Fragment), vp, ci, ci, vp, ci, C.POINTER(StepScalars), ci, cf, cf,
-                                           cf, C.c_uint64, C.c_int64, vp, vp, vp, vp, vp]
-    lib.mlcg_generate_fragment_jobs.argtypes = [vp, C.POINTER(FragmentJobs), vp, ci, ci, vp, ci, C.POINTER(StepScalars), ci,
-                                                cf, cf, cf, C.c_uint64, C.c_int64, vp, vp, vp, vp, vp]
-    lib.mlcg_generate_analogue_jobs.argtypes = [vp, C.POINTER(AnalogueJobs), vp, ci, ci, vp, ci, C.POINTER(StepScalars), ci,
-                                                cf, cf, cf, C.c_uint64, C.c_int64, vp, vp, vp, vp, vp]
+    # the arguments every host generation call ends with: n_nodes, B, N, ctx, T, steps, resample_steps, sigma_0, alpha_0,
+    # sigma_x, seed, sample_offset, sample_ids, x / atom class / bond outputs, stream
+    gen = [vp, ci, ci, vp, ci, C.POINTER(StepScalars), ci, cf, cf, cf, C.c_uint64, C.c_int64, vp, vp, vp, vp, vp]
+    lib.mlcg_generate.argtypes = [vp] + gen
+    lib.mlcg_generate_fragment.argtypes = [vp, C.POINTER(Fragment)] + gen
+    lib.mlcg_generate_fragment_jobs.argtypes = [vp, C.POINTER(FragmentJobs)] + gen
+    lib.mlcg_generate_analogue_jobs.argtypes = [vp, C.POINTER(AnalogueJobs)] + gen
     lib.mlcg_analogue_inputs.argtypes = [vp, C.POINTER(AnalogueJobs), ci, ci, vp, vp, vp]
     lib.mlcg_nonfinite.argtypes = [vp, vp]
     lib.mlcg_num_edge_tiles.argtypes = [vp]

@@ -102,26 +102,25 @@ struct mlcg_handle {
   DevBuf s_ld, s_la, s_rowd, s_rowa, s_x64, s_y_op, s_x, s_emb, s_add, s_raw, s_y_f32;
   // mlcg_generate device buffers
   DevBuf g_ctx, g_z, g_x, g_cls, g_el, g_dist, g_adj, g_bonds, g_ids;
-  // mlcg_generate_fragment(_jobs) device buffers: packed fragments, job table, job of every sample, z_known / fixed_mask,
-  // and the first IFM loop's context and outputs
-  DevBuf f_ffx, f_ffh, f_jobs, f_job, f_zk, f_fm, f_ctx, f_shift, f_rot, f_ngen, f_xg, f_clsg;
-  DevBuf hook_job;  // the one-job table of the eager hooks mlcg_ifm_context / mlcg_ifm_merge_inputs
-  // mlcg_generate_analogue_jobs: the parent table (AnalogueTable's blob); z_known / fixed_mask go to f_zk / f_fm.  The
-  // eager hook mlcg_analogue_inputs has a buffer of its own, so it never moves one a captured graph reads.
-  DevBuf a_tab, hook_parents;
+  // mlcg_generate_fragment(_jobs) / mlcg_generate_analogue_jobs device buffers: the uploaded job table (JobTable),
+  // z_known / fixed_mask, and the first IFM loop's context and outputs
+  DevBuf j_tab, f_zk, f_fm, f_ctx, f_shift, f_rot, f_ngen, f_xg, f_clsg;
+  // The tables of the eager hooks mlcg_ifm_context / mlcg_ifm_merge_inputs (one job) and mlcg_analogue_inputs: buffers of
+  // their own, so a hook never moves one a captured graph reads.
+  DevBuf hook_job, hook_parents;
   DevBuf nf_flag;  // set by k_decode when a generated coordinate is not finite (mlcg_nonfinite)
   std::vector<int64_t> ids_stage;
   // test gemm
   DevBuf tg_a, tg_w, tg_b, tg_c;
-  // CUDA-graph replay of mlcg_generate (whole reverse loop + GCN as one graph)
+  // CUDA-graph replay of the host generation calls (whole device sequence + GCN as one graph)
   DevBuf noise_ctl;               // {seed, sample_offset} read by the noise kernels when use_noise_ctl is set
   bool use_noise_ctl = false;
   cudaGraphExec_t gen_graph = nullptr;
-  std::vector<long long> gen_key;  // geometry / schedule the graph was captured for
+  std::vector<long long> gen_key;  // graph_key of the call the graph was captured for
   int gen_key_hits = 0;            // calls seen with the current key (1st runs eagerly, 2nd captures)
   long long gen_graph_launches = 0;
-  long long graph_captures = 0;    // CUDA graphs captured by mlcg_generate / mlcg_generate_fragment(_jobs)
-  cudaStream_t own_stream = nullptr;  // used by mlcg_generate when the caller passes the NULL stream (not capturable)
+  long long graph_captures = 0;    // CUDA graphs captured by the host generation calls
+  cudaStream_t own_stream = nullptr;  // used by the host generation calls when the caller passes the NULL stream (not capturable)
   // mlcg_egnn_forward_breakdown: events recorded after every launch of one forward, tagged with a kernel class
   bool bd_on = false;
   std::vector<std::pair<int, cudaEvent_t>> bd_ev;
@@ -454,8 +453,8 @@ extern "C" void mlcg_destroy(mlcg_handle* h) {
                     &h->h_res, &h->pq, &h->h_op, &h->agg_op, &h->t_op, &h->agg_f32, &h->t_f32, &h->a1, &h->m2, &h->t_dev,
                     &h->eps_dev, &h->s_ld, &h->s_la, &h->s_rowd, &h->s_rowa, &h->s_x64, &h->s_y_op, &h->s_x, &h->s_emb,
                     &h->s_add, &h->s_raw, &h->s_y_f32, &h->g_ctx, &h->g_z, &h->g_x, &h->g_cls, &h->g_el, &h->g_dist,
-                    &h->g_adj, &h->g_bonds, &h->g_ids, &h->f_ffx, &h->f_ffh, &h->f_jobs, &h->f_job, &h->hook_job, &h->f_zk, &h->f_fm, &h->f_ctx, &h->f_shift,
-                    &h->f_rot, &h->f_ngen, &h->f_xg, &h->f_clsg, &h->nf_flag, &h->tg_a, &h->tg_w, &h->tg_b, &h->tg_c})
+                    &h->g_adj, &h->g_bonds, &h->g_ids, &h->j_tab, &h->hook_job, &h->hook_parents, &h->f_zk, &h->f_fm, &h->f_ctx,
+                    &h->f_shift, &h->f_rot, &h->f_ngen, &h->f_xg, &h->f_clsg, &h->nf_flag, &h->tg_a, &h->tg_w, &h->tg_b, &h->tg_c})
     b->release();
   delete h;
 }
@@ -1127,66 +1126,73 @@ extern "C" int mlcg_decode(mlcg_handle* h, const float* z0, const float* eps0, f
 // ---------------------------------------------------------------------------------------------------------------
 // whole reverse loop
 // ---------------------------------------------------------------------------------------------------------------
-// The reverse loop of mlcg_sample with its noise draws numbered from `draw0` on (mlcg_sample: 0).
-static int sample_loop(mlcg_handle* h, int mode, int T, const mlcg_step_scalars* steps, int resample_steps,
-                       int diffusion_level, float merge_alpha, float merge_sigma, float sigma_0, float alpha_0, float sigma_x,
-                       const float* ctx, const float* z_known, const float* fixed_mask, const float* noise_tape, uint64_t seed,
-                       int64_t sample_offset, const int64_t* sample_ids, float* z, float* x_out, int32_t* atom_class_out,
-                       float* trace_z, float* trace_eps, uint64_t draw0, void* stream) {
+// Arguments of one reverse loop, in the order of mlcg_sample's parameters; its noise draws are numbered from `draw0` on
+// (mlcg_sample: 0).
+struct LoopArgs {
+  int mode = 0, T = 0;
+  const mlcg_step_scalars* steps = nullptr;
+  int resample_steps = 0, diffusion_level = 0;
+  float merge_alpha = 0.f, merge_sigma = 0.f, sigma_0 = 0.f, alpha_0 = 0.f, sigma_x = 0.f;
+  const float *ctx = nullptr, *z_known = nullptr, *fixed_mask = nullptr, *noise_tape = nullptr;
+  uint64_t seed = 0;
+  int64_t sample_offset = 0;
+  const int64_t* sample_ids = nullptr;
+  float* z = nullptr;
+  float* x_out = nullptr;
+  int32_t* atom_class_out = nullptr;
+  float *trace_z = nullptr, *trace_eps = nullptr;
+  uint64_t draw0 = 0;
+};
+
+// The reverse loop of mlcg_sample.
+static int sample_loop(mlcg_handle* h, const LoopArgs& a, void* stream) {
   STEP_PROLOGUE("sample");
   if (!h->egnn_loaded) FAIL(MLCG_E_STATE, "sample: load the EGNN weights first");
-  if (mode < 0 || mode > 3 || T <= 0 || !steps || !ctx || !z || !x_out || !atom_class_out || resample_steps < 0)
+  const int mode = a.mode;
+  if (mode < 0 || mode > 3 || a.T <= 0 || !a.steps || !a.ctx || !a.z || !a.x_out || !a.atom_class_out || a.resample_steps < 0)
     FAIL(MLCG_E_ARG, "sample: bad argument");
-  if ((mode == 1 || mode == 2) && (!z_known || !fixed_mask)) FAIL(MLCG_E_ARG, "sample: inpaint / merge need z_known and fixed_mask");
-  if (mode == 3 && !z_known) FAIL(MLCG_E_ARG, "sample: analogue needs z_known");
+  if ((mode == 1 || mode == 2) && (!a.z_known || !a.fixed_mask)) FAIL(MLCG_E_ARG, "sample: inpaint / merge need z_known and fixed_mask");
+  if (mode == 3 && !a.z_known) FAIL(MLCG_E_ARG, "sample: analogue needs z_known");
   const size_t zsz = (size_t)h->pl->B * h->pl->N * ZC;
   float* eps = h->eps_dev.as<float>();
   float* tdev = h->t_dev.as<float>();
-  uint64_t draw = draw0;
+  uint64_t draw = a.draw0;
   long long fwd = 0;
   auto next_noise = [&]() {
-    mlcg_noise n;
-    n.raw = noise_tape ? noise_tape + (size_t)draw * zsz : nullptr;
-    n.seed = seed;
-    n.draw = draw;
-    n.sample_offset = sample_offset;
-    n.sample_ids = sample_ids;
+    const mlcg_noise n{a.noise_tape ? a.noise_tape + (size_t)draw * zsz : nullptr, a.seed, draw, a.sample_offset, a.sample_ids};
     ++draw;
     return n;
   };
   auto network = [&](float tval) -> int {
     k_fill_f32<<<(h->pl->B + 127) / 128, 128, 0, st>>>(tdev, tval, h->pl->B);
     KCHECK();
-    if (trace_z) CK(cudaMemcpyAsync(trace_z + (size_t)fwd * zsz, z, zsz * sizeof(float), cudaMemcpyDeviceToDevice, st));
-    int rc = mlcg_egnn_forward(h, tdev, z, ctx, eps, stream);
+    if (a.trace_z) CK(cudaMemcpyAsync(a.trace_z + (size_t)fwd * zsz, a.z, zsz * sizeof(float), cudaMemcpyDeviceToDevice, st));
+    int rc = mlcg_egnn_forward(h, tdev, a.z, a.ctx, eps, stream);
     if (rc) return rc;
-    if (trace_eps) CK(cudaMemcpyAsync(trace_eps + (size_t)fwd * zsz, eps, zsz * sizeof(float), cudaMemcpyDeviceToDevice, st));
+    if (a.trace_eps) CK(cudaMemcpyAsync(a.trace_eps + (size_t)fwd * zsz, eps, zsz * sizeof(float), cudaMemcpyDeviceToDevice, st));
     ++fwd;
     return MLCG_OK;
   };
   auto denoise = [&](int s) -> int {
-    int rc = network(steps[s].t);
+    int rc = network(a.steps[s].t);
     if (rc) return rc;
     mlcg_noise n = next_noise();
-    return mlcg_step(h, z, eps, &steps[s], &n, stream);
+    return mlcg_step(h, a.z, eps, &a.steps[s], &n, stream);
   };
   auto reinject = [&](int s) -> int {
     mlcg_noise n = next_noise();
-    return mlcg_reinject(h, z, z_known, fixed_mask, &steps[s], &n, stream);
+    return mlcg_reinject(h, a.z, a.z_known, a.fixed_mask, &a.steps[s], &n, stream);
   };
   int rc;
   // modes 2 and 3 start from the known molecule forward-diffused to diffusion_level
   const bool from_known = (mode == 2 || mode == 3);
-  if (from_known) {
-    mlcg_noise n = next_noise();
-    if ((rc = mlcg_forward_diffuse(h, z, z_known, merge_alpha, merge_sigma, &n, stream))) return rc;
-  } else {
-    mlcg_noise n = next_noise();
-    if ((rc = mlcg_noise_init(h, z, &n, stream))) return rc;
-  }
-  const int r_eff = (mode == 0) ? resample_steps : std::max(resample_steps, 1);
-  for (int s = T - 1; s >= 0; --s) {
-    if (from_known && s > diffusion_level) continue;
+  const mlcg_noise n0 = next_noise();
+  if ((rc = from_known ? mlcg_forward_diffuse(h, a.z, a.z_known, a.merge_alpha, a.merge_sigma, &n0, stream)
+                       : mlcg_noise_init(h, a.z, &n0, stream)))
+    return rc;
+  const int r_eff = (mode == 0) ? a.resample_steps : std::max(a.resample_steps, 1);
+  for (int s = a.T - 1; s >= 0; --s) {
+    if (from_known && s > a.diffusion_level) continue;
     if (mode == 0) {
       for (int r = 0; r <= r_eff; ++r)
         if ((rc = denoise(s))) return rc;
@@ -1201,7 +1207,7 @@ static int sample_loop(mlcg_handle* h, int mode, int T, const mlcg_step_scalars*
   }
   if ((rc = network(0.0f))) return rc;
   mlcg_noise n = next_noise();
-  return mlcg_decode(h, z, eps, sigma_0, alpha_0, sigma_x, &n, x_out, atom_class_out, stream);
+  return mlcg_decode(h, a.z, eps, a.sigma_0, a.alpha_0, a.sigma_x, &n, a.x_out, a.atom_class_out, stream);
 }
 
 extern "C" int mlcg_sample(mlcg_handle* h, int mode, int T, const mlcg_step_scalars* steps, int resample_steps,
@@ -1209,9 +1215,10 @@ extern "C" int mlcg_sample(mlcg_handle* h, int mode, int T, const mlcg_step_scal
                            float sigma_x, const float* ctx, const float* z_known, const float* fixed_mask,
                            const float* noise_tape, uint64_t seed, int64_t sample_offset, const int64_t* sample_ids, float* z,
                            float* x_out, int32_t* atom_class_out, float* trace_z, float* trace_eps, void* stream) {
-  return sample_loop(h, mode, T, steps, resample_steps, diffusion_level, merge_alpha, merge_sigma, sigma_0, alpha_0, sigma_x,
-                     ctx, z_known, fixed_mask, noise_tape, seed, sample_offset, sample_ids, z, x_out, atom_class_out, trace_z,
-                     trace_eps, 0, stream);
+  const LoopArgs a{mode, T, steps, resample_steps, diffusion_level, merge_alpha, merge_sigma, sigma_0, alpha_0, sigma_x, ctx,
+                   z_known, fixed_mask, noise_tape, seed, sample_offset, sample_ids, z, x_out, atom_class_out, trace_z,
+                   trace_eps, 0};
+  return sample_loop(h, a, stream);
 }
 
 // ---------------------------------------------------------------------------------------------------------------
@@ -1341,16 +1348,54 @@ static int seer_device(mlcg_handle* h, void* stream) {
                            h->g_bonds.as<int8_t>(), h->pl->B, stream);
 }
 
-// The device part of mlcg_generate: reverse loop + GCN inputs + GCN.  Pure kernel / async-copy sequence on `stream`
-// (no allocation, no synchronisation once the workspaces exist), hence capturable into a CUDA graph.
-static int generate_device(mlcg_handle* h, int T, const mlcg_step_scalars* steps, int resample_steps, float sigma_0,
-                           float alpha_0, float sigma_x, uint64_t seed, int64_t sample_offset, void* stream) {
-  int rc = mlcg_sample(h, 0, T, steps, resample_steps, 0, 0.f, 0.f, sigma_0, alpha_0, sigma_x, h->g_ctx.as<float>(), nullptr,
-                       nullptr, nullptr, seed, sample_offset, h->g_ids.as<int64_t>(), h->g_z.as<float>(), h->g_x.as<float>(),
-                       h->g_cls.as<int32_t>(), nullptr, nullptr, stream);
-  if (rc) return rc;
-  return seer_device(h, stream);
-}
+// ---------------------------------------------------------------------------------------------------------------
+// host generation calls: mlcg_generate, mlcg_generate_fragment(_jobs), mlcg_generate_analogue_jobs
+// ---------------------------------------------------------------------------------------------------------------
+// The inputs and outputs every host generation call takes (mlcg.h); n_nodes, ctx, steps and ids are HOST arrays.
+struct GenCall {
+  const int32_t* n_nodes;
+  int B, N;
+  const float* ctx;
+  int T;
+  const mlcg_step_scalars* steps;
+  int resample_steps;
+  float sigma_0, alpha_0, sigma_x;
+  uint64_t seed;
+  int64_t sample_offset;
+  const int64_t* ids;  // NULL: sample_offset + b
+  float* x_out;        // x_out, cls_out, bonds_out: pinned host or device
+  int32_t* cls_out;
+  int8_t* bonds_out;
+  void* stream;
+};
+
+// A job table: sections appended to one host blob, each padded to a multiple of 4 bytes so that every pointer into the
+// device copy is aligned, and uploaded with one copy.
+enum { TAB_JOBS, TAB_JOB_OF_SAMPLE, TAB_X, TAB_H, TAB_FIXED, TAB_SECTIONS };
+struct JobTable {
+  std::vector<unsigned char> blob;
+  size_t off[TAB_SECTIONS] = {};
+  void add(int sec, const void* src, size_t bytes) {
+    off[sec] = blob.size();
+    blob.resize(off[sec] + ((bytes + 3) & ~(size_t)3));
+    if (bytes) memcpy(blob.data() + off[sec], src, bytes);
+  }
+  template <class P>
+  P* at(const DevBuf& d, int sec) const { return reinterpret_cast<P*>(d.as<unsigned char>() + off[sec]); }
+};
+
+// The part of a host generation call that depends on its kind.
+enum GenKind { GEN_PLAIN = 1, GEN_INPAINT, GEN_IFM, GEN_ANALOGUE_FIXED, GEN_ANALOGUE_FREE };
+struct GenParams {
+  int kind = GEN_PLAIN;
+  int loop_mode = 0;                   // mlcg_sample mode of the last reverse loop
+  int level = 0;                       // modes 2 / 3: the diffusion level the loop starts from ...
+  float alpha_L = 0.f, sigma_L = 0.f;  // ... and the forward diffusion to it
+  IfmNorms nrm{};                      // IFM: context normalisation
+  const JobTable* tab = nullptr;       // uploaded on every call (NULL: no table)
+  const int32_t* n_gen = nullptr;      // fragment kinds: (B) atoms still to be generated per sample (n_nodes - n_ff) ...
+  int Ng = 0;                          // ... IFM: padded to Ng in batch plan 1
+};
 
 static inline long long fbits(float f) {
   int32_t i;
@@ -1358,34 +1403,143 @@ static inline long long fbits(float f) {
   return (long long)i;
 }
 
-// Host side shared by mlcg_generate and mlcg_generate_fragment.  `key` holds everything the device sequence bakes into
-// kernel arguments.  A new key rebuilds the batch plan (mlcg_set_batch: plan 0 = n_nodes_host / N, plus plan 1 =
-// plan1_n_nodes / plan1_N when given) and drops the captured graph.  Every call uploads the per-call inputs -- context,
-// sample ids, {seed, sample_offset}, and whatever `upload(stream)` adds -- to handle-owned device buffers, then runs
-// `device(stream)`: eagerly on the first call with a key, captured into a CUDA graph on the second, replayed from then on.
-// The outputs are copied to x_out / atom_class_out / bonds_out (pinned host or device) and the stream is synchronised.
-template <class Upload, class Device>
-static int generate_graphed(mlcg_handle* h, const std::vector<long long>& key, const int32_t* n_nodes_host, int B, int N,
-                            const int32_t* plan1_n_nodes, int plan1_N, const float* ctx_host, uint64_t seed,
-                            int64_t sample_offset, const int64_t* sample_ids_host, float* x_out, int32_t* atom_class_out,
-                            int8_t* bonds_out, void* stream, Upload upload, Device device) {
-  CK(cudaSetDevice(h->device));  // the call may come from any host thread (pipeline.GenerationPipeline's feeder)
+// The key of the CUDA graph of a host generation call.  The device sequences read scalars only from the GenCall and the
+// GenParams, and every one of those that is baked into a kernel argument, or sizes a buffer or a batch plan, is here;
+// so two calls with equal keys launch the same sequence with the same arguments, and the graph captured for one replays
+// the other.  What is not in the key -- the context, the sample ids, {seed, sample_offset} and the job table's contents
+// -- is uploaded to handle-owned buffers on every call.  The kind tag keeps calls of different kinds apart.
+static std::vector<long long> graph_key(const mlcg_handle* h, const GenCall& c, const GenParams& p) {
+  std::vector<long long> k{p.kind, c.B, c.N, c.T, c.resample_steps, h->precision, fbits(c.sigma_0), fbits(c.alpha_0),
+                           fbits(c.sigma_x)};
+  k.reserve(k.size() + 3 * (size_t)std::max(c.B, 0) + 7 * (size_t)std::max(c.T, 0) + 32);
+  for (int b = 0; b < c.B; ++b) k.push_back(c.n_nodes[b]);
+  for (int s = 0; s < c.T; ++s) {
+    const mlcg_step_scalars& q = c.steps[s];
+    for (float v : {q.t, q.alpha_ts, q.c_eps, q.c_sigma, q.alpha_s, q.sigma_s, q.blend}) k.push_back(fbits(v));
+  }
+  k.insert(k.end(), {p.loop_mode, p.level, fbits(p.alpha_L), fbits(p.sigma_L), p.Ng});
+  for (int i = 0; i < 3; ++i) { k.push_back(fbits(p.nrm.mean[i])); k.push_back(fbits(p.nrm.mad[i])); }
+  if (p.tab) {  // its size and offsets: the job count, the packed atom count and B
+    k.push_back((long long)p.tab->blob.size());
+    k.insert(k.end(), p.tab->off, p.tab->off + TAB_SECTIONS);
+  }
+  if (p.n_gen) k.insert(k.end(), p.n_gen, p.n_gen + c.B);
+  return k;
+}
+
+// The checks every host generation call starts with.  `unloaded` is returned without both weight sets.
+static int check_gen_call(mlcg_handle* h, const char* what, int unloaded, const GenCall& c) {
+  if (!h) return MLCG_E_ARG;
+  if (!h->egnn_loaded || !h->seer_loaded) FAIL(unloaded, std::string(what) + ": load both weight sets first");
+  if (!c.n_nodes || !c.ctx || !c.steps || !c.x_out || !c.cls_out || !c.bonds_out)
+    FAIL(MLCG_E_ARG, std::string(what) + ": null pointer");
+  return MLCG_OK;
+}
+
+// The reverse loop of a host generation call: its schedule, decode scalars and noise keys, the device sample ids, z
+// workspace and context, the kind's loop mode and level, z_known / fixed_mask when it has a job table, and the outputs
+// the GCN reads.  Call sites change what differs.
+static LoopArgs gen_loop(mlcg_handle* h, const GenCall& c, const GenParams& p) {
+  return LoopArgs{p.loop_mode, c.T, c.steps, c.resample_steps, p.level, p.alpha_L, p.sigma_L, c.sigma_0, c.alpha_0,
+                  c.sigma_x, h->g_ctx.as<float>(), p.tab ? h->f_zk.as<float>() : nullptr,
+                  p.tab ? h->f_fm.as<float>() : nullptr, nullptr, c.seed, c.sample_offset, h->g_ids.as<int64_t>(),
+                  h->g_z.as<float>(), h->g_x.as<float>(), h->g_cls.as<int32_t>()};
+}
+
+// The device sequences up to the molecules in g_x / g_cls: pure kernel / async-copy sequences on `stream` (no
+// allocation, no synchronisation once the workspaces exist), hence capturable into a CUDA graph.
+typedef int (*GenDevice)(mlcg_handle* h, const GenCall& c, const GenParams& p, void* stream);
+
+// mlcg_generate: the reverse loop from noise.
+static int generate_plain_device(mlcg_handle* h, const GenCall& c, const GenParams& p, void* stream) {
+  return sample_loop(h, gen_loop(h, c, p), stream);
+}
+
+// Draw numbering of the merge loop of inertial fragment matching.  It starts at 0 like the first loop's, so both loops
+// draw the same normals per (sample, atom, draw) -- exactly what the eager composition
+// (MLConformerGenerator.edm_sample_tensors: two mlcg_sample calls) does, which this path reproduces bit for bit.
+static const uint64_t kMergeDrawBase = 0;
+
+// mlcg_generate_fragment_jobs (see mlcg.h): the launch sequence of the eager composition, on plan 0 (whole molecules)
+// and -- IFM -- plan 1 (the atoms still to be generated, stride Ng).  The plan switches happen on the host between
+// launches; each launch bakes in the pointers of its plan, so one captured graph holds both loops.
+static int generate_fragment_device(mlcg_handle* h, const GenCall& c, const GenParams& p, void* stream) {
   cudaStream_t st = (cudaStream_t)stream;
+  const int B = c.B, N = c.N;
+  const JobTable& t = *p.tab;
+  const float* ffx = t.at<float>(h->j_tab, TAB_X);
+  const float* ffh = t.at<float>(h->j_tab, TAB_H);
+  const int* job = t.at<int>(h->j_tab, TAB_JOB_OF_SAMPLE);
+  const FragJob* jobs = t.at<FragJob>(h->j_tab, TAB_JOBS);
+  float* zk = h->f_zk.as<float>();
+  float* fm = h->f_fm.as<float>();
+  LoopArgs a = gen_loop(h, c, p);
+  if (p.kind == GEN_INPAINT) {
+    // z_known / fixed_mask of EquivariantDiffusion.inpaint (prepare_fragment): the merge-input kernel with no generated atoms
+    k_ifm_merge_inputs<<<B, 64, 0, st>>>(nullptr, nullptr, nullptr, nullptr, ffx, ffh, job, jobs, 0, N, zk, fm);
+    KCHECK();
+    return sample_loop(h, a, stream);
+  }
+  // inertial fragment matching: per-sample context of the atoms still to be generated ...
+  k_ifm_context<<<(B + 127) / 128, 128, 0, st>>>(h->plans[0].d_n_nodes.as<int>(), job, jobs, B, p.nrm, h->f_ctx.as<float>(),
+                                                 h->f_shift.as<float>(), h->f_rot.as<float>(), h->f_ngen.as<int>());
+  KCHECK();
+  // ... generated on their own (plan 1) ...
+  LoopArgs gen = gen_loop(h, c, p);
+  gen.mode = 0;
+  gen.ctx = h->f_ctx.as<float>();
+  gen.x_out = h->f_xg.as<float>();
+  gen.atom_class_out = h->f_clsg.as<int32_t>();
+  h->pl = &h->plans[1];
+  const int rc = sample_loop(h, gen, stream);
+  h->pl = &h->plans[0];
+  if (rc) return rc;
+  // ... moved back to the reference frame next to the fixed fragment, and merged with it (plan 0)
+  k_ifm_merge_inputs<<<B, 64, 0, st>>>(h->f_xg.as<float>(), h->f_clsg.as<int32_t>(), h->f_shift.as<float>(), h->f_rot.as<float>(),
+                                       ffx, ffh, job, jobs, p.Ng, N, zk, fm);
+  KCHECK();
+  a.draw0 = kMergeDrawBase;
+  return sample_loop(h, a, stream);
+}
+
+static void launch_analogue_inputs(const JobTable& t, const DevBuf& d, int B, int N, float* z_known, float* fixed_mask,
+                                   cudaStream_t st) {
+  k_analogue_inputs<<<warp_grid(B), 128, 0, st>>>(t.at<float>(d, TAB_X), t.at<float>(d, TAB_H), t.at<int>(d, TAB_FIXED),
+                                                  t.at<int>(d, TAB_JOB_OF_SAMPLE), t.at<AnalogueJob>(d, TAB_JOBS), B, N,
+                                                  z_known, fixed_mask);
+}
+
+// mlcg_generate_analogue_jobs: the parents' z_known / fixed_mask, then the loop from diffusion level L with draws numbered
+// from 0, as mlcg_sample numbers them, so the graphed call equals the eager composition.
+static int generate_analogue_device(mlcg_handle* h, const GenCall& c, const GenParams& p, void* stream) {
+  launch_analogue_inputs(*p.tab, h->j_tab, c.B, c.N, h->f_zk.as<float>(), h->f_fm.as<float>(), (cudaStream_t)stream);
+  KCHECK();
+  return sample_loop(h, gen_loop(h, c, p), stream);
+}
+
+// Host side of every host generation call.  A new key (graph_key) rebuilds the batch plan (mlcg_set_batch: plan 0 =
+// n_nodes / N, plus plan 1 = p.n_gen / p.Ng for IFM) and drops the captured graph.  Every call uploads the per-call
+// inputs -- context, sample ids, {seed, sample_offset} and the job table -- to handle-owned device buffers, then runs
+// `device` and the GCN: eagerly on the first call with a key, captured into a CUDA graph on the second, replayed from
+// then on.  The outputs are copied to c.x_out / c.cls_out / c.bonds_out and the stream is synchronised.
+static int generate_graphed(mlcg_handle* h, const GenCall& c, const GenParams& p, GenDevice device) {
+  CK(cudaSetDevice(h->device));  // the call may come from any host thread (pipeline.GenerationPipeline's feeder)
+  const int B = c.B, N = c.N;
+  cudaStream_t st = (cudaStream_t)c.stream;
   if (st == nullptr) {
     // the legacy NULL stream cannot be captured; the call is synchronous and takes host buffers, so run it on a
     // private stream
     if (h->own_stream == nullptr) CK(cudaStreamCreateWithFlags(&h->own_stream, cudaStreamNonBlocking));
     CK(cudaDeviceSynchronize());
     st = h->own_stream;
-    stream = (void*)st;
   }
-  const bool same = (key == h->gen_key);
-  if (!same) {
-    int rc = mlcg_set_batch(h, n_nodes_host, B, N);  // also drops any previously captured graph
+  std::vector<long long> key = graph_key(h, c, p);
+  if (key != h->gen_key) {
+    int rc = mlcg_set_batch(h, c.n_nodes, B, N);  // also drops any previously captured graph
     if (rc) return rc;
     // set_batch drained the device: plan 1 may be rewritten too (outside any capture)
-    if (plan1_n_nodes && (rc = build_plan(h, h->plans[1], plan1_n_nodes, B, plan1_N))) return rc;
-    h->gen_key = key;
+    if (p.kind == GEN_IFM && (rc = build_plan(h, h->plans[1], p.n_gen, B, p.Ng))) return rc;
+    h->gen_key = std::move(key);
   }
   h->gen_key_hits++;
   const size_t bn = (size_t)B * N, dd = (size_t)B * SEER_D * SEER_D;
@@ -1401,26 +1555,43 @@ static int generate_graphed(mlcg_handle* h, const std::vector<long long>& key, c
   CK(h->g_ids.ensure((size_t)B * sizeof(int64_t)));
   // global sample ids (the RNG key): always read from this device buffer, so a captured graph replays with any ids
   h->ids_stage.resize((size_t)B);
-  for (int b = 0; b < B; ++b) h->ids_stage[b] = sample_ids_host ? sample_ids_host[b] : sample_offset + b;
+  for (int b = 0; b < B; ++b) h->ids_stage[b] = c.ids ? c.ids[b] : c.sample_offset + b;
   static int graphs_enabled = -1;
   if (graphs_enabled < 0) {
     const char* e = getenv("MLCG_GRAPH");
     graphs_enabled = (e == nullptr) ? 1 : (atoi(e) != 0);
   }
-  CK(cudaMemcpyAsync(h->g_ctx.p, ctx_host, (size_t)B * 3 * 4, cudaMemcpyHostToDevice, st));
+  CK(cudaMemcpyAsync(h->g_ctx.p, c.ctx, (size_t)B * 3 * 4, cudaMemcpyHostToDevice, st));
   CK(cudaMemcpyAsync(h->g_ids.p, h->ids_stage.data(), (size_t)B * sizeof(int64_t), cudaMemcpyHostToDevice, st));
-  const unsigned long long ctl[2] = {(unsigned long long)seed, (unsigned long long)sample_offset};
+  const unsigned long long ctl[2] = {(unsigned long long)c.seed, (unsigned long long)c.sample_offset};
   CK(cudaMemcpyAsync(h->noise_ctl.p, ctl, sizeof(ctl), cudaMemcpyHostToDevice, st));
-  int rc = upload(st);
-  if (rc) return rc;
+  if (p.tab) {  // the job table and the z_known / fixed_mask it expands to
+    CK(h->j_tab.ensure(p.tab->blob.size()));
+    CK(h->f_zk.ensure(bn * ZC * 4));
+    CK(h->f_fm.ensure(bn * 4));
+    if (p.kind == GEN_IFM) {  // the first loop's context, frame and outputs
+      CK(h->f_ctx.ensure((size_t)B * 3 * 4));
+      CK(h->f_shift.ensure((size_t)B * 3 * 4));
+      CK(h->f_rot.ensure((size_t)B * 9 * 4));
+      CK(h->f_ngen.ensure((size_t)B * 4));
+      CK(h->f_xg.ensure((size_t)B * p.Ng * 3 * 4));
+      CK(h->f_clsg.ensure((size_t)B * p.Ng * 4));
+    }
+    CK(cudaMemcpyAsync(h->j_tab.p, p.tab->blob.data(), p.tab->blob.size(), cudaMemcpyHostToDevice, st));
+  }
   h->use_noise_ctl = true;  // the noise kernels read {seed, sample_offset} from device memory (graph-replayable)
+  auto run = [&]() {  // the kind's sequence, then the GCN
+    int rc = device(h, c, p, st);
+    return rc ? rc : seer_device(h, st);
+  };
+  int rc = MLCG_OK;
   if (graphs_enabled && h->gen_graph == nullptr && h->gen_key_hits >= 2) {
     // second call with this key: all workspaces exist and every kernel attribute has been set by the eager first call,
     // so the launch sequence can be captured
     cudaGraph_t graph = nullptr;
     const long long launches0 = h->launches;
     CK(cudaStreamBeginCapture(st, cudaStreamCaptureModeThreadLocal));
-    rc = device(stream);
+    rc = run();
     cudaError_t ce = cudaStreamEndCapture(st, &graph);
     if (rc == MLCG_OK && ce == cudaSuccess && graph != nullptr) {
       ce = cudaGraphInstantiate(&h->gen_graph, graph, 0);
@@ -1441,14 +1612,14 @@ static int generate_graphed(mlcg_handle* h, const std::vector<long long>& key, c
     CK(cudaGraphLaunch(h->gen_graph, st));
     h->launches += h->gen_graph_launches;
   } else {
-    rc = device(stream);
+    rc = run();
   }
   h->use_noise_ctl = false;
   if (rc) return rc;
   // the outputs may be pinned host buffers or device buffers (multi-GPU driver: results stay on the device for the gather)
-  CK(cudaMemcpyAsync(x_out, h->g_x.p, bn * 3 * 4, cudaMemcpyDefault, st));
-  CK(cudaMemcpyAsync(atom_class_out, h->g_cls.p, bn * 4, cudaMemcpyDefault, st));
-  CK(cudaMemcpyAsync(bonds_out, h->g_bonds.p, dd, cudaMemcpyDefault, st));
+  CK(cudaMemcpyAsync(c.x_out, h->g_x.p, bn * 3 * 4, cudaMemcpyDefault, st));
+  CK(cudaMemcpyAsync(c.cls_out, h->g_cls.p, bn * 4, cudaMemcpyDefault, st));
+  CK(cudaMemcpyAsync(c.bonds_out, h->g_bonds.p, dd, cudaMemcpyDefault, st));
   CK(cudaStreamSynchronize(st));
   return MLCG_OK;
 }
@@ -1457,76 +1628,10 @@ extern "C" int mlcg_generate(mlcg_handle* h, const int32_t* n_nodes_host, int B,
                              const mlcg_step_scalars* steps, int resample_steps, float sigma_0, float alpha_0, float sigma_x,
                              uint64_t seed, int64_t sample_offset, const int64_t* sample_ids_host, float* x_host,
                              int32_t* atom_class_host, int8_t* bonds_host, void* stream) {
-  if (!h) return MLCG_E_ARG;
-  if (!h->egnn_loaded || !h->seer_loaded) FAIL(MLCG_E_STATE, "generate: load both weight sets first");
-  if (!n_nodes_host || !ctx_host || !steps || !x_host || !atom_class_host || !bonds_host) FAIL(MLCG_E_ARG, "generate: null pointer");
-  // Key of the captured graph: batch geometry, schedule and every scalar baked into kernel arguments.
-  std::vector<long long> key;
-  key.reserve((size_t)B + 8 * (size_t)T + 16);
-  key.push_back(B); key.push_back(N); key.push_back(T); key.push_back(resample_steps); key.push_back(h->precision);
-  key.push_back(fbits(sigma_0)); key.push_back(fbits(alpha_0)); key.push_back(fbits(sigma_x));
-  for (int b = 0; b < B; ++b) key.push_back(n_nodes_host[b]);
-  for (int s = 0; s < T; ++s) {
-    key.push_back(fbits(steps[s].t)); key.push_back(fbits(steps[s].alpha_ts)); key.push_back(fbits(steps[s].c_eps));
-    key.push_back(fbits(steps[s].c_sigma));
-  }
-  return generate_graphed(
-      h, key, n_nodes_host, B, N, nullptr, 0, ctx_host, seed, sample_offset, sample_ids_host, x_host, atom_class_host,
-      bonds_host, stream, [](cudaStream_t) { return (int)MLCG_OK; },
-      [&](void* s) { return generate_device(h, T, steps, resample_steps, sigma_0, alpha_0, sigma_x, seed, sample_offset, s); });
-}
-
-// Draw numbering of the merge loop of inertial fragment matching.  It starts at 0 like the first loop's, so both loops
-// draw the same normals per (sample, atom, draw) -- exactly what the eager composition
-// (MLConformerGenerator.edm_sample_tensors: two mlcg_sample calls) does, which this path reproduces bit for bit.
-static const uint64_t kMergeDrawBase = 0;
-
-// The device part of mlcg_generate_fragment_jobs (see mlcg.h): the launch sequence of the eager composition, on plan 0
-// (whole molecules) and -- mode 2 -- plan 1 (the atoms still to be generated, stride Ng).  The plan switches happen on the
-// host between launches; each launch bakes in the pointers of its plan, so one captured graph holds both loops.
-static int generate_fragment_device(mlcg_handle* h, int mode, int Ng, const IfmNorms& nrm, int T,
-                                    const mlcg_step_scalars* steps, int resample_steps, int diffusion_level, float merge_alpha,
-                                    float merge_sigma, float sigma_0, float alpha_0, float sigma_x, uint64_t seed,
-                                    int64_t sample_offset, void* stream) {
-  cudaStream_t st = (cudaStream_t)stream;
-  const int B = h->plans[0].B, N = h->plans[0].N;
-  const int64_t* ids = h->g_ids.as<int64_t>();
-  const int* job = h->f_job.as<int>();
-  const FragJob* jobs = h->f_jobs.as<FragJob>();
-  float* zk = h->f_zk.as<float>();
-  float* fm = h->f_fm.as<float>();
-  int rc;
-  if (mode == 1) {
-    // z_known / fixed_mask of EquivariantDiffusion.inpaint (prepare_fragment): the merge-input kernel with no generated atoms
-    k_ifm_merge_inputs<<<B, 64, 0, st>>>(nullptr, nullptr, nullptr, nullptr, h->f_ffx.as<float>(), h->f_ffh.as<float>(), job,
-                                         jobs, 0, N, zk, fm);
-    KCHECK();
-    rc = sample_loop(h, 1, T, steps, resample_steps, diffusion_level, 0.f, 0.f, sigma_0, alpha_0, sigma_x, h->g_ctx.as<float>(),
-                     zk, fm, nullptr, seed, sample_offset, ids, h->g_z.as<float>(), h->g_x.as<float>(), h->g_cls.as<int32_t>(),
-                     nullptr, nullptr, 0, stream);
-    if (rc) return rc;
-    return seer_device(h, stream);
-  }
-  // inertial fragment matching: per-sample context of the atoms still to be generated ...
-  k_ifm_context<<<(B + 127) / 128, 128, 0, st>>>(h->plans[0].d_n_nodes.as<int>(), job, jobs, B, nrm, h->f_ctx.as<float>(),
-                                                 h->f_shift.as<float>(), h->f_rot.as<float>(), h->f_ngen.as<int>());
-  KCHECK();
-  // ... generated on their own (plan 1) ...
-  h->pl = &h->plans[1];
-  rc = sample_loop(h, 0, T, steps, resample_steps, diffusion_level, 0.f, 0.f, sigma_0, alpha_0, sigma_x, h->f_ctx.as<float>(),
-                   nullptr, nullptr, nullptr, seed, sample_offset, ids, h->g_z.as<float>(), h->f_xg.as<float>(),
-                   h->f_clsg.as<int32_t>(), nullptr, nullptr, 0, stream);
-  h->pl = &h->plans[0];
-  if (rc) return rc;
-  // ... moved back to the reference frame next to the fixed fragment, and merged with it (plan 0)
-  k_ifm_merge_inputs<<<B, 64, 0, st>>>(h->f_xg.as<float>(), h->f_clsg.as<int32_t>(), h->f_shift.as<float>(), h->f_rot.as<float>(),
-                                       h->f_ffx.as<float>(), h->f_ffh.as<float>(), job, jobs, Ng, N, zk, fm);
-  KCHECK();
-  rc = sample_loop(h, 2, T, steps, resample_steps, diffusion_level, merge_alpha, merge_sigma, sigma_0, alpha_0, sigma_x,
-                   h->g_ctx.as<float>(), zk, fm, nullptr, seed, sample_offset, ids, h->g_z.as<float>(), h->g_x.as<float>(),
-                   h->g_cls.as<int32_t>(), nullptr, nullptr, kMergeDrawBase, stream);
-  if (rc) return rc;
-  return seer_device(h, stream);
+  const GenCall c{n_nodes_host, B, N, ctx_host, T, steps, resample_steps, sigma_0, alpha_0, sigma_x, seed, sample_offset,
+                  sample_ids_host, x_host, atom_class_host, bonds_host, stream};
+  if (const int rc = check_gen_call(h, "generate", MLCG_E_STATE, c)) return rc;
+  return generate_graphed(h, c, GenParams{}, generate_plain_device);
 }
 
 extern "C" int mlcg_generate_fragment_jobs(mlcg_handle* h, const mlcg_fragment_jobs* fj, const int32_t* n_nodes_host, int B,
@@ -1534,10 +1639,10 @@ extern "C" int mlcg_generate_fragment_jobs(mlcg_handle* h, const mlcg_fragment_j
                                            int resample_steps, float sigma_0, float alpha_0, float sigma_x, uint64_t seed,
                                            int64_t sample_offset, const int64_t* sample_ids_host, float* x_out,
                                            int32_t* atom_class_out, int8_t* bonds_out, void* stream) {
-  if (!h) return MLCG_E_ARG;
-  if (!h->egnn_loaded || !h->seer_loaded) FAIL(MLCG_E_ARG, "generate_fragment: load both weight sets first");
-  if (!fj || !n_nodes_host || !ctx_host || !steps || !x_out || !atom_class_out || !bonds_out || !fj->job_of_sample_host ||
-      !fj->n_ff_host || !fj->ff_x_host || !fj->ff_h_host)
+  const GenCall c{n_nodes_host, B, N, ctx_host, T, steps, resample_steps, sigma_0, alpha_0, sigma_x, seed, sample_offset,
+                  sample_ids_host, x_out, atom_class_out, bonds_out, stream};
+  if (const int rc = check_gen_call(h, "generate_fragment", MLCG_E_ARG, c)) return rc;
+  if (!fj || !fj->job_of_sample_host || !fj->n_ff_host || !fj->ff_x_host || !fj->ff_h_host)
     FAIL(MLCG_E_ARG, "generate_fragment: null pointer");
   const int mode = fj->mode, n_jobs = fj->n_jobs;
   if (mode != 1 && mode != 2) FAIL(MLCG_E_ARG, "generate_fragment: mode must be 1 (inpaint) or 2 (inertial fragment matching)");
@@ -1561,76 +1666,36 @@ extern "C" int mlcg_generate_fragment_jobs(mlcg_handle* h, const mlcg_fragment_j
       memcpy(q.ffsum, fj->ff_weighted_com_host + (size_t)j * 3, sizeof(q.ffsum));
     }
   }
-  // per sample: its job's fragment size, which must leave at least one atom to generate
-  std::vector<int32_t> n_ff_of((size_t)B), n_gen;
+  // per sample: the atoms its job's fragment leaves to generate, at least one
+  std::vector<int32_t> n_gen((size_t)B);
   int min_n_ff = N;
   for (int b = 0; b < B; ++b) {
     const int j = fj->job_of_sample_host[b];
     if (j < 0 || j >= n_jobs) FAIL(MLCG_E_ARG, "generate_fragment: job index out of range (sample " + std::to_string(b) + ")");
-    n_ff_of[b] = jobs[j].n_ff;
-    if (n_ff_of[b] >= n_nodes_host[b])
+    n_gen[b] = n_nodes_host[b] - jobs[j].n_ff;
+    if (n_gen[b] <= 0)
       FAIL(MLCG_E_ARG, "generate_fragment: the fragment must have fewer atoms than every sample (sample " + std::to_string(b) + ")");
-    min_n_ff = std::min(min_n_ff, (int)n_ff_of[b]);
+    min_n_ff = std::min(min_n_ff, jobs[j].n_ff);
   }
-  // first IFM loop: the atoms still to be generated, padded to the longest of them
-  const int Ng = N - min_n_ff;
-  IfmNorms nrm{};
+  JobTable t;
+  t.add(TAB_JOBS, jobs.data(), (size_t)n_jobs * sizeof(FragJob));
+  t.add(TAB_JOB_OF_SAMPLE, fj->job_of_sample_host, (size_t)B * 4);
+  t.add(TAB_X, fj->ff_x_host, (size_t)n_ff_total * 3 * 4);
+  t.add(TAB_H, fj->ff_h_host, (size_t)n_ff_total * 8 * 4);
+  GenParams p;
+  p.kind = mode == 2 ? GEN_IFM : GEN_INPAINT;
+  p.loop_mode = mode;
+  p.tab = &t;
+  p.n_gen = n_gen.data();
   if (mode == 2) {
-    memcpy(nrm.mean, fj->norm_mean_host, sizeof(nrm.mean));
-    memcpy(nrm.mad, fj->norm_mad_host, sizeof(nrm.mad));
-    n_gen.resize(B);
-    for (int b = 0; b < B; ++b) n_gen[b] = n_nodes_host[b] - n_ff_of[b];
+    p.level = fj->diffusion_level;
+    p.alpha_L = fj->merge_alpha;
+    p.sigma_L = fj->merge_sigma;
+    memcpy(p.nrm.mean, fj->norm_mean_host, sizeof(p.nrm.mean));
+    memcpy(p.nrm.mad, fj->norm_mad_host, sizeof(p.nrm.mad));
+    p.Ng = N - min_n_ff;  // first loop: the atoms still to be generated, padded to the longest of them
   }
-  // Key of the captured graph: the geometry and every scalar baked into kernel arguments.  It starts with -mode, so it
-  // never equals a key of mlcg_generate (which starts with B).  The job count and the packed fragment length fix the sizes
-  // of the buffers the graph reads.  The fragments, the job table, the job of every sample, the context, the ids and
-  // {seed, sample_offset} are uploaded on every call, so a replay with other references or fragments of the same sizes
-  // reuses the graph and never sees a previous call's inputs.
-  std::vector<long long> key;
-  key.reserve(2 * (size_t)B + 7 * (size_t)T + 32);
-  key.push_back(-mode); key.push_back(B); key.push_back(N); key.push_back(T); key.push_back(resample_steps);
-  key.push_back(h->precision); key.push_back(n_jobs); key.push_back(n_ff_total);
-  key.push_back(fbits(sigma_0)); key.push_back(fbits(alpha_0)); key.push_back(fbits(sigma_x));
-  if (mode == 2) {
-    key.push_back(fj->diffusion_level); key.push_back(fbits(fj->merge_alpha)); key.push_back(fbits(fj->merge_sigma));
-    for (int c = 0; c < 3; ++c) { key.push_back(fbits(nrm.mean[c])); key.push_back(fbits(nrm.mad[c])); }
-  }
-  for (int b = 0; b < B; ++b) key.push_back(n_nodes_host[b]);
-  for (int b = 0; b < B; ++b) key.push_back(n_ff_of[b]);
-  for (int s = 0; s < T; ++s) {
-    const mlcg_step_scalars& c = steps[s];
-    for (float v : {c.t, c.alpha_ts, c.c_eps, c.c_sigma, c.alpha_s, c.sigma_s, c.blend}) key.push_back(fbits(v));
-  }
-  const size_t bn = (size_t)B * N, bg = (size_t)B * Ng;
-  auto upload = [&](cudaStream_t st) -> int {
-    CK(h->f_ffx.ensure((size_t)n_ff_total * 3 * 4));
-    CK(h->f_ffh.ensure((size_t)n_ff_total * 8 * 4));
-    CK(h->f_jobs.ensure((size_t)n_jobs * sizeof(FragJob)));
-    CK(h->f_job.ensure((size_t)B * 4));
-    CK(h->f_zk.ensure(bn * ZC * 4));
-    CK(h->f_fm.ensure(bn * 4));
-    if (mode == 2) {
-      CK(h->f_ctx.ensure((size_t)B * 3 * 4));
-      CK(h->f_shift.ensure((size_t)B * 3 * 4));
-      CK(h->f_rot.ensure((size_t)B * 9 * 4));
-      CK(h->f_ngen.ensure((size_t)B * 4));
-      CK(h->f_xg.ensure(bg * 3 * 4));
-      CK(h->f_clsg.ensure(bg * 4));
-    }
-    CK(cudaMemcpyAsync(h->f_ffx.p, fj->ff_x_host, (size_t)n_ff_total * 3 * 4, cudaMemcpyHostToDevice, st));
-    CK(cudaMemcpyAsync(h->f_ffh.p, fj->ff_h_host, (size_t)n_ff_total * 8 * 4, cudaMemcpyHostToDevice, st));
-    CK(cudaMemcpyAsync(h->f_jobs.p, jobs.data(), (size_t)n_jobs * sizeof(FragJob), cudaMemcpyHostToDevice, st));
-    CK(cudaMemcpyAsync(h->f_job.p, fj->job_of_sample_host, (size_t)B * 4, cudaMemcpyHostToDevice, st));
-    return MLCG_OK;
-  };
-  const int diffusion_level = mode == 2 ? fj->diffusion_level : 0;
-  const float merge_alpha = mode == 2 ? fj->merge_alpha : 0.f, merge_sigma = mode == 2 ? fj->merge_sigma : 0.f;
-  return generate_graphed(h, key, n_nodes_host, B, N, mode == 2 ? n_gen.data() : nullptr, Ng, ctx_host, seed, sample_offset,
-                          sample_ids_host, x_out, atom_class_out, bonds_out, stream, upload, [&](void* s) {
-                            return generate_fragment_device(h, mode, Ng, nrm, T, steps, resample_steps, diffusion_level,
-                                                            merge_alpha, merge_sigma, sigma_0, alpha_0, sigma_x, seed,
-                                                            sample_offset, s);
-                          });
+  return generate_graphed(h, c, p, generate_fragment_device);
 }
 
 // One fragment for every sample: the one-job case of mlcg_generate_fragment_jobs.
@@ -1642,39 +1707,18 @@ extern "C" int mlcg_generate_fragment(mlcg_handle* h, const mlcg_fragment* frag,
   if (!h) return MLCG_E_ARG;
   if (!frag) FAIL(MLCG_E_ARG, "generate_fragment: null pointer");
   std::vector<int32_t> job_of_sample((size_t)std::max(B, 1), 0);  // never empty: B <= 0 fails the B check
-  mlcg_fragment_jobs fj{};
-  fj.mode = frag->mode;
-  fj.n_jobs = 1;
-  fj.job_of_sample_host = job_of_sample.data();
-  fj.n_ff_host = &frag->n_ff;
-  fj.ff_x_host = frag->ff_x_host;
-  fj.ff_h_host = frag->ff_h_host;
-  fj.diffusion_level = frag->diffusion_level;
-  fj.merge_alpha = frag->merge_alpha;
-  fj.merge_sigma = frag->merge_sigma;
-  fj.moi_gen_origin_host = frag->moi_gen_origin_host;
-  fj.ff_weighted_com_host = frag->ff_weighted_com_host;
-  fj.norm_mean_host = frag->norm_mean_host;
-  fj.norm_mad_host = frag->norm_mad_host;
+  const mlcg_fragment_jobs fj{frag->mode, 1, job_of_sample.data(), &frag->n_ff, frag->ff_x_host, frag->ff_h_host,
+                              frag->diffusion_level, frag->merge_alpha, frag->merge_sigma, frag->moi_gen_origin_host,
+                              frag->ff_weighted_com_host, frag->norm_mean_host, frag->norm_mad_host};
   return mlcg_generate_fragment_jobs(h, &fj, n_nodes_host, B, N, ctx_host, T, steps, resample_steps, sigma_0, alpha_0,
                                      sigma_x, seed, sample_offset, sample_ids_host, x_out, atom_class_out, bonds_out, stream);
 }
 
-// The parent table of an analogue call, validated and packed into one host blob (one upload): the job table, the job of
-// every sample, then the parents' coordinates, one-hots and fixed flags back to back.  Every section is a multiple of 4
-// bytes, so every pointer into the device copy is aligned.
-struct AnalogueTable {
-  std::vector<unsigned char> blob;
-  size_t off_jobs = 0, off_job = 0, off_x = 0, off_h = 0, off_fix = 0;
-  int n_atoms_total = 0;
-  bool any_fixed = false;
-  template <class P>
-  P* at(const DevBuf& d, size_t off) const { return reinterpret_cast<P*>(d.as<unsigned char>() + off); }
-};
-
-// n_nodes_host may be null (the eager hook: no per-sample atom counts to check).
+// The parent table of an analogue call, validated and packed: the job table, the job of every sample, then the parents'
+// coordinates, one-hots and fixed flags back to back.  n_nodes_host may be null (the eager hook: no per-sample atom
+// counts to check).
 static int analogue_table(mlcg_handle* h, const char* what, const mlcg_analogue_jobs* aj, const int32_t* n_nodes_host, int B,
-                          int N, AnalogueTable& t) {
+                          int N, JobTable& t, bool& any_fixed) {
   const std::string w(what);
   if (!aj || !aj->job_of_sample_host || !aj->n_atoms_host || !aj->coords_host || !aj->one_hot_host || !aj->fixed_host)
     FAIL(MLCG_E_ARG, w + ": null pointer");
@@ -1701,36 +1745,22 @@ static int analogue_table(mlcg_handle* h, const char* what, const mlcg_analogue_
     if (n_nodes_host && n_nodes_host[b] != jobs[j].n_atoms)
       FAIL(MLCG_E_ARG, w + ": n_nodes must equal the parent's atom count (sample " + std::to_string(b) + ")");
   }
-  t.n_atoms_total = total;
-  t.any_fixed = with_fixed > 0;
-  t.off_jobs = 0;
-  t.off_job = t.off_jobs + (size_t)n_jobs * sizeof(AnalogueJob);
-  t.off_x = t.off_job + (size_t)B * 4;
-  t.off_h = t.off_x + (size_t)total * 3 * 4;
-  t.off_fix = t.off_h + (size_t)total * 8 * 4;
-  t.blob.resize(t.off_fix + (size_t)total * 4);
-  unsigned char* p = t.blob.data();
-  memcpy(p + t.off_jobs, jobs.data(), (size_t)n_jobs * sizeof(AnalogueJob));
-  memcpy(p + t.off_job, aj->job_of_sample_host, (size_t)B * 4);
-  memcpy(p + t.off_x, aj->coords_host, (size_t)total * 3 * 4);
-  memcpy(p + t.off_h, aj->one_hot_host, (size_t)total * 8 * 4);
-  memcpy(p + t.off_fix, aj->fixed_host, (size_t)total * 4);
+  any_fixed = with_fixed > 0;
+  t.add(TAB_JOBS, jobs.data(), (size_t)n_jobs * sizeof(AnalogueJob));
+  t.add(TAB_JOB_OF_SAMPLE, aj->job_of_sample_host, (size_t)B * 4);
+  t.add(TAB_X, aj->coords_host, (size_t)total * 3 * 4);
+  t.add(TAB_H, aj->one_hot_host, (size_t)total * 8 * 4);
+  t.add(TAB_FIXED, aj->fixed_host, (size_t)total * 4);
   return MLCG_OK;
-}
-
-static void launch_analogue_inputs(const AnalogueTable& t, const DevBuf& d, int B, int N, float* z_known, float* fixed_mask,
-                                   cudaStream_t st) {
-  k_analogue_inputs<<<warp_grid(B), 128, 0, st>>>(t.at<float>(d, t.off_x), t.at<float>(d, t.off_h), t.at<int>(d, t.off_fix),
-                                                  t.at<int>(d, t.off_job), t.at<AnalogueJob>(d, t.off_jobs), B, N, z_known,
-                                                  fixed_mask);
 }
 
 extern "C" int mlcg_analogue_inputs(mlcg_handle* h, const mlcg_analogue_jobs* aj, int B, int N, float* z_known,
                                     float* fixed_mask, void* stream) {
   if (!h) return MLCG_E_ARG;
   if (!z_known || !fixed_mask) FAIL(MLCG_E_ARG, "analogue_inputs: null pointer");
-  AnalogueTable t;
-  int rc = analogue_table(h, "analogue_inputs", aj, nullptr, B, N, t);
+  JobTable t;
+  bool any_fixed;
+  int rc = analogue_table(h, "analogue_inputs", aj, nullptr, B, N, t, any_fixed);
   if (rc) return rc;
   cudaStream_t st = (cudaStream_t)stream;
   CK(h->hook_parents.ensure(t.blob.size()));
@@ -1740,61 +1770,30 @@ extern "C" int mlcg_analogue_inputs(mlcg_handle* h, const mlcg_analogue_jobs* aj
   return MLCG_OK;
 }
 
-// Draw numbering of the analogue loop: from 0, as mlcg_sample numbers it, so the graphed call equals the eager composition.
 extern "C" int mlcg_generate_analogue_jobs(mlcg_handle* h, const mlcg_analogue_jobs* aj, const int32_t* n_nodes_host, int B,
                                            int N, const float* ctx_host, int T, const mlcg_step_scalars* steps,
                                            int resample_steps, float sigma_0, float alpha_0, float sigma_x, uint64_t seed,
                                            int64_t sample_offset, const int64_t* sample_ids_host, float* x_out,
                                            int32_t* atom_class_out, int8_t* bonds_out, void* stream) {
-  if (!h) return MLCG_E_ARG;
-  if (!h->egnn_loaded || !h->seer_loaded) FAIL(MLCG_E_ARG, "generate_analogue: load both weight sets first");
-  if (!n_nodes_host || !ctx_host || !steps || !x_out || !atom_class_out || !bonds_out)
-    FAIL(MLCG_E_ARG, "generate_analogue: null pointer");
-  if (T <= 0 || resample_steps < 0) FAIL(MLCG_E_ARG, "generate_analogue: need T > 0 and resample_steps >= 0");
-  AnalogueTable t;
-  int rc = analogue_table(h, "generate_analogue", aj, n_nodes_host, B, N, t);
+  const GenCall c{n_nodes_host, B, N, ctx_host, T, steps, resample_steps, sigma_0, alpha_0, sigma_x, seed, sample_offset,
+                  sample_ids_host, x_out, atom_class_out, bonds_out, stream};
+  int rc = check_gen_call(h, "generate_analogue", MLCG_E_ARG, c);
   if (rc) return rc;
+  if (T <= 0 || resample_steps < 0) FAIL(MLCG_E_ARG, "generate_analogue: need T > 0 and resample_steps >= 0");
+  JobTable t;
+  bool any_fixed;
+  if ((rc = analogue_table(h, "generate_analogue", aj, n_nodes_host, B, N, t, any_fixed))) return rc;
   const int L = aj->diffusion_level;
   if (L < 1 || L > T) FAIL(MLCG_E_ARG, "generate_analogue: diffusion_level must lie in [1, T]");
+  GenParams p;
   // mode 2 (merge_fragments) re-injects the fixed atoms; mode 3 is the same loop with nothing to re-inject
-  const int mode = t.any_fixed ? 2 : 3;
-  // Key of the captured graph: the geometry and every scalar baked into kernel arguments.  It starts with -(10 + mode),
-  // so it never equals a key of mlcg_generate (B first) or mlcg_generate_fragment_jobs (-1 / -2).  The job count and the
-  // packed parent length fix the layout of the uploaded table; the parents, flags, context, ids and seed are uploaded on
-  // every call, so new parents of the same sizes replay the graph.
-  std::vector<long long> key;
-  key.reserve((size_t)B + 7 * (size_t)T + 32);
-  key.push_back(-(10 + mode)); key.push_back(B); key.push_back(N); key.push_back(T); key.push_back(resample_steps);
-  key.push_back(h->precision); key.push_back(aj->n_jobs); key.push_back(t.n_atoms_total);
-  key.push_back(fbits(sigma_0)); key.push_back(fbits(alpha_0)); key.push_back(fbits(sigma_x));
-  key.push_back(L); key.push_back(fbits(aj->merge_alpha)); key.push_back(fbits(aj->merge_sigma));
-  for (int b = 0; b < B; ++b) key.push_back(n_nodes_host[b]);
-  for (int s = 0; s < T; ++s) {
-    const mlcg_step_scalars& c = steps[s];
-    for (float v : {c.t, c.alpha_ts, c.c_eps, c.c_sigma, c.alpha_s, c.sigma_s, c.blend}) key.push_back(fbits(v));
-  }
-  const size_t bn = (size_t)B * N;
-  auto upload = [&](cudaStream_t st) -> int {
-    CK(h->a_tab.ensure(t.blob.size()));
-    CK(h->f_zk.ensure(bn * ZC * 4));
-    CK(h->f_fm.ensure(bn * 4));
-    CK(cudaMemcpyAsync(h->a_tab.p, t.blob.data(), t.blob.size(), cudaMemcpyHostToDevice, st));
-    return MLCG_OK;
-  };
-  auto device = [&](void* s) -> int {
-    cudaStream_t st = (cudaStream_t)s;
-    float* zk = h->f_zk.as<float>();
-    float* fm = h->f_fm.as<float>();
-    launch_analogue_inputs(t, h->a_tab, B, N, zk, fm, st);
-    KCHECK();
-    int rc2 = sample_loop(h, mode, T, steps, resample_steps, L, aj->merge_alpha, aj->merge_sigma, sigma_0, alpha_0, sigma_x,
-                          h->g_ctx.as<float>(), zk, fm, nullptr, seed, sample_offset, h->g_ids.as<int64_t>(),
-                          h->g_z.as<float>(), h->g_x.as<float>(), h->g_cls.as<int32_t>(), nullptr, nullptr, 0, s);
-    if (rc2) return rc2;
-    return seer_device(h, s);
-  };
-  return generate_graphed(h, key, n_nodes_host, B, N, nullptr, 0, ctx_host, seed, sample_offset, sample_ids_host, x_out,
-                          atom_class_out, bonds_out, stream, upload, device);
+  p.kind = any_fixed ? GEN_ANALOGUE_FIXED : GEN_ANALOGUE_FREE;
+  p.loop_mode = any_fixed ? 2 : 3;
+  p.level = L;
+  p.alpha_L = aj->merge_alpha;
+  p.sigma_L = aj->merge_sigma;
+  p.tab = &t;
+  return generate_graphed(h, c, p, generate_analogue_device);
 }
 
 // ---------------------------------------------------------------------------------------------------------------

@@ -270,23 +270,15 @@ class Engine:
         """End-to-end with host inputs: returns (x (B,N,3) f32, atom_class (B,N) i32, bonds (B,42,42) i8) in pinned host
         buffers, or -- `device_out=True`, used by the multi-GPU driver whose gather runs on the device -- in device
         tensors.  `sample_ids` (B int64): global ids keying the device noise (default `sample_offset + b`)."""
-        nn, ctxh, ids, out = self._host_call_inputs("generate_host", n_nodes, max_n_nodes, ctx, sample_ids, out, device_out)
-        B, N = int(nn.size), int(max_n_nodes)
-        gamma, steps = self._steps_cached(T, 3)
-        dec = decode_scalars(gamma)
-        rc = self.lib.mlcg_generate(self.h, nn.ctypes.data_as(C.c_void_p), B, N, _ptr(ctxh), T, steps, resample_steps,
-                                    dec["sigma_0"], dec["alpha_0"], dec["sigma_x"], seed, sample_offset,
-                                    None if ids is None else ids.ctypes.data_as(C.c_void_p), _ptr(out[0]),
-                                    _ptr(out[1]), _ptr(out[2]), self._stream())
-        self._check(rc, "generate")
-        self.check_finite("generate")
-        self.B, self.N = B, N
-        self.n_nodes = torch.from_numpy(nn.copy())
-        return out
+        return self._generate("generate_host", "generate", self.lib.mlcg_generate, None, n_nodes, max_n_nodes, ctx, T, 3,
+                              resample_steps, seed, sample_offset, sample_ids, out, device_out)
 
-    def _host_call_inputs(self, what, n_nodes, max_n_nodes, ctx, sample_ids, out, device_out):
-        """Host inputs of generate_host / generate_fragment_host: atom counts (int32), pinned (B,3) context, sample ids
-        (int64 or None) and the output buffers (`out`, or new pinned host / device tensors)."""
+    def _generate(self, name, what, call, table, n_nodes, max_n_nodes, ctx, T, blend_power, resample_steps, seed,
+                  sample_offset, sample_ids, out, device_out):
+        """The host generation call `call` (an mlcg_generate* prototype) once its kind's table (a ctypes structure passed
+        by reference, or None) is built: host inputs, schedule, errors and non-finite warnings under `what`, and the batch
+        bookkeeping.  Argument errors found here name the public method `name`.  Returns the outputs: `out`, or new
+        pinned host / device tensors (x (B,N,3), atom_class (B,N), bonds (B,42,42))."""
         nn = np.ascontiguousarray(np.asarray(n_nodes, dtype=np.int32).reshape(-1))
         B, N = int(nn.size), int(max_n_nodes)
         ctxh = torch.from_numpy(np.ascontiguousarray(ctx, dtype=np.float32).reshape(B, 3)).pin_memory()
@@ -294,7 +286,7 @@ class Engine:
         if sample_ids is not None:
             ids = np.ascontiguousarray(np.asarray(sample_ids, dtype=np.int64).reshape(-1))
             if ids.size != B:
-                raise ValueError("%s: sample_ids must hold one id per sample" % what)
+                raise ValueError("%s: sample_ids must hold one id per sample" % name)
         if out is None:
             if device_out:
                 out = (torch.empty(B, N, 3, device=self.device), torch.empty(B, N, dtype=torch.int32, device=self.device),
@@ -302,7 +294,33 @@ class Engine:
             else:
                 out = (torch.empty(B, N, 3).pin_memory(), torch.empty(B, N, dtype=torch.int32).pin_memory(),
                        torch.empty(B, 42, 42, dtype=torch.int8).pin_memory())
-        return nn, ctxh, ids, out
+        gamma, steps = self._steps_cached(T, blend_power)
+        dec = decode_scalars(gamma)
+        head = (self.h,) if table is None else (self.h, C.byref(table))
+        rc = call(*head, nn.ctypes.data_as(C.c_void_p), B, N, _ptr(ctxh), T, steps, resample_steps, dec["sigma_0"],
+                  dec["alpha_0"], dec["sigma_x"], seed, sample_offset,
+                  None if ids is None else ids.ctypes.data_as(C.c_void_p), _ptr(out[0]), _ptr(out[1]), _ptr(out[2]),
+                  self._stream())
+        self._check(rc, what)
+        self.check_finite(what)
+        self.B, self.N = B, N
+        self.n_nodes = torch.from_numpy(nn.copy())
+        return out
+
+    @staticmethod
+    def _pack_molecules(what, noun, mols):
+        """(coordinates (n,3), one-hot (n,8)) pairs -> atom counts (int32) and the coordinates (sum n,3) and one-hots
+        (sum n,8) back to back, float32."""
+        xs, hs = [], []
+        for x, h in mols:
+            x = np.asarray(torch.as_tensor(x).detach().cpu().numpy(), dtype=np.float32)
+            h = np.asarray(torch.as_tensor(h).detach().cpu().numpy(), dtype=np.float32)
+            if x.ndim != 2 or x.shape[1] != 3 or h.shape != (x.shape[0], 8):
+                raise ValueError("%s: %s must be coordinates (n,3) and a one-hot (n,8)" % (what, noun))
+            xs.append(x)
+            hs.append(h)
+        return (np.array([x.shape[0] for x in xs], dtype=np.int32), np.ascontiguousarray(np.concatenate(xs).reshape(-1, 3)),
+                np.ascontiguousarray(np.concatenate(hs).reshape(-1, 8)))
 
     def generate_fragment_host(self, n_nodes: np.ndarray, max_n_nodes: int, ctx: np.ndarray, fragment_x, fragment_h,
                                inertial_fragment_matching: bool = True, reference_context=None, context_norms=None,
@@ -316,11 +334,13 @@ class Engine:
         otherwise the fragment is inpainted.  `ctx` (B,3) is the normalised reference context of every sample.  Same
         outputs, noise keys and graph replay as generate_host; the result equals the eager composition of
         MLConformerGenerator.edm_sample_tensors + the GCN bit for bit."""
-        return self._fragment_jobs_call("generate_fragment_host", n_nodes, max_n_nodes, ctx, np.zeros(np.size(n_nodes), np.int32),
+        what = "generate_fragment_host"
+        fj, keep = self._fragment_table(what, np.size(n_nodes), np.zeros(np.size(n_nodes), np.int32),
                                         [(fragment_x, fragment_h)], inertial_fragment_matching,
                                         None if reference_context is None else [reference_context], context_norms, T,
-                                        resample_steps, blend_power, diffusion_level, seed, sample_offset, sample_ids, out,
-                                        device_out)
+                                        blend_power, diffusion_level)
+        return self._generate(what, "generate_fragment", self.lib.mlcg_generate_fragment_jobs, fj, n_nodes, max_n_nodes,
+                              ctx, T, blend_power, resample_steps, seed, sample_offset, sample_ids, out, device_out)
 
     def generate_fragment_jobs_host(self, n_nodes: np.ndarray, max_n_nodes: int, ctx: np.ndarray, job_of_sample,
                                     fragments, inertial_fragment_matching: bool = True, reference_contexts=None,
@@ -332,58 +352,37 @@ class Engine:
         reference context reference_contexts[job_of_sample[b]].  `ctx` (B,3) is every sample's normalised context; the
         loop settings are shared.  Same outputs, noise keys and graph replay as generate_fragment_host, and every sample
         equals a call holding only its own job with the same sample id, bit for bit."""
-        return self._fragment_jobs_call("generate_fragment_jobs_host", n_nodes, max_n_nodes, ctx, job_of_sample, fragments,
-                                        inertial_fragment_matching, reference_contexts, context_norms, T, resample_steps,
-                                        blend_power, diffusion_level, seed, sample_offset, sample_ids, out, device_out)
+        what = "generate_fragment_jobs_host"
+        fj, keep = self._fragment_table(what, np.size(n_nodes), job_of_sample, fragments, inertial_fragment_matching,
+                                        reference_contexts, context_norms, T, blend_power, diffusion_level)
+        return self._generate(what, "generate_fragment", self.lib.mlcg_generate_fragment_jobs, fj, n_nodes, max_n_nodes,
+                              ctx, T, blend_power, resample_steps, seed, sample_offset, sample_ids, out, device_out)
 
-    def _fragment_jobs_call(self, what, n_nodes, max_n_nodes, ctx, job_of_sample, fragments, inertial_fragment_matching,
-                            reference_contexts, context_norms, T, resample_steps, blend_power, diffusion_level, seed,
-                            sample_offset, sample_ids, out, device_out):
-        nn, ctxh, ids, out = self._host_call_inputs(what, n_nodes, max_n_nodes, ctx, sample_ids, out, device_out)
-        B, N = int(nn.size), int(max_n_nodes)
+    def _fragment_table(self, what, B, job_of_sample, fragments, inertial_fragment_matching, reference_contexts,
+                        context_norms, T, blend_power, diffusion_level):
+        """mlcg_fragment_jobs and the host arrays it points to, which must outlive the call."""
         job = np.ascontiguousarray(np.asarray(job_of_sample, dtype=np.int32).reshape(-1))
         if job.size != B:
             raise ValueError("%s: job_of_sample must hold one job per sample" % what)
-        ffx, ffh = [], []
-        for fx, fh in fragments:
-            fx = np.asarray(torch.as_tensor(fx).detach().cpu().numpy(), dtype=np.float32)
-            fh = np.asarray(torch.as_tensor(fh).detach().cpu().numpy(), dtype=np.float32)
-            if fx.ndim != 2 or fx.shape[1] != 3 or fh.shape != (fx.shape[0], 8):
-                raise ValueError("%s: the fragment must be coordinates (n,3) and a one-hot (n,8)" % what)
-            ffx.append(fx)
-            ffh.append(fh)
-        n_ff = np.array([f.shape[0] for f in ffx], dtype=np.int32)
-        packed_x = np.ascontiguousarray(np.concatenate(ffx, axis=0).reshape(-1, 3), dtype=np.float32)
-        packed_h = np.ascontiguousarray(np.concatenate(ffh, axis=0).reshape(-1, 8), dtype=np.float32)
-        gamma, steps = self._steps_cached(T, blend_power)
-        dec = decode_scalars(gamma)
-        fj = _lib.FragmentJobs(2 if inertial_fragment_matching else 1, len(ffx), job.ctypes.data, n_ff.ctypes.data,
-                               packed_x.ctypes.data, packed_h.ctypes.data)
-        keep = []
+        n_ff, packed_x, packed_h = self._pack_molecules(what, "the fragment", fragments)
+        keep = [job, n_ff, packed_x, packed_h]
+        fj = _lib.FragmentJobs(2 if inertial_fragment_matching else 1, n_ff.size, *(a.ctypes.data for a in keep))
         if inertial_fragment_matching:
-            if reference_contexts is None or len(reference_contexts) != len(ffx):
+            if reference_contexts is None or len(reference_contexts) != n_ff.size:
                 raise ValueError("%s: inertial fragment matching needs the raw reference_context of every job" % what)
             from .config import CONTEXT_NORMS
             from .mol_utils import ifm_moi_prologue
             norms = CONTEXT_NORMS if context_norms is None else context_norms
-            pro = [ifm_moi_prologue(torch.from_numpy(fx), ref) for fx, ref in zip(ffx, reference_contexts)]
-            keep = [torch.stack([p[0] for p in pro]).contiguous(), torch.stack([p[1] for p in pro]).contiguous()] + \
+            pro = [ifm_moi_prologue(torch.from_numpy(fx), ref)
+                   for fx, ref in zip(np.split(packed_x, np.cumsum(n_ff)[:-1]), reference_contexts)]
+            ifm = [torch.stack([p[0] for p in pro]).contiguous(), torch.stack([p[1] for p in pro]).contiguous()] + \
                 [torch.as_tensor(norms[k], dtype=torch.float32).contiguous() for k in ("mean", "mad")]
-            lvl = forward_level_scalars(gamma, diffusion_level)
+            keep += ifm
+            lvl = forward_level_scalars(self._steps_cached(T, blend_power)[0], diffusion_level)
             fj.diffusion_level, fj.merge_alpha, fj.merge_sigma = int(diffusion_level), lvl["alpha"], lvl["sigma"]
             fj.moi_gen_origin_host, fj.ff_weighted_com_host, fj.norm_mean_host, fj.norm_mad_host = (
-                t.data_ptr() for t in keep)
-        rc = self.lib.mlcg_generate_fragment_jobs(self.h, C.byref(fj), nn.ctypes.data_as(C.c_void_p), B, N, _ptr(ctxh), T,
-                                                  steps, resample_steps, dec["sigma_0"], dec["alpha_0"], dec["sigma_x"],
-                                                  seed, sample_offset,
-                                                  None if ids is None else ids.ctypes.data_as(C.c_void_p), _ptr(out[0]),
-                                                  _ptr(out[1]), _ptr(out[2]), self._stream())
-        del keep
-        self._check(rc, "generate_fragment")
-        self.check_finite("generate_fragment")
-        self.B, self.N = B, N
-        self.n_nodes = torch.from_numpy(nn.copy())
-        return out
+                t.data_ptr() for t in ifm)
+        return fj, keep
 
     @staticmethod
     def _analogue_table(what, job_of_sample, B, parents, fixed):
@@ -393,23 +392,15 @@ class Engine:
             raise ValueError("%s: job_of_sample must hold one job per sample" % what)
         if fixed is not None and len(fixed) != len(parents):
             raise ValueError("%s: fixed must hold one flag array per parent" % what)
-        px, ph, pf = [], [], []
-        for j, (x, h) in enumerate(parents):
-            x = np.asarray(torch.as_tensor(x).detach().cpu().numpy(), dtype=np.float32)
-            h = np.asarray(torch.as_tensor(h).detach().cpu().numpy(), dtype=np.float32)
-            if x.ndim != 2 or x.shape[1] != 3 or h.shape != (x.shape[0], 8):
-                raise ValueError("%s: a parent must be coordinates (n,3) and a one-hot (n,8)" % what)
-            f = np.zeros(x.shape[0], np.int32) if fixed is None or fixed[j] is None else \
-                np.asarray(fixed[j]).reshape(-1).astype(np.int32)
-            if f.size != x.shape[0]:
+        n_atoms, px, ph = Engine._pack_molecules(what, "a parent", parents)
+        pf = []
+        for j, n in enumerate(n_atoms):
+            f = np.zeros(n, np.int32) if fixed is None or fixed[j] is None else np.asarray(fixed[j]).reshape(-1).astype(np.int32)
+            if f.size != n:
                 raise ValueError("%s: the fixed flags must hold one entry per parent atom" % what)
-            px.append(x)
-            ph.append(h)
             pf.append(f)
-        keep = [job, np.array([x.shape[0] for x in px], dtype=np.int32),
-                np.ascontiguousarray(np.concatenate(px).reshape(-1, 3)), np.ascontiguousarray(np.concatenate(ph).reshape(-1, 8)),
-                np.ascontiguousarray(np.concatenate(pf))]
-        return _lib.AnalogueJobs(len(px), *(a.ctypes.data for a in keep)), keep
+        keep = [job, n_atoms, px, ph, np.ascontiguousarray(np.concatenate(pf))]
+        return _lib.AnalogueJobs(n_atoms.size, *(a.ctypes.data for a in keep)), keep
 
     def analogue_inputs(self, job_of_sample, parents, fixed, max_n_nodes: int):
         """Device version of the analogue jobs' first step (mlcg_analogue_inputs): (z_known (B,N,11), fixed_mask (B,N)) with
@@ -435,27 +426,14 @@ class Engine:
         atom or none has.  `ctx` (B,3) is every sample's normalised context.  Same outputs, noise keys and graph replay as
         generate_fragment_jobs_host; every sample equals a call holding only its own job with the same id, bit for bit,
         and the result equals the eager composition analogue_inputs + sample + the GCN."""
-        nn, ctxh, ids, out = self._host_call_inputs("generate_analogue_jobs_host", n_nodes, max_n_nodes, ctx, sample_ids,
-                                                    out, device_out)
-        B, N = int(nn.size), int(max_n_nodes)
-        aj, keep = self._analogue_table("generate_analogue_jobs_host", job_of_sample, B, parents, fixed)
-        gamma, steps = self._steps_cached(T, blend_power)
-        dec = decode_scalars(gamma)
+        what = "generate_analogue_jobs_host"
+        aj, keep = self._analogue_table(what, job_of_sample, np.size(n_nodes), parents, fixed)
         if not 1 <= int(diffusion_level) <= T:
             raise ValueError("generate_analogue_jobs_host: diffusion_level must lie in [1, T=%d]" % T)
-        lvl = forward_level_scalars(gamma, int(diffusion_level))
+        lvl = forward_level_scalars(self._steps_cached(T, blend_power)[0], int(diffusion_level))
         aj.diffusion_level, aj.merge_alpha, aj.merge_sigma = int(diffusion_level), lvl["alpha"], lvl["sigma"]
-        rc = self.lib.mlcg_generate_analogue_jobs(self.h, C.byref(aj), nn.ctypes.data_as(C.c_void_p), B, N, _ptr(ctxh), T,
-                                                  steps, resample_steps, dec["sigma_0"], dec["alpha_0"], dec["sigma_x"],
-                                                  seed, sample_offset,
-                                                  None if ids is None else ids.ctypes.data_as(C.c_void_p), _ptr(out[0]),
-                                                  _ptr(out[1]), _ptr(out[2]), self._stream())
-        del keep
-        self._check(rc, "generate_analogue")
-        self.check_finite("generate_analogue")
-        self.B, self.N = B, N
-        self.n_nodes = torch.from_numpy(nn.copy())
-        return out
+        return self._generate(what, "generate_analogue", self.lib.mlcg_generate_analogue_jobs, aj, n_nodes, max_n_nodes,
+                              ctx, T, blend_power, resample_steps, seed, sample_offset, sample_ids, out, device_out)
 
     # ------------------------------------------------------------------------------------------------------------
     def num_edges(self) -> int:
