@@ -160,6 +160,10 @@ int mlcg_seer_forward(mlcg_handle* h, const int32_t* elements, const float* dist
  *    geometry (B, N, per-sample atom counts, the kind's table sizes) and every scalar baked into the sequence (precision,
  *    schedule, decode scalars, the kind's loop settings).  A new key rebuilds the batch plan (mlcg_set_batch); calls of
  *    different kinds therefore invalidate each other's graph.
+ *  - a captured graph never outlives a buffer it references.  Every other call on the handle may run between two
+ *    generation calls; one that reallocates such a buffer -- mlcg_set_batch, new weights, or mlcg_seer_forward with more
+ *    molecules per 3072-molecule chunk than the graph's batch, which grows the GCN workspaces -- first synchronises the
+ *    device and drops the graph and its key, so the next generation call runs eagerly and the one after captures again.
  *  - the context, the sample ids, {seed, sample_offset} and the kind's job table are uploaded on every call, so a replay
  *    never sees a previous call's inputs, and new inputs of the same sizes replay the graph.
  *  - the noise is keyed by (seed, global sample id), and every kernel works on each sample alone: a sample's result does

@@ -112,9 +112,12 @@ struct mlcg_handle {
   std::vector<int64_t> ids_stage;
   // test gemm
   DevBuf tg_a, tg_w, tg_b, tg_c;
-  // CUDA-graph replay of the host generation calls (whole device sequence + GCN as one graph)
+  // CUDA-graph replay of the host generation calls (whole device sequence + GCN as one graph).  The graph holds the
+  // addresses of the weights, the batch plans and every workspace above except the hook and test-gemm buffers; those grow
+  // only through grow(), which drops the graph first.
   DevBuf noise_ctl;               // {seed, sample_offset} read by the noise kernels when use_noise_ctl is set
   bool use_noise_ctl = false;
+  bool capturing = false;         // a generation call's device sequence is being captured into gen_graph
   cudaGraphExec_t gen_graph = nullptr;
   std::vector<long long> gen_key;  // graph_key of the call the graph was captured for
   int gen_key_hits = 0;            // calls seen with the current key (1st runs eagerly, 2nd captures)
@@ -147,6 +150,43 @@ struct mlcg_handle {
   } while (0)
 
 static thread_local std::string g_create_err;
+
+// Drops the captured generation graph and its key once nothing is in flight: the next host generation call runs eagerly,
+// the one after captures again.
+static int drop_gen_graph(mlcg_handle* h) {
+  CK(cudaDeviceSynchronize());
+  if (h->gen_graph) { cudaGraphExecDestroy(h->gen_graph); h->gen_graph = nullptr; }
+  h->gen_key.clear();
+  h->gen_key_hits = 0;
+  return MLCG_OK;
+}
+
+// Grows a handle buffer that a captured generation graph may reference (see mlcg_handle).  Reallocating frees the old
+// address, so an existing graph is dropped first; any entry point -- mlcg_seer_forward with more molecules than the
+// graph's batch, say -- may grow a workspace between two generation calls.  A growth during a capture would bake an
+// address into the graph that the eager first call should have fixed; it is a bug and fails the call.
+static int grow(mlcg_handle* h, DevBuf& b, size_t need) {
+  if (need <= b.bytes) return MLCG_OK;
+  if (h->capturing) FAIL(MLCG_E_STATE, "internal error: a workspace grew during a CUDA graph capture");
+  if (h->gen_graph) {
+    const int rc = drop_gen_graph(h);
+    if (rc) return rc;
+  }
+  CK(b.ensure(need));
+  return MLCG_OK;
+}
+#define GROW(buf, bytes)                     \
+  do {                                       \
+    const int _rc = grow(h, (buf), (bytes)); \
+    if (_rc) return _rc;                     \
+  } while (0)
+
+// Sets a flag for the lifetime of a scope, whichever way the scope is left.
+struct FlagScope {
+  bool& f;
+  explicit FlagScope(bool& flag) : f(flag) { f = true; }
+  ~FlagScope() { f = false; }
+};
 
 // kernel classes of one EGNN forward (mlcg_egnn_forward_breakdown)
 enum { BD_START = -1, BD_PREPARE = 0, BD_PQ = 1, BD_EDGE_GCL = 2, BD_EDGE_EQUIV = 3, BD_FIXUP = 4, BD_MLP1 = 5, BD_MLP2 = 6,
@@ -466,10 +506,7 @@ extern "C" const char* mlcg_last_error(mlcg_handle* h) { return h ? h->err.c_str
 // ---------------------------------------------------------------------------------------------------------------
 static int copy_weights(mlcg_handle* h, const mlcg_weight_desc* w, int n, std::map<std::string, Wt>& dst) {
   // new weights invalidate a captured generation graph (it holds the old buffers' addresses); nothing may be in flight
-  CK(cudaDeviceSynchronize());
-  if (h->gen_graph) { cudaGraphExecDestroy(h->gen_graph); h->gen_graph = nullptr; }
-  h->gen_key.clear();
-  h->gen_key_hits = 0;
+  if (const int rc = drop_gen_graph(h)) return rc;
   for (int i = 0; i < n; ++i) {
     if (!w[i].name || !w[i].data || w[i].rows <= 0 || w[i].cols <= 0) FAIL(MLCG_E_ARG, "bad weight descriptor");
     Wt t;
@@ -499,7 +536,7 @@ static int need(mlcg_handle* h, std::map<std::string, Wt>& m, const std::string&
 }
 static int pad_vec(mlcg_handle* h, DevBuf& dst, const float* src, int stride, int n_real, int n_pad, int dst_off = 0,
                    int alloc = -1, float scale = 1.0f) {
-  CK(dst.ensure((size_t)(alloc < 0 ? n_pad : alloc) * sizeof(float)));
+  GROW(dst, (size_t)(alloc < 0 ? n_pad : alloc) * sizeof(float));
   k_pad_vector<<<(n_pad + 127) / 128, 128>>>(src, stride, n_real, dst.as<float>() + dst_off, n_pad, scale);
   KCHECK();
   return MLCG_OK;
@@ -562,7 +599,7 @@ extern "C" int mlcg_load_egnn(mlcg_handle* h, const mlcg_weight_desc* w, int n) 
     if (mode == PREC_FP32_SIMT) continue;
     const size_t blk448 = (size_t)HP * CHUNK_BYTES;
     // W1 split into the P (cols 0..419) and Q (cols 420..839) projections: N = 896 as two 448-row tiles
-    CK(L.w1ab_op.ensure(2 * kc * blk448));
+    GROW(L.w1ab_op, 2 * kc * blk448);
     for (int half = 0; half < 2; ++half) {
       PackArgs a{};
       a.src = L.w1.d; a.ld = 2 * HID + 2; a.n_real = HID; a.n_src_off = 0; a.bn = HP; a.n_kc = kc;
@@ -573,7 +610,7 @@ extern "C" int mlcg_load_egnn(mlcg_handle* h, const mlcg_weight_desc* w, int n) 
       h->launches++;
     }
     {  // W2 with b2 folded into K column 420
-      CK(L.w2_op.ensure(kc * blk448));
+      GROW(L.w2_op, kc * blk448);
       PackArgs a{};
       a.src = L.w2.d; a.ld = HID; a.n_real = HID; a.bn = HP; a.n_kc = kc; a.seg_len = HP; a.kreal0 = HID;
       a.bias = L.b2.d; a.bias_k = BIAS_COL; a.dst = L.w2_op.as<uint8_t>(); a.scale = es;
@@ -581,7 +618,7 @@ extern "C" int mlcg_load_egnn(mlcg_handle* h, const mlcg_weight_desc* w, int n) 
       h->launches++;
     }
     if (!L.equiv) {
-      CK(L.w3_op.ensure(2 * kc * blk448));
+      GROW(L.w3_op, 2 * kc * blk448);
       PackArgs a{};
       a.src = L.w3.d; a.ld = 2 * HID; a.n_real = HID; a.bn = HP; a.n_kc = 2 * kc; a.seg_len = HP;
       a.kreal0 = HID; a.kofs0 = 0; a.kreal1 = HID; a.kofs1 = HID; a.bias = nullptr; a.bias_k = -1;
@@ -589,7 +626,7 @@ extern "C" int mlcg_load_egnn(mlcg_handle* h, const mlcg_weight_desc* w, int n) 
       a.dst = L.w3_op.as<uint8_t>();
       CK(launch_pack(mode, a, 1, 0));
       h->launches++;
-      CK(L.w4_op.ensure(kc * blk448));
+      GROW(L.w4_op, kc * blk448);
       PackArgs b{};
       b.src = L.w4.d; b.ld = HID; b.n_real = HID; b.bn = HP; b.n_kc = kc; b.seg_len = HP; b.kreal0 = HID;
       b.bias = nullptr; b.bias_k = -1; b.dst = L.w4_op.as<uint8_t>();
@@ -622,7 +659,7 @@ extern "C" int mlcg_load_seer(mlcg_handle* h, const mlcg_weight_desc* w, int n) 
     if ((r = pad_vec(h, S.b_pad, S.b.d, 1, nn, npad))) return r;
     if (h->precision == PREC_FP32_SIMT) return MLCG_OK;
     const int kc = (kk + epc(seer_mode) - 1) / epc(seer_mode);
-    CK(S.w_op.ensure((size_t)(npad / 256) * ksplit * kc * 256 * CHUNK_BYTES));
+    GROW(S.w_op, (size_t)(npad / 256) * ksplit * kc * 256 * CHUNK_BYTES);
     PackArgs a{};
     a.src = S.w.d; a.ld = kk; a.n_real = nn; a.bn = 256; a.n_kc = ksplit * kc; a.seg_len = kc * epc(seer_mode);
     a.kreal0 = kk; a.kofs0 = 0; a.bias = nullptr; a.bias_k = -1; a.dst = S.w_op.as<uint8_t>();
@@ -756,15 +793,15 @@ static int build_plan(mlcg_handle* h, BatchPlan& p, const int32_t* n_nodes, int 
   p.n_mtiles = (p.M + TILE_M - 1) / TILE_M;
   p.n_etiles = (int)tiles.size();
   const size_t mpad = (size_t)p.n_mtiles * TILE_M;
-  CK(p.d_n_nodes.ensure(B * sizeof(int)));
-  CK(p.d_node_off.ensure((B + 1) * sizeof(int)));
-  CK(p.d_node_mol.ensure(p.M * sizeof(int)));
-  CK(p.d_node_edge_off.ensure(p.M * sizeof(int)));
-  CK(p.d_tiles.ensure(tiles.size() * sizeof(EdgeTile)));
+  GROW(p.d_n_nodes, B * sizeof(int));
+  GROW(p.d_node_off, (B + 1) * sizeof(int));
+  GROW(p.d_node_mol, p.M * sizeof(int));
+  GROW(p.d_node_edge_off, p.M * sizeof(int));
+  GROW(p.d_tiles, tiles.size() * sizeof(EdgeTile));
   p.n_fix = (int)fix_node.size();
-  CK(p.d_fix_node.ensure(std::max<size_t>(fix_node.size(), 1) * sizeof(int)));
-  CK(p.fix_agg.ensure(std::max<size_t>(fix_node.size(), 1) * HP * sizeof(float)));
-  CK(p.fix_dx.ensure(std::max<size_t>(fix_node.size(), 1) * 4 * sizeof(float)));
+  GROW(p.d_fix_node, std::max<size_t>(fix_node.size(), 1) * sizeof(int));
+  GROW(p.fix_agg, std::max<size_t>(fix_node.size(), 1) * HP * sizeof(float));
+  GROW(p.fix_dx, std::max<size_t>(fix_node.size(), 1) * 4 * sizeof(float));
   CK(cudaMemcpy(p.d_n_nodes.p, n_nodes, B * sizeof(int), cudaMemcpyHostToDevice));
   CK(cudaMemcpy(p.d_node_off.p, p.h_node_off.data(), (B + 1) * sizeof(int), cudaMemcpyHostToDevice));
   CK(cudaMemcpy(p.d_node_mol.p, node_mol.data(), p.M * sizeof(int), cudaMemcpyHostToDevice));
@@ -775,17 +812,17 @@ static int build_plan(mlcg_handle* h, BatchPlan& p, const int32_t* n_nodes, int 
   CK(cudaMemset(p.fix_agg.p, 0, std::max<size_t>(fix_node.size(), 1) * HP * sizeof(float)));
   CK(cudaMemset(p.fix_dx.p, 0, std::max<size_t>(fix_node.size(), 1) * 4 * sizeof(float)));
   // workspaces (zero-initialised on growth; padded rows / columns are never written afterwards)
-  CK(h->x0.ensure(mpad * 3 * sizeof(float)));
-  CK(h->xa.ensure(mpad * 3 * sizeof(float)));
-  CK(h->xb.ensure(mpad * 3 * sizeof(float)));
-  CK(h->h_res.ensure(mpad * HP * sizeof(float)));
-  CK(h->pq.ensure(mpad * 2 * HP * sizeof(float)));
-  CK(h->t_dev.ensure(B * sizeof(float)));
-  CK(h->nf_flag.ensure(sizeof(int)));
-  CK(h->eps_dev.ensure((size_t)B * N * ZC * sizeof(float)));
+  GROW(h->x0, mpad * 3 * sizeof(float));
+  GROW(h->xa, mpad * 3 * sizeof(float));
+  GROW(h->xb, mpad * 3 * sizeof(float));
+  GROW(h->h_res, mpad * HP * sizeof(float));
+  GROW(h->pq, mpad * 2 * HP * sizeof(float));
+  GROW(h->t_dev, B * sizeof(float));
+  GROW(h->nf_flag, sizeof(int));
+  GROW(h->eps_dev, (size_t)B * N * ZC * sizeof(float));
   if (h->precision == PREC_FP32_SIMT) {
-    CK(h->agg_f32.ensure(mpad * HP * sizeof(float)));
-    CK(h->t_f32.ensure(mpad * HP * sizeof(float)));
+    GROW(h->agg_f32, mpad * HP * sizeof(float));
+    GROW(h->t_f32, mpad * HP * sizeof(float));
     // chunk the edge list so the materialised edge activations stay bounded
     const int cap = 49152;
     p.simt_chunks.clear();
@@ -802,13 +839,13 @@ static int build_plan(mlcg_handle* h, BatchPlan& p, const int32_t* n_nodes, int 
       p.simt_chunks.push_back(c);
       nb = c.node_end;
     }
-    CK(h->a1.ensure((size_t)(cap + 64) * HP * sizeof(float)));
-    CK(h->m2.ensure((size_t)(cap + 64) * HP * sizeof(float)));
+    GROW(h->a1, (size_t)(cap + 64) * HP * sizeof(float));
+    GROW(h->m2, (size_t)(cap + 64) * HP * sizeof(float));
   } else {
     const size_t opb = (size_t)p.n_mtiles * h->kc448() * A_CHUNK_BYTES;
-    CK(h->h_op.ensure(opb));
-    CK(h->agg_op.ensure(opb));
-    CK(h->t_op.ensure(opb));
+    GROW(h->h_op, opb);
+    GROW(h->agg_op, opb);
+    GROW(h->t_op, opb);
   }
   return MLCG_OK;
 }
@@ -819,11 +856,8 @@ extern "C" int mlcg_set_batch(mlcg_handle* h, const int32_t* n_nodes, int B, int
   CK(cudaSetDevice(h->device));
   // The plan buffers below are rewritten with synchronous copies on the NULL stream while earlier calls may still be
   // running on the caller's (possibly non-blocking) streams: drain the device first.  set_batch is documented synchronous.
-  CK(cudaDeviceSynchronize());
-  // any change of the batch plan invalidates the graph captured by mlcg_generate / mlcg_generate_fragment
-  if (h->gen_graph) { cudaGraphExecDestroy(h->gen_graph); h->gen_graph = nullptr; }
-  h->gen_key.clear();
-  h->gen_key_hits = 0;
+  // Any change of the batch plan invalidates the graph captured by the host generation calls.
+  if (const int rc = drop_gen_graph(h)) return rc;
   h->batch_set = false;
   h->pl = &h->plans[0];
   const int rc = build_plan(h, h->plans[0], n_nodes, B, N);
@@ -1243,17 +1277,17 @@ static int seer_chunk(mlcg_handle* h, const int32_t* elements, const float* dist
   const int kcH = SEER_H / epc(mode), kcE = SEER_E / epc(mode);
   const int split3 = (!simt && seer_split3()) ? 1 : 0, ks = split3 ? 3 : 1;
   auto& m = h->seer_w;
-  CK(h->s_ld.ensure((size_t)B * SEER_D * SEER_D * 4));
-  CK(h->s_la.ensure((size_t)B * SEER_D * SEER_D * 4));
-  CK(h->s_rowd.ensure(rpad * 4));
-  CK(h->s_rowa.ensure(rpad * 4));
-  CK(h->s_x64.ensure(rpad * SEER_E * 4));
-  CK(h->s_x.ensure(rpad * SEER_H * 4));
-  CK(h->s_emb.ensure(rpad * 4));
-  CK(h->s_add.ensure(rpad * SEER_E * 4));
-  CK(h->s_raw.ensure(rpad * 224 * 4));
-  if (simt) CK(h->s_y_f32.ensure(rpad * SEER_H * 4));
-  else CK(h->s_y_op.ensure((size_t)mt * ks * kcH * A_CHUNK_BYTES));
+  GROW(h->s_ld, (size_t)B * SEER_D * SEER_D * 4);
+  GROW(h->s_la, (size_t)B * SEER_D * SEER_D * 4);
+  GROW(h->s_rowd, rpad * 4);
+  GROW(h->s_rowa, rpad * 4);
+  GROW(h->s_x64, rpad * SEER_E * 4);
+  GROW(h->s_x, rpad * SEER_H * 4);
+  GROW(h->s_emb, rpad * 4);
+  GROW(h->s_add, rpad * SEER_E * 4);
+  GROW(h->s_raw, rpad * 224 * 4);
+  if (simt) GROW(h->s_y_f32, rpad * SEER_H * 4);
+  else GROW(h->s_y_op, (size_t)mt * ks * kcH * A_CHUNK_BYTES);
   k_lnorm<<<B, 64, 0, st>>>(dist, h->s_ld.as<float>(), h->s_rowd.as<float>());
   KCHECK();
   k_lnorm<<<B, 64, 0, st>>>(adj, h->s_la.as<float>(), h->s_rowa.as<float>());
@@ -1521,7 +1555,8 @@ static int generate_analogue_device(mlcg_handle* h, const GenCall& c, const GenP
 // n_nodes / N, plus plan 1 = p.n_gen / p.Ng for IFM) and drops the captured graph.  Every call uploads the per-call
 // inputs -- context, sample ids, {seed, sample_offset} and the job table -- to handle-owned device buffers, then runs
 // `device` and the GCN: eagerly on the first call with a key, captured into a CUDA graph on the second, replayed from
-// then on.  The outputs are copied to c.x_out / c.cls_out / c.bonds_out and the stream is synchronised.
+// then on.  The outputs are copied to c.x_out / c.cls_out / c.bonds_out and the stream is synchronised.  Another entry
+// point that grows a buffer the graph references (grow()) drops the graph, so the next call runs eagerly and recaptures.
 static int generate_graphed(mlcg_handle* h, const GenCall& c, const GenParams& p, GenDevice device) {
   CK(cudaSetDevice(h->device));  // the call may come from any host thread (pipeline.GenerationPipeline's feeder)
   const int B = c.B, N = c.N;
@@ -1543,16 +1578,16 @@ static int generate_graphed(mlcg_handle* h, const GenCall& c, const GenParams& p
   }
   h->gen_key_hits++;
   const size_t bn = (size_t)B * N, dd = (size_t)B * SEER_D * SEER_D;
-  CK(h->g_ctx.ensure((size_t)B * 3 * 4));
-  CK(h->g_z.ensure(bn * ZC * 4));
-  CK(h->g_x.ensure(bn * 3 * 4));
-  CK(h->g_cls.ensure(bn * 4));
-  CK(h->g_el.ensure((size_t)B * SEER_D * 4));
-  CK(h->g_dist.ensure(dd * 4));
-  CK(h->g_adj.ensure(dd * 4));
-  CK(h->g_bonds.ensure(dd));
-  CK(h->noise_ctl.ensure(2 * sizeof(unsigned long long)));
-  CK(h->g_ids.ensure((size_t)B * sizeof(int64_t)));
+  GROW(h->g_ctx, (size_t)B * 3 * 4);
+  GROW(h->g_z, bn * ZC * 4);
+  GROW(h->g_x, bn * 3 * 4);
+  GROW(h->g_cls, bn * 4);
+  GROW(h->g_el, (size_t)B * SEER_D * 4);
+  GROW(h->g_dist, dd * 4);
+  GROW(h->g_adj, dd * 4);
+  GROW(h->g_bonds, dd);
+  GROW(h->noise_ctl, 2 * sizeof(unsigned long long));
+  GROW(h->g_ids, (size_t)B * sizeof(int64_t));
   // global sample ids (the RNG key): always read from this device buffer, so a captured graph replays with any ids
   h->ids_stage.resize((size_t)B);
   for (int b = 0; b < B; ++b) h->ids_stage[b] = c.ids ? c.ids[b] : c.sample_offset + b;
@@ -1566,20 +1601,22 @@ static int generate_graphed(mlcg_handle* h, const GenCall& c, const GenParams& p
   const unsigned long long ctl[2] = {(unsigned long long)c.seed, (unsigned long long)c.sample_offset};
   CK(cudaMemcpyAsync(h->noise_ctl.p, ctl, sizeof(ctl), cudaMemcpyHostToDevice, st));
   if (p.tab) {  // the job table and the z_known / fixed_mask it expands to
-    CK(h->j_tab.ensure(p.tab->blob.size()));
-    CK(h->f_zk.ensure(bn * ZC * 4));
-    CK(h->f_fm.ensure(bn * 4));
+    GROW(h->j_tab, p.tab->blob.size());
+    GROW(h->f_zk, bn * ZC * 4);
+    GROW(h->f_fm, bn * 4);
     if (p.kind == GEN_IFM) {  // the first loop's context, frame and outputs
-      CK(h->f_ctx.ensure((size_t)B * 3 * 4));
-      CK(h->f_shift.ensure((size_t)B * 3 * 4));
-      CK(h->f_rot.ensure((size_t)B * 9 * 4));
-      CK(h->f_ngen.ensure((size_t)B * 4));
-      CK(h->f_xg.ensure((size_t)B * p.Ng * 3 * 4));
-      CK(h->f_clsg.ensure((size_t)B * p.Ng * 4));
+      GROW(h->f_ctx, (size_t)B * 3 * 4);
+      GROW(h->f_shift, (size_t)B * 3 * 4);
+      GROW(h->f_rot, (size_t)B * 9 * 4);
+      GROW(h->f_ngen, (size_t)B * 4);
+      GROW(h->f_xg, (size_t)B * p.Ng * 3 * 4);
+      GROW(h->f_clsg, (size_t)B * p.Ng * 4);
     }
     CK(cudaMemcpyAsync(h->j_tab.p, p.tab->blob.data(), p.tab->blob.size(), cudaMemcpyHostToDevice, st));
   }
-  h->use_noise_ctl = true;  // the noise kernels read {seed, sample_offset} from device memory (graph-replayable)
+  // the noise kernels read {seed, sample_offset} from device memory (graph-replayable) until the call returns, on every
+  // path out of it; eager calls of the other entry points take them from their arguments
+  const FlagScope noise_from_ctl(h->use_noise_ctl);
   auto run = [&]() {  // the kind's sequence, then the GCN
     int rc = device(h, c, p, st);
     return rc ? rc : seer_device(h, st);
@@ -1591,7 +1628,10 @@ static int generate_graphed(mlcg_handle* h, const GenCall& c, const GenParams& p
     cudaGraph_t graph = nullptr;
     const long long launches0 = h->launches;
     CK(cudaStreamBeginCapture(st, cudaStreamCaptureModeThreadLocal));
-    rc = run();
+    {
+      const FlagScope in_capture(h->capturing);
+      rc = run();
+    }
     cudaError_t ce = cudaStreamEndCapture(st, &graph);
     if (rc == MLCG_OK && ce == cudaSuccess && graph != nullptr) {
       ce = cudaGraphInstantiate(&h->gen_graph, graph, 0);
@@ -1603,7 +1643,6 @@ static int generate_graphed(mlcg_handle* h, const GenCall& c, const GenParams& p
     h->launches = launches0;  // nothing has run yet
     if (rc != MLCG_OK || h->gen_graph == nullptr) {
       cudaGetLastError();
-      h->use_noise_ctl = false;
       if (rc == MLCG_OK) FAIL(MLCG_E_STATE, "generate: CUDA graph capture failed");
       return rc;
     }
@@ -1614,7 +1653,6 @@ static int generate_graphed(mlcg_handle* h, const GenCall& c, const GenParams& p
   } else {
     rc = run();
   }
-  h->use_noise_ctl = false;
   if (rc) return rc;
   // the outputs may be pinned host buffers or device buffers (multi-GPU driver: results stay on the device for the gather)
   CK(cudaMemcpyAsync(c.x_out, h->g_x.p, bn * 3 * 4, cudaMemcpyDefault, st));
